@@ -15,7 +15,10 @@ The same JSON line also carries
     device-resident callers (batched IK, trajectory stack) end to end, each with its CPU baseline;
   * `small_batch`: kin_eval latency at the sizes the reference's solver callbacks really use (1, 10, 64, 1024).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the headline step returned in its last timed step (see dump_outputs) so that two builds can
+be compared output for output: the inputs depend only on the arguments (seeded generators).
 """
 import argparse
 import ctypes as C
@@ -56,6 +59,23 @@ def peaks():
         d = json.load(open(p))
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_SAMPLE = 16384          # configurations written by --dump-outputs: T + J of the sample are 45.6 MB in float64
+
+
+def dump_outputs(out_dir, T, J):
+    """T.npy / J.npy: the columns of T (N_LINKS * 12 rows) and J (6 * N_DOF rows) of a fixed sample of the batch, in the
+    SoA layout kin_eval writes them in (row-major: rows x sampled configurations, float64); sample_index.npy: the sampled
+    configuration indices (ascending, stored as float64), drawn with seed 0."""
+    import torch
+    n = T.shape[1]
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    sel = torch.as_tensor(idx, device=T.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "T.npy"), T[:, sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "J.npy"), J[:, sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "sample_index.npy"), idx.astype(np.float64))
 
 
 def ncu_traffic():
@@ -239,7 +259,13 @@ def main():
     ap.add_argument("--skip-variants", dest="no_variants", action="store_true", help="skip the other BASELINE.md rows / layouts")
     ap.add_argument("--skip-callers", dest="no_callers", action="store_true", help="skip the IK / trajectory-stack rows")
     ap.add_argument("--skip-e2e", dest="no_e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the headline step's outputs as DIR/<name>.npy "
+                                                          "(with --gpus > 1: rank 0's shard only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no outputs")
     if args.impl == "reference":
         return reference_main(args)
 
@@ -342,6 +368,8 @@ def main():
         sampler.start()
     total_ms, per, launches = timed(call, args.steps, W)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, T, J)           # before the variant rows below overwrite T / J
     ms_per_step = total_ms / args.steps
     value = world * N / (ms_per_step * 1e-3)
     kern_ms = float(np.mean(per))

@@ -29,13 +29,19 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_device_is_a_loud_error():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    m, joints, _ = scenes.product_fetch()
-    K.set_joint_angles(m, joints, np.zeros(8))
-    with pytest.raises(K.KinError):
-        K.get_transform(m, K.find_link(m, "gripper_link"))
+    """Runs in a child process that sees no CUDA device, so that it also runs on a machine with a GPU."""
+    import subprocess
+    import sys
+    root = os.path.dirname(DATA)
+    code = ("import sys; sys.path[:0] = [%r, %r]\n"
+            "import numpy as np, pytest, kinematics_jl_b200 as K, scenes\n"
+            "m, joints, _ = scenes.product_fetch()\n"
+            "K.set_joint_angles(m, joints, np.zeros(8))\n"
+            "with pytest.raises(K.KinError, match='no CUDA device'):\n"
+            "    K.get_transform(m, K.find_link(m, 'gripper_link'))\n") % (root, os.path.join(root, "tests"))
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True, timeout=600)
+    assert out.returncode == 0, out.stdout + out.stderr
 
 
 def test_mechanism_mirror_structure():
