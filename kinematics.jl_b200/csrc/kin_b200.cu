@@ -57,6 +57,8 @@ struct JitKernel {
     bool ok = false, from_cache = false;
     int regs = 0, block = 0, occ = 0, slots = 0, smem_limit = 0;
     bool cooperative = false;       // grid-wide barrier inside (input batching): launched cooperatively
+    cudaKernel_t fill = nullptr;    // const_fill: the kernel writing the configuration-independent rows (KNCF of them)
+    int fill_rows = 0;
     double compile_ms = 0;
     std::string log;
     ~JitKernel() { if (lib) cudaLibraryUnload(lib); }
@@ -466,6 +468,12 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
         qb = o.coll ? env_ll("KIN_JIT_QBATCH_COLL", 0) : env_ll("KIN_JIT_QBATCH", qb);
         if (qb >= 1 && (qb >= 2 || o.coll)) { o.qbatch = (int)qb; o.min_blocks = 1; }
     }
+    // ... whose rows that do not depend on the configuration (175 of the 348 of FK-all + gripper Jacobian for Fetch) are
+    // then written by a second, fill-shaped kernel instead of one store per configuration (kin_gen_skeleton.cuh:
+    // kin_const_fill_kernel; DESIGN 4.4).  SoA only: a constant row is one contiguous run there, not in the tiled / AoS
+    // layouts.  (KIN_JIT_CONST_FILL=0 stores every row per thread, for A/B measurements.)
+    if (o.layout == KIN_LAYOUT_SOA && o.qbatch > 0 && !o.coll && (o.want_T || o.want_J))
+        o.const_fill = (int)env_ll("KIN_JIT_CONST_FILL", 1) ? 1 : 0;
     return o;
 }
 
@@ -571,6 +579,13 @@ std::shared_ptr<JitKernel> get_jit_with(KinModel *m, DeviceProgram *dp, const ki
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k->occ, (const void *)k->kern, k->block, smem);
     if (e != cudaSuccess || k->occ < 1) { k->log = "occupancy query failed"; cudaGetLastError(); g_jit_failures.fetch_add(1); return nullptr; }
     k->cooperative = o.qbatch > 0;
+    k->fill_rows = g.config.find("#define KCFILL 1") != std::string::npos ? (int)(g.const_T.size() + g.const_J.size()) : 0;
+    if (k->fill_rows > 0 && cudaLibraryGetKernel(&k->fill, k->lib, "kin_const_fill_kernel") != cudaSuccess) {
+        k->log = "loading the constant-row fill kernel";
+        cudaGetLastError();
+        g_jit_failures.fetch_add(1);
+        return nullptr;
+    }
     k->compile_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (std::getenv("KIN_JIT_VERBOSE"))
         std::fprintf(stderr, "[libkin_b200] specialised kernel %s: %d registers, %zu B shared, %d CTAs/SM, %.0f ms%s\n", key.c_str(), k->regs, smem,
@@ -618,6 +633,14 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
     }
     g_launches.fetch_add(1);
     g_jit_launches.fetch_add(1);
+    if (k.fill_rows > 0) {
+        // one 32-byte vector per thread, 256 threads per CTA, blockIdx.y = constant row
+        const long long vec = 32 / (o.precision ? sizeof(float) : sizeof(double));
+        const long long gx = (c->n / vec + 1 + 255) / 256;
+        CUDA_TRY(cudaLaunchKernel((const void *)k.fill, dim3((unsigned)gx, (unsigned)k.fill_rows), dim3(256), args, 0, stream));
+        g_launches.fetch_add(1);
+        g_jit_launches.fetch_add(1);
+    }
     return KIN_OK;
 }
 

@@ -10,10 +10,10 @@
 namespace kin {
 
 std::string GenOptions::key() const {
-    char b[192];
-    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d", precision, layout, (int)want_T, (int)want_J,
+    char b[200];
+    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d", precision, layout, (int)want_T, (int)want_J,
                   (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, (int)ws, block, min_blocks, qbatch,
-                  ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min);
+                  ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min, const_fill);
     return b;
 }
 
@@ -419,7 +419,33 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
       << "\n#define KTILED " << (o.layout == 2 ? 1 : 0) << "\n#define KAOS " << (o.layout == 1 ? 1 : 0) << "\n#define KWS " << (o.ws ? 1 : 0) << "\n";
     c << "#define KBS " << o.block << "\n#define KMINB " << o.min_blocks << "\n#define KWARP " << o.warp << "\n#define KIK " << o.ik << "\n#define KQB " << o.qbatch << "\n#define KSYNC_ON "
       << o.ksync << "\n#define KES32 " << o.es32 << "\n";
+    // the configuration-independent outputs as a table of rows (kin_gen_skeleton.cuh: kin_const_fill_kernel): component (T: k,
+    // J: -1 - k) and value, written as the literals phase 1 stores -- the outputs keep their bits, sign of zero included
+    // -- and, for the store macros, which components the table holds.  Phase 1 keeps every KST_* line (kin_eval_host and
+    // the tests read the generated text); the skeleton drops the listed ones at compile time.
+    const bool cfill = o.const_fill && o.layout == 0 && !o.warp && !o.ik && !o.ws && (!out.const_T.empty() || !out.const_J.empty());
+    c << "#define KCFILL " << (cfill ? 1 : 0) << "\n";
     c << "namespace kin {\n";
+    for (int a = 0; a < 2; ++a) {
+        const std::vector<std::pair<int, double>> &tab = a ? out.const_J : out.const_T;
+        c << "__host__ __device__ constexpr bool " << (a ? "kcf_J" : "kcf_T") << "(int k) {";
+        if (cfill && !tab.empty()) {
+            c << "\n    switch (k) {";
+            for (size_t i = 0; i < tab.size(); ++i) c << (i % 16 ? " " : "\n    ") << "case " << tab[i].first << ":";
+            c << " return true;\n    default: return false;\n    }\n}\n";
+        } else {
+            c << " return false; }\n";
+        }
+    }
+    if (cfill) {
+        const size_t nT = out.const_T.size(), nc = nT + out.const_J.size();
+        auto row = [&](size_t i) { return i < nT ? out.const_T[i] : std::make_pair(-1 - out.const_J[i - nT].first, out.const_J[i - nT].second); };
+        c << "typedef KREAL real;\nconstexpr int KNCF = " << nc << ";\n__device__ const int KCF_ROW[KNCF] = {";
+        for (size_t i = 0; i < nc; ++i) c << (i ? ", " : "") << (i % 16 ? "" : "\n    ") << row(i).first;
+        c << "};\n__device__ const real KCF_VAL[KNCF] = {";
+        for (size_t i = 0; i < nc; ++i) c << (i ? ", " : "") << (i % 6 ? "" : "\n    ") << E.lit(row(i).second);
+        c << "};\n";
+    }
     c << "constexpr int KND = " << ND << ", KDC = " << DC << ", KS = " << S << ", KNFK = " << (o.want_T ? h.n_fk : 0) << ", KNJAC = "
       << (o.want_J ? h.n_jac : 0) << ", KROWS = " << rows << ";\n";
     c << "constexpr int KGRADMODE = " << o.grad_mode << ";\n";

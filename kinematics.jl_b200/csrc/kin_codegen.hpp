@@ -46,6 +46,8 @@ struct GenOptions {
     int bulk = 0;               // 1: tiled layout, FK / Jacobian only: outputs staged per warp and written with cp.async.bulk (TMA)
     int prims = 0;              // 1: the SDF table holds rows other than boxes (sphere / cylinder): the row loops test the kind
     int es32 = 0;               // 1: SoA component stride held in 32 bits (ld < 2^32): one IMAD.WIDE per store address
+    int const_fill = 0;         // 1: SoA, one thread per configuration: the outputs of GenSource::const_T / const_J are not
+                                //    stored per thread; kin_const_fill_kernel writes those rows as contiguous runs (KCFILL)
     std::string key() const;    // cache key of the option set
 };
 

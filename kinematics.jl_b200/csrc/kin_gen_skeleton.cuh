@@ -542,6 +542,41 @@ __device__ __forceinline__ void bulk_flush(real_ *gdst, real_ *&b0, real_ *&b1, 
 }
 #endif
 
+#if KCFILL
+// =====================================================================================================================
+// The SoA outputs that do not depend on the configuration (GenOptions::const_fill; for Fetch with the 8 arm joints 175
+// of the 348 rows of FK-all + gripper Jacobian).  Phase 1 does not store them (KST_* drops the components kcf_T / kcf_J
+// list at compile time); this kernel, launched right after kin_gen_kernel on the same stream, writes those KNCF rows,
+// columns [0, n), one 32-byte vector (STG.E.ENL2.256) per thread, one short-lived CTA per 256 vectors of a row
+// (blockIdx.y = row).  That shape fills at ~7.6 TB/s on B200; a fill inside the persistent kernel -- static split,
+// claimed pieces or slices between the tiles -- measured slower than storing the rows per thread (DESIGN 4.4).  CTA 0 of
+// a row also writes its scalar head / tail where the row does not start / end on a 32-byte boundary (batch_stride % 4
+// != 0, offset pointers, ragged n); padding columns (ld > n) are never touched.
+// =====================================================================================================================
+__device__ __forceinline__ void st_fill32(double *p, const double v) {
+    asm volatile("st.global.v4.f64 [%0], {%1, %1, %1, %1};" ::"l"(p), "d"(v) : "memory");
+}
+__device__ __forceinline__ void st_fill32(float *p, const float v) {
+    asm volatile("st.global.v8.f32 [%0], {%1, %1, %1, %1, %1, %1, %1, %1};" ::"l"(p), "f"(v) : "memory");
+}
+extern "C" __global__ void __launch_bounds__(256) kin_const_fill_kernel(const __grid_constant__ kin::GenArgs A) {
+    using namespace kin;
+    constexpr int E = 32 / (int)sizeof(real);
+    const int row = KCF_ROW[blockIdx.y];
+    const real v = KCF_VAL[blockIdx.y];
+    real *p = row >= 0 ? reinterpret_cast<real *>(A.T_out) + row * A.ld : reinterpret_cast<real *>(A.J_out) + (-1 - row) * A.ld;
+    const long long n = A.n;
+    const long long head = min(n, (long long)((32 - ((unsigned long long)p & 31)) & 31) / (long long)sizeof(real));
+    const long long body = (n - head) / E, tail = head + body * E;
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < body) st_fill32(p + head + j * E, v);
+    if (blockIdx.x == 0) {
+        if (threadIdx.x < head) p[threadIdx.x] = v;
+        if (tail + threadIdx.x < n) p[tail + threadIdx.x] = v;
+    }
+}
+#endif
+
 extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __grid_constant__ kin::GenArgs A) {
     using namespace kin;
     constexpr int BS = KBS;
@@ -683,13 +718,13 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
             #define KREC_BASE(rec) (KTILED ? (n >> 5) * ((long long)(rec) * 32) + (n & 31) : n)
 #if KWANT_T
             real *Tn = reinterpret_cast<real *>(A.T_out) + KREC_BASE(12 * KNFK);
-            #define KST_T(k, v) __stcs(Tn + KOFF(k), (v))
+            #define KST_T(k, v) do { if (!kcf_T(k)) __stcs(Tn + KOFF(k), (v)); } while (0)
 #else
             #define KST_T(k, v)
 #endif
 #if KWANT_J
             real *Jn = reinterpret_cast<real *>(A.J_out) + KREC_BASE(KROWS * KND * KNJAC);
-            #define KST_J(k, v) __stcs(Jn + KOFF(k), (v))
+            #define KST_J(k, v) do { if (!kcf_J(k)) __stcs(Jn + KOFF(k), (v)); } while (0)
 #else
             #define KST_J(k, v)
 #endif
