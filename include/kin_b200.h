@@ -106,6 +106,11 @@ typedef enum { KIN_PRIM_BOX = 0, KIN_PRIM_SPHERE = 1, KIN_PRIM_CYLINDER = 2 } Ki
 #define KIN_MAX_JOINTS 32          /* control joints (bitmask width), base columns excluded */
 #define KIN_MAX_SPHERES 512
 #define KIN_MAX_BOXES 128
+/* Self-collision pairs per model (kin_model_set_self_pairs).  The kernel does not stage the table: every lane of a warp
+ * loads the same 8-byte entry at the same time (one broadcast load through L1), so the table costs no shared memory and
+ * no occupancy.  4096 pairs are 32 KB, a table that stays resident in L1 beside the collision kernels' shared scratch,
+ * and hold every pair of 91 spheres -- several times the pair counts of the default policy on the models here. */
+#define KIN_MAX_SELF_PAIRS 4096
 
 typedef struct KinModel KinModel;
 
@@ -249,6 +254,28 @@ KIN_API int kin_collision(KinModel *model, int32_t precision, int32_t layout, co
  * lanes per configuration, warp-shuffle min / argmin / sum; SoA, tiled: one thread per configuration). */
 KIN_API int kin_collision_summary(KinModel *model, int32_t precision, int32_t layout, const void *q, int64_t n, double margin,
                                   void *dmin_out, int32_t *amin_out, void *cost_out, void *stream);
+
+/* Self-collision between the model's collision spheres (an EXTENSION: collision.jl has sphere-vs-environment only).
+ * The model holds a table of P sphere pairs (i, j).  Per configuration and pair p, with world centres c_i, c_j and radii
+ * r_i, r_j:
+ *   L = |c_i - c_j|,  d_p = L - r_i - r_j
+ *   grad_p[k] = u . (J_i[:,k] - J_j[:,k]),  u = (c_i - c_j) / L,  J_s = 3 x n_dof positional Jacobian of sphere s's centre
+ *               (zero in the columns that do not move s).  When L == 0 the gradient is 0.
+ *   truncation as collision.jl:84-86: d_p > truncation_dist -> value truncation_dist, gradient 0; then vals_offset is
+ *   subtracted from every written value (IneqConst's d - margin directly).
+ *   dmin[n] = min_p d_p (untruncated, no offset), amin[n] = 1-based index of the first pair attaining it, in table order.
+ * No box table is needed.  One kernel launch per call: phase 1 of kin_eval (FK, joint frames, sphere centres) followed by
+ * the pair loop, for every batch size, precision and layout. */
+/* replaces the model's self-collision pair table; pairs[n_pairs][2] = 1-based sphere ids, i != j, both <= n_spheres.
+ * n_pairs = 0 removes it.  kin_model_set_spheres removes it too (its ids would be stale); set_boxes / set_primitives keep it. */
+KIN_API int kin_model_set_self_pairs(KinModel *model, int32_t n_pairs, const int32_t *pairs);
+KIN_API int kin_model_n_self_pairs(const KinModel *model);
+/* vals_out: P per configuration; grads_out: (n_dof, P) column-major per configuration; dmin_out [N]; amin_out [N].
+ * Every output is nullable, but at least one of vals_out / dmin_out must be given.  Layout and precision as kin_collision
+ * (vals / grads in `layout`, dmin / amin plain [N] arrays; amin int32).  A call with dmin / amin only writes those. */
+KIN_API int kin_self_collision(KinModel *model, int32_t precision, int32_t layout, const void *q, int64_t n,
+                               double truncation_dist, double vals_offset, void *vals_out, void *grads_out,
+                               void *dmin_out, int32_t *amin_out, void *stream);
 
 /* BoxSDF / UnionSDF call and gradient! at arbitrary points (sdf.jl:34-41, 67-74, 108-119): for a
  * union of n_boxes boxes (HOST tables, same format as KinModelDesc), pts (DEVICE, N points x 3

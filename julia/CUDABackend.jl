@@ -28,6 +28,7 @@
 #   d = sdf_points(sdf, P); g = sdf_gradient(sdf, P)                    # sdf.jl:34-41,67-74,108-119 for (N, 3) points
 #   q, f, its, dmin = inverse_kinematics_batch(dm, link, targets, q0, joints; collision=true, margin=0.02)
 #                                                                       # inverse_kinematics.jl:1-30 for N targets at once
+#   set_self_pairs!(dm, pairs); v, g = compute_self_coll_dists_and_grads(dm, Q)   # self-collision (extension), (N, P)
 module CUDABackend
 
 using CUDA
@@ -351,6 +352,52 @@ function collision_summary(dm::DeviceMechanism, Q::CuMatrix{Float64}; layout::Sy
         (Ptr{Cvoid}, Cint, Cint, CuPtr{Cvoid}, Int64, Cdouble, CuPtr{Cvoid}, CuPtr{Cint}, CuPtr{Cvoid}, Ptr{Cvoid}),
         dm.handle, KIN_F64, layout_code(layout), pointer(Q), N, margin, pointer(dmin), pointer(amin), pointer(cost), cuda_stream()))
     return dmin, amin, cost
+end
+
+# Self-collision between the collision spheres (extension: collision.jl is sphere-vs-environment only).  The pair table
+# is explicit here: pairs (2, P), column p = 1-based sphere ids (i, j), i != j (the default policy -- no same-link, rigid
+# or adjacent pairs -- lives in the Python mirror's self_collision_pairs).  Replacing the sphere table drops it.
+function set_self_pairs!(dm::DeviceMechanism, pairs::Matrix{Cint})
+    @assert size(pairs, 1) == 2
+    GC.@preserve pairs check(ccall((:kin_model_set_self_pairs, libkin), Cint, (Ptr{Cvoid}, Cint, Ptr{Cint}),
+                                   dm.handle, size(pairs, 2), pointer(pairs)))
+end
+
+n_self_pairs(dm::DeviceMechanism) = Int(ccall((:kin_model_n_self_pairs, libkin), Cint, (Ptr{Cvoid},), dm.handle))
+
+function self_collision!(dm::DeviceMechanism, Q::CuMatrix{Float64}, layout::Symbol, truncation_dist, margin, vals, grads,
+                         dmin, amin)
+    vp(x) = x === nothing ? CuPtr{Cvoid}(0) : reinterpret(CuPtr{Cvoid}, pointer(x))
+    check(ccall((:kin_self_collision, libkin), Cint,
+        (Ptr{Cvoid}, Cint, Cint, CuPtr{Cvoid}, Int64, Cdouble, Cdouble, CuPtr{Cvoid}, CuPtr{Cvoid}, CuPtr{Cvoid}, CuPtr{Cint}, Ptr{Cvoid}),
+        dm.handle, KIN_F64, layout_code(layout), pointer(Q), nbatch(Q, layout), truncation_dist, margin, vp(vals), vp(grads),
+        vp(dmin), amin === nothing ? CuPtr{Cint}(0) : pointer(amin), cuda_stream()))
+end
+
+# d_p = |c_i - c_j| - r_i - r_j per pair: (N, P) / (P, N)
+function compute_self_coll_dists(dm::DeviceMechanism, Q::CuMatrix{Float64}; layout::Symbol=:soa)
+    vals = out_array(nbatch(Q, layout), layout, n_self_pairs(dm))
+    self_collision!(dm, Q, layout, Inf, 0.0, vals, nothing, nothing, nothing)
+    return vals
+end
+
+# ... and d d_p / d q = u' (J_i - J_j), u = (c_i - c_j) / |c_i - c_j| (0 when the centres coincide); d_p > truncation_dist
+# gives truncation_dist and a zero gradient, then margin is subtracted: (N, P), (N, n_dof, P) / (P, N), (n_dof, P, N)
+function compute_self_coll_dists_and_grads(dm::DeviceMechanism, Q::CuMatrix{Float64}; truncation_dist=Inf, margin=0.0,
+                                           layout::Symbol=:soa)
+    N, P = nbatch(Q, layout), n_self_pairs(dm)
+    vals = out_array(N, layout, P)
+    grads = out_array(N, layout, dm.n_dof, P)
+    self_collision!(dm, Q, layout, truncation_dist, margin, vals, grads, nothing, nothing)
+    return vals, grads
+end
+
+# the smallest untruncated d_p per configuration and the first pair attaining it (1-based): 12 bytes written per configuration
+function self_collision_summary(dm::DeviceMechanism, Q::CuMatrix{Float64}; layout::Symbol=:soa)
+    N = nbatch(Q, layout)
+    dmin = CuArray{Float64}(undef, N); amin = CuArray{Cint}(undef, N)
+    self_collision!(dm, Q, layout, Inf, 0.0, nothing, nothing, dmin, amin)
+    return dmin, amin
 end
 
 # sdf(p) and gradient!(sdf, p, out) (sdf.jl:34-41, 67-74, 108-119) for a batch of points P (N, 3) [SoA] / (3, N) [AoS]

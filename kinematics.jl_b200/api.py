@@ -11,10 +11,11 @@ from .load_urdf import parse_urdf
 from .algorithm import get_jacobian, get_jacobian_, get_transform
 from .sdf import BoxSDF, CylinderSDF, SphereSDF, UnionSDF
 from .collision import (SweptSphereCollisionChecker, add_coll_links, compute_coll_dists,
-                        compute_coll_dists_and_grads, compute_coll_summary)
+                        compute_coll_dists_and_grads, compute_coll_summary, compute_self_coll_dists,
+                        compute_self_coll_dists_and_grads, compute_self_coll_summary, self_collision_pairs)
 
 from .inverse_kinematics import ik_objective, ik_solve_device, inverse_kinematics, inverse_kinematics_batch
-from .planning import (ConfigurationConstraint, EqConst, IneqConst, Objective, PoseConstraint, construct_problem,
+from .planning import (ConfigurationConstraint, EqConst, IneqConst, Objective, PoseConstraint, SelfIneqConst, construct_problem,
                        create_straight_trajectory, gather_packed, gather_stacked, nloptize, plan_trajectory, pose_constraint, scipynize,
                        shard_range, smoothness_objective)
 from .lib import POSE_CONSTRAINT, POSE_IK_OBJECTIVE

@@ -8,7 +8,7 @@ import numpy as np
 
 from . import lib as _lib
 from .algorithm import _check_joints
-from .device import current_q, device_model, evaluate
+from .device import current_q, device_model, evaluate, evaluate_self
 from .mechanism import Link, Mechanism, SphereMetaData, add_new_link
 from .transform import Transform
 
@@ -106,3 +106,81 @@ def compute_coll_summary(sscc, joints, sdf, margin=0.0, dtype=None):
     if m._single:
         return float(dmin[0]), int(amin[0]), float(cost[0])
     return dmin, amin, cost
+
+
+# ---- self-collision between the checker's spheres (an extension: collision.jl is sphere-vs-environment only) ----
+def self_collision_pairs(sscc, joints, ignore=(), skip_adjacent=True):
+    """The default self-collision pair table of ``sscc`` under the control joints ``joints``: (P, 2) int32 1-based
+    sphere ids (i < j, in sphere order).  A pair of spheres is dropped when
+      * both sit on the same link;
+      * their links move rigidly together: they have the same nearest ancestor whose parent joint is in ``joints``
+        (or none), so their distance is constant -- leaving a joint out of ``joints`` merges the links around it;
+      * ``skip_adjacent``: one link is the parent of the other through a single joint (SRDF "Adjacent");
+      * the (unordered) pair of their link names is in ``ignore``."""
+    m = sscc.mech
+    ctrl = {j.id for j in joints}
+
+    def group(lid):                       # nearest controlled ancestor (the root when there is none)
+        l = m.links[lid - 1]
+        while l.plink_id != -1 and l.pjoint_id not in ctrl:
+            l = m.links[l.plink_id - 1]
+        return l.id
+
+    ignored = {frozenset(p) for p in ignore}
+    parents = list(sscc._parents)
+    groups = [group(l) for l in parents]
+    pairs = []
+    for i in range(len(parents)):
+        for j in range(i + 1, len(parents)):
+            li, lj = m.links[parents[i] - 1], m.links[parents[j] - 1]
+            if li.id == lj.id or groups[i] == groups[j]:
+                continue
+            if skip_adjacent and (li.plink_id == lj.id or lj.plink_id == li.id):
+                continue
+            if frozenset((li.name, lj.name)) in ignored:
+                continue
+            pairs.append((i + 1, j + 1))
+    return np.asarray(pairs, dtype=np.int32).reshape(-1, 2)
+
+
+def _prepare_self(sscc, joints, pairs):
+    m = sscc.mech
+    _check_joints(m, joints)
+    dm = device_model(m)
+    dm.set_spheres(sscc._parents, sscc._centers, sscc.sphere_radii)
+    dm.set_self_pairs(self_collision_pairs(sscc, joints) if pairs is None else pairs)
+    return m, dm
+
+
+def compute_self_coll_dists(sscc, joints, pairs=None, layout=None, dtype=None):
+    """Self-collision distances ``d_p = |c_i - c_j| - r_i - r_j`` of the sphere pairs (extension; ``kin_self_collision``;
+    ``pairs`` (P, 2) 1-based, default ``self_collision_pairs(sscc, joints)``).  single -> ndarray (P,); batch -> (N, P)."""
+    m, dm = _prepare_self(sscc, joints, pairs)
+    Q, ql, N = current_q(m, dtype)
+    vals = evaluate_self(dm, Q, ql, N, layout=layout)["vals"]
+    return vals[0].double().cpu().numpy() if m._single else vals
+
+
+def compute_self_coll_dists_and_grads(sscc, joints, pairs=None, truncation_dist=np.inf, vals_offset=0.0, layout=None,
+                                      dtype=None):
+    """... and their gradients ``u . (J_i - J_j)`` in q (0 where the centres coincide); ``d > truncation_dist`` gives
+    ``truncation_dist`` and a zero gradient (collision.jl:84-86), then ``vals_offset`` is subtracted.
+    single -> (vals (P,), grads (n_dof, P)); batch -> (N, P), (N, n_dof, P)."""
+    m, dm = _prepare_self(sscc, joints, pairs)
+    Q, ql, N = current_q(m, dtype)
+    out = evaluate_self(dm, Q, ql, N, layout=layout, with_grads=True, truncation_dist=truncation_dist,
+                        vals_offset=vals_offset)
+    if m._single:
+        return out["vals"][0].double().cpu().numpy(), out["grads"][0].double().cpu().numpy()
+    return out["vals"], out["grads"]
+
+
+def compute_self_coll_summary(sscc, joints, pairs=None, dtype=None):
+    """Per configuration the smallest self-collision distance and the pair attaining it (1-based, first minimum), without
+    materialising the P distances.  single -> (float, int); batch -> tensors (N,), (N,) int32."""
+    m, dm = _prepare_self(sscc, joints, pairs)
+    Q, ql, N = current_q(m, dtype)
+    out = evaluate_self(dm, Q, ql, N, with_vals=False, want_summary=True)
+    if m._single:
+        return float(out["dmin"][0]), int(out["amin"][0])
+    return out["dmin"], out["amin"]

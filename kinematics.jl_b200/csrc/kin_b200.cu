@@ -77,6 +77,17 @@ struct DeviceProgram {
     int block[2][3] = {{0, 0, 0}, {0, 0, 0}}, occ[2][3] = {{0, 0, 0}, {0, 0, 0}}, regs[2][3] = {{0, 0, 0}, {0, 0, 0}};
     int bs_index[2][3] = {{0, 0, 0}, {0, 0, 0}};
     size_t smem[2][3] = {{0, 0, 0}, {0, 0, 0}};
+    // the same for the self-collision kernels (kin_self_collision), configured on first use
+    int self_block[2][3] = {{0, 0, 0}, {0, 0, 0}}, self_occ[2][3] = {{0, 0, 0}, {0, 0, 0}}, self_bs_index[2][3] = {{0, 0, 0}, {0, 0, 0}};
+    size_t self_smem[2][3] = {{0, 0, 0}, {0, 0, 0}};
+};
+
+// A model's self-collision pair table on its device (kin_model_set_self_pairs): 0-based sphere ids.  Reference-counted
+// like the programs, so that a launch keeps the table it was given alive while the table is replaced.
+struct DevicePairs {
+    int2 *d = nullptr;
+    int n = 0;
+    ~DevicePairs() { cudaFree(d); }
 };
 
 struct HostStage {          // resources of kin_eval_host, created on first use
@@ -98,6 +109,7 @@ struct KinModel {
     // programs are reference-counted: a launch keeps its program alive even if kin_model_set_spheres /
     // kin_model_set_boxes on another thread drops the cache entry meanwhile
     std::map<std::vector<int>, std::shared_ptr<DeviceProgram>> cache;
+    std::shared_ptr<DevicePairs> self_pairs;   // null: no pair table
     HostStage stage;
 };
 
@@ -205,6 +217,12 @@ const int kBS[kNumBS] = {128, 96, 64, 32};
 const KernelFn kKernels[2][3][kNumBS][2][2] = {{KIN_BS_ROW(double, 0), KIN_BS_ROW(double, 1), KIN_BS_ROW(double, 2)},
                                                {KIN_BS_ROW(float, 0), KIN_BS_ROW(float, 1), KIN_BS_ROW(float, 2)}};
 
+// self-collision instances (kin_self_collision): [precision][layout][block size][joint frames in registers]
+#define KIN_KS(real, lay, bs) {kin::kin_eval_kernel<real, lay, bs, true, 0, true>, kin::kin_eval_kernel<real, lay, bs, true, kin::JF_REGS, true>}
+#define KIN_BS_ROW_S(real, lay) {KIN_KS(real, lay, 128), KIN_KS(real, lay, 96), KIN_KS(real, lay, 64), KIN_KS(real, lay, 32)}
+const KernelFn kSelfKernels[2][3][kNumBS][2] = {{KIN_BS_ROW_S(double, 0), KIN_BS_ROW_S(double, 1), KIN_BS_ROW_S(double, 2)},
+                                                {KIN_BS_ROW_S(float, 0), KIN_BS_ROW_S(float, 1), KIN_BS_ROW_S(float, 2)}};
+
 // Warp-specialised fused kernel (kin_kernels_ws.cuh): FP64, SoA / tiled, collision, <= 8 columns, a chain without
 // save slots, ring fits in shared memory, and a batch large enough to fill one 384-thread CTA per SM a few times.
 // [layout: SoA, tiled][planar base][collision-only call: the producer also does the box search]
@@ -239,7 +257,7 @@ bool ws_eligible(const KinModel *m, const KinCall *c, const DeviceProgram *dp) {
     return kin::ws_smem_bytes(h, false) <= (size_t)m->dev_smem;
 }
 
-int configure(KinModel *m, DeviceProgram *dp, int pi, int li) {
+int configure(KinModel *m, DeviceProgram *dp, int pi, int li, bool self = false) {
     const kin::ProgHeader &h = dp->prog.h;
     const int coll = h.n_sph > 0 ? 1 : 0, jr = (coll && h.n_dof <= kin::JF_REGS) ? 1 : 0;
     const size_t rs = pi ? sizeof(float) : sizeof(double);
@@ -255,13 +273,18 @@ int configure(KinModel *m, DeviceProgram *dp, int pi, int li) {
         size_t smem = tab + rs * (size_t)h.n_slots * b;
         if (li == KIN_LAYOUT_AOS) smem += rs * (size_t)kin::AOS_STAGE_REALS * (b / 32);   // warp-private staging
         if (smem > (size_t)dev_smem) continue;
-        KernelFn k = kKernels[pi][li][bi][coll][jr];
+        KernelFn k = self ? kSelfKernels[pi][li][bi][jr] : kKernels[pi][li][bi][coll][jr];
         CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, dev_smem));
         int occ = 0;
         CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, b, smem));
         if (occ * b > best_threads) { best = bi; best_threads = occ * b; best_occ = occ; best_smem = smem; }
     }
     if (best < 0) return fail(KIN_ERR_LIMIT, "model does not fit the shared-memory scratch of one CTA");
+    if (self) {
+        dp->self_block[pi][li] = kBS[best]; dp->self_bs_index[pi][li] = best; dp->self_occ[pi][li] = best_occ;
+        dp->self_smem[pi][li] = best_smem;
+        return KIN_OK;
+    }
     cudaFuncAttributes fa;
     CUDA_TRY(cudaFuncGetAttributes(&fa, kKernels[pi][li][best][coll][jr]));
     dp->block[pi][li] = kBS[best]; dp->bs_index[pi][li] = best; dp->occ[pi][li] = best_occ; dp->smem[pi][li] = best_smem;
@@ -850,7 +873,7 @@ int kin_model_set_spheres(KinModel *m, int32_t n, const int32_t *link, const dou
     DeviceGuard guard(m->device);
     std::lock_guard<std::mutex> lock(m->mu);
     int rc = load_spheres(m->hm, n, link, center, radius);
-    if (rc == KIN_OK) clear_cache(m);
+    if (rc == KIN_OK) { clear_cache(m); m->self_pairs.reset(); }     // the pair table's sphere ids would be stale
     return rc;
 }
 
@@ -880,6 +903,32 @@ int kin_model_set_primitives(KinModel *m, int32_t n, const int32_t *kinds, const
     }
     return KIN_OK;
 }
+
+int kin_model_set_self_pairs(KinModel *m, int32_t n_pairs, const int32_t *pairs) {
+    if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
+    if (n_pairs < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative n_pairs");
+    if (n_pairs > KIN_MAX_SELF_PAIRS) return fail(KIN_ERR_LIMIT, "n_pairs exceeds KIN_MAX_SELF_PAIRS");
+    if (n_pairs > 0 && !pairs) return fail(KIN_ERR_INVALID_ARGUMENT, "null pair table");
+    DeviceGuard guard(m->device);
+    std::lock_guard<std::mutex> lock(m->mu);
+    const int S = m->hm.n_sph;
+    std::vector<int2> host(n_pairs);
+    for (int p = 0; p < n_pairs; ++p) {      // validate before touching the model: a failed call leaves it unchanged
+        const int i = pairs[2 * p], j = pairs[2 * p + 1];
+        if (i < 1 || i > S || j < 1 || j > S) return fail(KIN_ERR_INVALID_ARGUMENT, "self-collision pair: sphere id out of range");
+        if (i == j) return fail(KIN_ERR_INVALID_ARGUMENT, "self-collision pair: a sphere paired with itself");
+        host[p] = make_int2(i - 1, j - 1);
+    }
+    if (n_pairs == 0) { m->self_pairs.reset(); return KIN_OK; }
+    auto dp = std::make_shared<DevicePairs>();
+    CUDA_TRY(cudaMalloc(&dp->d, sizeof(int2) * host.size()));
+    CUDA_TRY(cudaMemcpy(dp->d, host.data(), sizeof(int2) * host.size(), cudaMemcpyHostToDevice));
+    dp->n = n_pairs;
+    m->self_pairs = dp;
+    return KIN_OK;
+}
+
+int kin_model_n_self_pairs(const KinModel *m) { return m && m->self_pairs ? m->self_pairs->n : 0; }
 
 int kin_model_n_dof(const KinModel *m) { return m ? m->hm.n_dof() : 0; }
 int kin_model_n_spheres(const KinModel *m) { return m ? m->hm.n_sph : 0; }
@@ -1748,6 +1797,60 @@ int kin_collision(KinModel *m, int32_t precision, int32_t layout, const void *q,
     c.truncation_dist = truncation_dist; c.grad_mode = grad_mode; c.scratch_mode = scratch_mode;
     c.vals_out = vals_out; c.grads_out = grads_out; c.argmin_out = argmin_out; c.stream = stream;
     return kin_eval(m, &c);
+}
+
+int kin_self_collision(KinModel *m, int32_t precision, int32_t layout, const void *q, int64_t n, double truncation_dist,
+                       double vals_offset, void *vals_out, void *grads_out, void *dmin_out, int32_t *amin_out, void *stream) {
+    if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
+    if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
+    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS && layout != KIN_LAYOUT_TILED32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
+    if (n < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative batch size");
+    if (n > 0 && !q) return fail(KIN_ERR_INVALID_ARGUMENT, "q is null");
+    if (!vals_out && !dmin_out) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: neither vals_out nor dmin_out given");
+    if (grads_out && !vals_out) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: grads_out needs vals_out");
+    if (std::isnan(truncation_dist)) return fail(KIN_ERR_INVALID_ARGUMENT, "truncation_dist is NaN");
+    DeviceGuard guard(m->device);
+    std::shared_ptr<DevicePairs> pairs;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        pairs = m->self_pairs;
+    }
+    if (!pairs) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: the model has no pair table (kin_model_set_self_pairs)");
+    if (n == 0) return KIN_OK;
+    // phase 1 of a collision call computes the sphere centres and joint frames: the self-collision kernels run the
+    // program of a plain collision call (no links requested, clean scratch); only the pointer's presence matters
+    KinCall c;
+    std::memset(&c, 0, sizeof c);
+    c.precision = precision; c.layout = layout; c.n = n; c.q = q;
+    c.vals_out = vals_out ? vals_out : dmin_out; c.scratch_mode = KIN_SCRATCH_CLEAN;
+    std::shared_ptr<DeviceProgram> dp;
+    int rc = get_program(m, &c, dp);
+    if (rc != KIN_OK) return rc;
+    const int pi = precision == KIN_F32 ? 1 : 0, li = layout;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        if (dp->self_block[pi][li] == 0 && (rc = configure(m, dp.get(), pi, li, true)) != KIN_OK) return rc;
+    }
+    kin::KernelArgs a;
+    std::memset(&a, 0, sizeof a);
+    a.h = dp->prog.h;
+    a.tab_i = dp->d_int;
+    a.tab_r = pi ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
+    a.q = q;
+    a.vals_out = vals_out; a.grads_out = grads_out;
+    a.n = n; a.ld = n;
+    a.truncation_dist = truncation_dist; a.vals_offset = vals_offset;
+    a.self_pairs = pairs->d; a.n_self_pairs = pairs->n;
+    a.dmin_out = dmin_out; a.amin_out = amin_out;
+    const int block = dp->self_block[pi][li];
+    const long long tiles = (n + block - 1) / block;
+    long long grid = (long long)dp->self_occ[pi][li] * m->n_sm;
+    if (grid > tiles) grid = tiles;
+    const int jr = dp->prog.h.n_dof <= kin::JF_REGS ? 1 : 0;
+    kSelfKernels[pi][li][dp->self_bs_index[pi][li]][jr]<<<(unsigned)grid, block, dp->self_smem[pi][li], (cudaStream_t)stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    g_launches.fetch_add(1);
+    return KIN_OK;
 }
 
 }  // extern "C"

@@ -52,6 +52,11 @@ struct KernelArgs {
     int grad_mode, scratch_ref;  // scratch_ref = 1: reproduce the reference's shared Jacobian scratch
     double truncation_dist, vals_offset;
     void *ws_ring;               // kin_eval_ws_kernel only: global hand-over ring (kin_kernels_ws.cuh)
+    // self-collision instances only (SELF = true); appended so that the fields above keep their offsets
+    const int2 *self_pairs;      // [n_self_pairs] 0-based sphere ids (i, j), read with warp-uniform loads through L1
+    void *dmin_out;              // [n] min over pairs of the untruncated distance, nullable
+    int32_t *amin_out;           // [n] 1-based pair index of the first minimum, nullable
+    int n_self_pairs;
 };
 
 // AoS layout only.  A thread owns one record, so a plain store of component k by 32 lanes hits 32
@@ -86,7 +91,9 @@ __device__ __forceinline__ void warp_store_records(real *stage, real *rec0, size
 // of 64 threads, 2 warps per sub-partition) may use up to 255 registers per thread, while a 9th warp
 // would cap every thread at 168 and spill.  With the frames in registers the collision kernel is
 // therefore built for 4 x 64 threads per SM.
-template <typename real, int LAY, int BS, bool COLL, int JR>
+// SELF (with COLL; kin_self_collision, an extension): phase 1 as for a collision call (sphere centres, joint frames),
+// then the self-collision phase over the model's pair table instead of phase 2.
+template <typename real, int LAY, int BS, bool COLL, int JR, bool SELF = false>
 __global__ void __launch_bounds__(BS, (JR > 0 && COLL) ? (BS == 64 ? 4 : BS == 128 ? 2 : BS == 32 ? 8 : 2) : 1)
 kin_eval_kernel(const __grid_constant__ KernelArgs A) {
     // LAY: 0 = SoA (x[comp * ld + n]), 1 = AoS (x[n * rec + comp]), 2 = tiled (AoSoA-32:
@@ -359,7 +366,7 @@ kin_eval_kernel(const __grid_constant__ KernelArgs A) {
         }
 
         // =========================== phase 2 ===========================
-        if (COLL) {
+        if (COLL && !SELF) {
             __syncthreads();
             const bool want_grads = A.grads_out != nullptr;
             const bool stale = want_grads && A.scratch_ref;
@@ -494,6 +501,87 @@ kin_eval_kernel(const __grid_constant__ KernelArgs A) {
                     Gp += (size_t)ND * es;      // (a pointer bumped inside the loop is live across its early exit: two extra moves per column)
                 }
             }
+        }
+
+        // ===================== self-collision phase (extension) =====================
+        // Pair p = (i, j) of the model's table: L = |c_i - c_j|, d = L - r_i - r_j; gradient column k =
+        // u . (J_i[:,k] - J_j[:,k]) with u = (c_i - c_j) / L (0 when L == 0).  A column that moves both spheres moves
+        // them rigidly together, so its two terms cancel exactly: only the columns of mask_i XOR mask_j are evaluated,
+        // the others are written as 0.  Truncation and offset as phase 2; (dmin, amin) over the untruncated d.
+        if constexpr (SELF) {
+            const int P = A.n_self_pairs;
+            const real trunc = (real)A.truncation_dist, voff = (real)A.vals_offset;
+            real *Vp = A.vals_out ? reinterpret_cast<real *>(A.vals_out) + rec_base(n, P) : nullptr;
+            real *Gp = A.grads_out ? reinterpret_cast<real *>(A.grads_out) + rec_base(n, (long long)ND * P) : nullptr;
+            real best = CUDART_INF;
+            int bi = 0;
+            #pragma unroll 1
+            for (int p = 0; p < P; ++p) {
+                const int2 pr = __ldg(A.self_pairs + p);          // the same address in every lane: one broadcast load
+                KIN_DASSERT(pr.x >= 0 && pr.x < S && pr.y >= 0 && pr.y < S && pr.x != pr.y);
+                const real *ci = &SCR(so_cent + 3 * pr.x), *cj = &SCR(so_cent + 3 * pr.y);
+                const real xi = ci[0], yi = ci[BS], zi = ci[2 * BS], xj = cj[0], yj = cj[BS], zj = cj[2 * BS];
+                const real dx = xi - xj, dy = yi - yj, dz = zi - zj;
+                const real L = sqrt_(fma_(dx, dx, fma_(dy, dy, dz * dz)));
+                const real d = L - tr[ro_sph + pr.x * SPH_REALS + 3] - tr[ro_sph + pr.y * SPH_REALS + 3];
+                if (d < best) { best = d; bi = p; }
+                if (!Vp) continue;
+                const bool truncated = d > trunc;
+                *Vp = (truncated ? trunc : d) - voff;
+                Vp += es;
+                if (!Gp) continue;
+                const unsigned mi = (unsigned)ti[io_sph_mask + pr.x], mj = (unsigned)ti[io_sph_mask + pr.y];
+                const unsigned mx = (truncated || !(L > real(0))) ? 0u : (mi ^ mj);
+                const real inv = mx ? real(1) / L : real(0);
+                const real ux = dx * inv, uy = dy * inv, uz = dz * inv;
+                // column j of this pair's gradient; the frame of j comes from registers (jfr, j static) or scratch
+                auto column = [&](const JFrame<real> &f, int j) -> real {
+                    const bool on_i = (mi >> j) & 1u;
+                    real cx, cy, cz;
+                    jac_col(f, (rev_mask >> j) & 1u, on_i ? xi : xj, on_i ? yi : yj, on_i ? zi : zj, cx, cy, cz);
+                    const real g = fma_(ux, cx, fma_(uy, cy, uz * cz));
+                    return on_i ? g : -g;
+                };
+                if (AOS) {
+                    // the ND values of this pair are contiguous in the configuration's record: staged in chunks of
+                    // AOS_STAGE_ROWS columns and written by the whole warp (control flow is warp-uniform up to here)
+                    const size_t rec = (size_t)ND * P;
+                    for (int k0 = 0; k0 < (JR > 0 ? 1 : ND); k0 += AOS_STAGE_ROWS) {
+                        real gv[AOS_STAGE_ROWS];
+                        #pragma unroll
+                        for (int kk = 0; kk < AOS_STAGE_ROWS; ++kk) {
+                            const int j = JR > 0 ? kk : k0 + kk;
+                            gv[kk] = real(0);
+                            if (j < ND && ((mx >> j) & 1u)) {
+                                JFrame<real> f;
+                                if (JR > 0) f = jfr[kk < (JR > 0 ? JR : 1) ? kk : 0];
+                                else {
+                                    const real *jf = jf0 + 6 * BS * j;
+                                    f.o[0] = jf[0]; f.o[1] = jf[BS]; f.o[2] = jf[2 * BS];
+                                    f.a[0] = jf[3 * BS]; f.a[1] = jf[4 * BS]; f.a[2] = jf[5 * BS];
+                                }
+                                gv[kk] = column(f, j);
+                            }
+                        }
+                        warp_store_records<real, AOS_STAGE_ROWS>(stage, reinterpret_cast<real *>(A.grads_out) + n_w0 * rec + (size_t)p * ND + k0,
+                                                                 rec, gv, min(AOS_STAGE_ROWS, ND - k0), lane, n_valid);
+                    }
+                    continue;
+                }
+                const real *jf = jf0;
+                FOR_COLUMNS(j) {
+                    real g = real(0);
+                    if ((mx >> j) & 1u) {
+                        JF_LOAD(f, j, jf)
+                        g = column(f, j);
+                    }
+                    Gp[(size_t)j * es] = g;
+                    jf += 6 * BS;
+                }
+                Gp += (size_t)ND * es;
+            }
+            if (A.dmin_out) reinterpret_cast<real *>(A.dmin_out)[n] = best;
+            if (A.amin_out) A.amin_out[n] = bi + 1;
         }
     }
     #undef SCR

@@ -76,8 +76,8 @@ class DeviceModel:
         self.h = h
         self.n_dof = len(ctrl_ids) + (3 if m.with_base else 0)
         self.n_links = len(m.links)
-        self._sph_sig = self._box_sig = None
-        self.n_spheres = self.n_boxes = 0
+        self._sph_sig = self._box_sig = self._pair_sig = None
+        self.n_spheres = self.n_boxes = self.n_self_pairs = 0
 
     def __del__(self):
         try:
@@ -95,6 +95,15 @@ class DeviceModel:
         if sig != self._sph_sig:
             _lib.check(_lib.lib().kin_model_set_spheres(self.h, len(links), _iptr(links), _dptr(centers), _dptr(radii)))
             self._sph_sig, self.n_spheres = sig, len(links)
+            self._pair_sig, self.n_self_pairs = None, 0         # the library dropped the pair table with the old spheres
+
+    def set_self_pairs(self, pairs):
+        """Self-collision pair table: (P, 2) 1-based sphere ids (``kin_model_set_self_pairs``)."""
+        pairs = np.ascontiguousarray(np.asarray(pairs, dtype=np.int32).reshape(-1, 2))
+        sig = pairs.tobytes()
+        if sig != self._pair_sig:
+            _lib.check(_lib.lib().kin_model_set_self_pairs(self.h, len(pairs), _iptr(pairs)))
+            self._pair_sig, self.n_self_pairs = sig, len(pairs)
 
     def set_boxes(self, poses, widths, kinds=None):
         poses = np.ascontiguousarray(np.asarray(poses, dtype=np.float64).reshape(-1, 4, 4).transpose(0, 2, 1)).reshape(-1, 16)
@@ -265,4 +274,47 @@ def evaluate(dm: DeviceModel, Q, q_layout, N, *, layout=None, fk_links=None, jac
         regs, smem, block, grid = C.c_int32(), C.c_int32(), C.c_int32(), C.c_int32()
         _lib.check(_lib.lib().kin_query_launch(dm.h, C.byref(c), C.byref(regs), C.byref(smem), C.byref(block), C.byref(grid)))
         out["launch"] = {"regs": regs.value, "smem_bytes": smem.value, "block": block.value, "grid": grid.value}
+    return out
+
+
+def evaluate_self(dm: DeviceModel, Q, q_layout, N, *, layout=None, with_vals=True, with_grads=False,
+                  truncation_dist=np.inf, vals_offset=0.0, want_summary=False, stream=None):
+    """One ``kin_self_collision`` over the model's pair table.  vals / grads are allocated in the layout of the call
+    (default: the layout of Q) and returned as batch-first views vals (N, P), grads (N, n_dof, P); dmin (N,) and
+    amin (N,) int32 are plain arrays."""
+    import torch
+    layout = q_layout if layout is None else layout
+    tiled = layout == _lib.TILED32
+    if tiled:
+        Q = tile32(Q.contiguous() if q_layout == _lib.AOS else Q)
+    elif layout != q_layout:
+        Q = Q.t().contiguous().t() if layout == _lib.SOA else Q.contiguous()
+    dt, dev, nd, P = Q.dtype, Q.device, dm.n_dof, dm.n_self_pairs
+    NT = (N + 31) // 32
+
+    def alloc(shape_soa, shape_aos):
+        if tiled:
+            return torch.empty((NT,) + tuple(shape_soa[:-1]) + (32,), dtype=dt, device=dev)
+        return torch.empty(shape_soa if layout == _lib.SOA else shape_aos, dtype=dt, device=dev)
+
+    def view(x, perm_soa, perm_aos):
+        if tiled:
+            return untile32(x, N).permute(0, *[p + 1 for p in perm_soa[1:]])
+        return x.permute(*perm_soa) if layout == _lib.SOA else x.permute(*perm_aos)
+
+    V = alloc((P, N), (N, P)) if with_vals else None
+    G = alloc((P, nd, N), (N, P, nd)) if with_grads else None
+    dmin = torch.empty(N, dtype=dt, device=dev) if want_summary else None
+    amin = torch.empty(N, dtype=torch.int32, device=dev) if want_summary else None
+    ptr = lambda t: None if t is None else t.data_ptr()
+    _lib.check(_lib.lib().kin_self_collision(dm.h, _lib.F32 if dt == torch.float32 else _lib.F64, layout, Q.data_ptr(), N,
+                                             float(truncation_dist), float(vals_offset), ptr(V), ptr(G), ptr(dmin), ptr(amin),
+                                             torch.cuda.current_stream(dev).cuda_stream if stream is None else stream))
+    out = {}
+    if V is not None:
+        out["vals"] = view(V, (1, 0), (0, 1))
+    if G is not None:
+        out["grads"] = view(G, (2, 1, 0), (0, 2, 1))
+    if want_summary:
+        out["dmin"], out["amin"] = dmin, amin
     return out

@@ -65,7 +65,8 @@ EXPORTS = ["kin_last_error", "kin_abi_version", "kin_build_id", "kin_debug_build
            "kin_model_set_boxes", "kin_model_set_primitives", "kin_sdf_points_prims", "kin_collision_summary", "kin_model_n_dof", "kin_model_n_spheres", "kin_model_n_boxes", "kin_eval",
            "kin_eval_host", "kin_fk_links", "kin_fk_jacobian", "kin_collision", "kin_launch_count",
            "kin_query_launch", "kin_sdf_points", "kin_program_dump", "kin_pose_residual", "kin_pose_residual_multi", "kin_probe_fp64",
-           "kin_jit_status", "kin_jit_stats", "kin_codegen_dump", "kin_ik_solve", "kin_host_transfer_bytes"]
+           "kin_jit_status", "kin_jit_stats", "kin_codegen_dump", "kin_ik_solve", "kin_host_transfer_bytes",
+           "kin_model_set_self_pairs", "kin_model_n_self_pairs", "kin_self_collision"]
 
 
 def source_files():
@@ -206,6 +207,10 @@ def lib():
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.kin_collision_summary.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_double, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kin_model_set_self_pairs.argtypes = [C.c_void_p, C.c_int32, _ip]
+        L.kin_model_n_self_pairs.argtypes = [C.c_void_p]
+        L.kin_self_collision.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_double, C.c_double,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.kin_pose_residual.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p,
                                         C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
         L.kin_pose_residual_multi.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, _ip, _ip,

@@ -8,7 +8,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import lib as _lib
-from .collision import compute_coll_dists_and_grads
+from .collision import compute_coll_dists_and_grads, compute_self_coll_dists_and_grads, self_collision_pairs
 from .mechanism import set_joint_angles
 
 
@@ -82,6 +82,38 @@ class IneqConst:
         for i in range(self.n_wp):
             J[i * self.n_dof:(i + 1) * self.n_dof, i * self.n_coll:(i + 1) * self.n_coll] = blocks[i]
         return J
+
+
+class SelfIneqConst:
+    """The self-collision counterpart of ``IneqConst`` (extension): per waypoint ``val = self dists - margin`` over a
+    pair table (default ``self_collision_pairs(sscc, joints)``), truncated at ``margin + 0.05`` like ``IneqConst``, with
+    the same ``(vals, blocks)`` contract; ``n_coll`` is the number of pairs."""
+
+    def __init__(self, sscc, joints, n_wp, margin, pairs=None):
+        self.sscc, self.joints = sscc, list(joints)
+        self.pairs = self_collision_pairs(sscc, joints) if pairs is None else np.asarray(pairs, dtype=np.int32).reshape(-1, 2)
+        self.n_wp, self.margin = int(n_wp), float(margin)
+        self.n_dof = len(joints) + (3 if sscc.mech.with_base else 0)
+        self.n_coll = len(self.pairs)
+        self.n_cons = self.n_coll * self.n_wp
+
+    def __call__(self, xi):
+        """xi: flat (n_dof * n_wp,) -> numpy (val_vec (n_cons,), blocks (n_wp, n_dof, n_coll)); CUDA tensor
+        (P, n_wp, n_dof) -> tensors (P, n_wp, n_coll), (P, n_wp, n_dof, n_coll)."""
+        import torch
+        single = not (isinstance(xi, torch.Tensor) and xi.dim() == 3)
+        X = torch.as_tensor(np.asarray(xi, dtype=np.float64).reshape(1, self.n_wp, self.n_dof), device="cuda") if single else xi
+        P = X.shape[0]
+        set_joint_angles(self.sscc.mech, self.joints, X.reshape(P * self.n_wp, self.n_dof))
+        vals, grads = compute_self_coll_dists_and_grads(self.sscc, self.joints, self.pairs, truncation_dist=self.margin + 0.05,
+                                                        vals_offset=self.margin, layout=_lib.SOA)
+        vals = vals.reshape(P, self.n_wp, self.n_coll)
+        grads = grads.reshape(P, self.n_wp, self.n_dof, self.n_coll)
+        if single:
+            return vals[0].reshape(-1).cpu().numpy(), grads[0].cpu().numpy()
+        return vals, grads
+
+    dense = IneqConst.dense
 
 
 def nloptize(cons):
@@ -228,7 +260,7 @@ def scipynize(obj):
         key = np.asarray(xi, dtype=np.float64).tobytes()
         if cache.get("key") != key:
             val, jac = obj(xi)
-            if isinstance(obj, IneqConst):
+            if isinstance(obj, (IneqConst, SelfIneqConst)):
                 jac = obj.dense(jac)
             cache.update(key=key, val=val, jac=jac)
         return cache["val"], cache["jac"]
@@ -242,14 +274,16 @@ def construct_problem(sscc, joints, sdf, q_start, q_goal, n_wp, n_dof, margin, p
 
 
 def plan_trajectory(sscc, joints, sdf, q_start, q_goal, n_wp, margin=2e-2, partial_consts=(), ftol_abs=1e-3,
-                    solver="SCIPY"):
+                    solver="SCIPY", self_margin=None):
     """planning.jl:332-401.  The three back-ends of the reference are third-party solvers; of them only scipy is
     installed here, and it is the reference's own ``solver=:SCIPY`` path (:388-394) that is reproduced: SLSQP with
     the scipynize'd objective, inequality (collision) and equality (start / goal / pose) constraints.  Every
     constraint evaluation -- n_wp waypoints per SLSQP iteration -- is one batched GPU call.  (NLopt's LD_SLSQP, the
     default of the reference, is the same algorithm; its joint-limit bounds are passed to scipy as well.)
+    ``self_margin`` (extension): also keep every default self-collision pair (``self_collision_pairs``) at least this far
+    apart -- a ``SelfIneqConst`` as a second inequality constraint; start / goal must then be free of self-collision too.
     Returns (q_seq (n_wp, n_dof), scipy result)."""
-    from .collision import compute_coll_dists
+    from .collision import compute_coll_dists, compute_self_coll_dists
     m = sscc.mech
     n_dof = len(joints) + (3 if m.with_base else 0)
     q_start, q_goal = np.asarray(q_start, dtype=np.float64), np.asarray(q_goal, dtype=np.float64)
@@ -257,6 +291,8 @@ def plan_trajectory(sscc, joints, sdf, q_start, q_goal, n_wp, margin=2e-2, parti
     for q in (q_start, q_goal):                                        # planning.jl:349-353
         set_joint_angles(m, joints, q)
         assert np.all(compute_coll_dists(sscc, joints, sdf) > 0.0), "start / goal configuration is in collision"
+        if self_margin is not None:
+            assert np.all(compute_self_coll_dists(sscc, joints) > 0.0), "start / goal configuration is in self-collision"
     xi_init = create_straight_trajectory(q_start, q_goal, n_wp)
     F, G, H, n_whole = construct_problem(sscc, joints, sdf, q_start, q_goal, n_wp, n_dof, margin, partial_consts)
     if solver != "SCIPY":
@@ -269,8 +305,12 @@ def plan_trajectory(sscc, joints, sdf, q_start, q_goal, n_wp, margin=2e-2, parti
     f, df = scipynize(F)
     g, dg = scipynize(G)
     h, dh = scipynize(H)
+    constraints = [{"type": "ineq", "fun": g, "jac": dg}, {"type": "eq", "fun": h, "jac": dh}]
+    if self_margin is not None:
+        gs, dgs = scipynize(SelfIneqConst(sscc, joints, n_wp, self_margin))
+        constraints.insert(1, {"type": "ineq", "fun": gs, "jac": dgs})
     ret = minimize(f, xi_init, jac=df, method="SLSQP", bounds=bounds, options={"ftol": ftol_abs, "maxiter": 200},
-                   constraints=[{"type": "ineq", "fun": g, "jac": dg}, {"type": "eq", "fun": h, "jac": dh}])
+                   constraints=constraints)
     return ret.x.reshape(n_wp, n_dof), ret
 
 
