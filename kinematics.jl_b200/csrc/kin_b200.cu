@@ -56,7 +56,8 @@ struct JitKernel {
     cudaKernel_t kern = nullptr;
     bool ok = false, from_cache = false;
     int regs = 0, block = 0, occ = 0, slots = 0, smem_limit = 0;
-    bool cooperative = false;       // grid-wide barrier inside (input batching): launched cooperatively
+    bool sched = false;             // claimed tiles: a zeroed tile counter per launch
+    bool cooperative = false;       // AoS input batching: a grid-wide barrier inside, launched cooperatively
     cudaKernel_t fill = nullptr;    // const_fill: the kernel writing the configuration-independent rows (KNCF of them)
     int fill_rows = 0;
     double compile_ms = 0;
@@ -364,7 +365,7 @@ int validate_call(const KinModel *m, const KinCall *c) {
 constexpr long long kJitMinBatch = 32 * 1024;      // below this the compile is not worth it: interpreting kernels ...
 constexpr long long kWarpMaxBatch = 2048;          // ... except for smaller batches that keep coming (a solver loop): after
 constexpr int kSmallCallsBeforeJit = 4;            // this many calls of the same program its specialised kernel is built
-constexpr long long kQbatchMinBatch = 1 << 18;     // input batching (grid-wide barriers) only pays for long launches
+constexpr long long kSchedMinBatch = 1 << 18;      // claimed tiles + L2 epochs + constant-row fill: from this batch size on
 
 long long env_ll(const char *name, long long dflt) {
     const char *e = std::getenv(name);
@@ -408,12 +409,12 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     //                     (the warps of a CTA then share instruction fetches: the fused kernel is 90 KB of code, far
     //                     beyond the instruction cache) and 32-bit component strides: 3.68 -> 3.13
     //   collision, tiled: 256 threads x 1 CTA/SM, no barriers: 3.11
-    //   FK / Jacobian only: 128 threads x 1 CTA/SM + input batching (below)
+    //   FK / Jacobian only: 128 threads, as many CTAs/SM as the registers allow (2), claimed tiles (below)
     const bool tiled = c->layout == KIN_LAYOUT_TILED32;
     // small batches: one warp per configuration (kin_gen_skeleton.cuh, KWARP)
     o.warp = use_warp_kernel(c, h) ? 1 : 0;
     if (o.warp) {
-        o.block = 128; o.min_blocks = 1; o.qbatch = 0; o.ksync = 0; o.es32 = 0; o.fd_cold = 0;
+        o.block = 128; o.min_blocks = 1; o.ksync = 0; o.es32 = 0; o.fd_cold = 0;
         o.grad_mode = o.want_grads ? c->grad_mode : -1;
         return o;
     }
@@ -466,36 +467,34 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     // 2^24 configurations, FK-all + Jacobian: 7.67 -> 7.61 ms (0.950 -> 0.959 of the HBM peak), 8.36 -> 8.05 without the input
     // batching (profiles/sweep_bulk.py): the write path, not the store instructions, bounds the kernel -- a small gain
     o.bulk = (tiled && !o.coll && !o.keep_irrelevant && (o.want_T || o.want_J)) ? (int)env_ll("KIN_JIT_BULK", 1) : 0;
-    o.qbatch = 0;
-    // input batching (kin_gen_skeleton.cuh): the FK / Jacobian-only kernels are bound by the DRAM write path and use
-    // no other shared memory, so the configurations of as many tiles as fit twice in ~200 KB are fetched per batch
-    // behind a grid-wide barrier (one CTA per SM, cooperative launch)
-    if (h.n_dof > 0 && !std::getenv("KIN_JIT_NO_QBATCH")) {
+    // FK / Jacobian-only kernels, bound by the DRAM write path: tiles claimed from a counter, the inputs of an epoch of
+    // tiles prefetched into L2 in one burst (kin_gen_skeleton.cuh, KSCHED; measurements: DESIGN 4.4, profiles/ab_sched.py).
+    // A call that writes little per configuration (the gripper transform + its Jacobian: 480 B) is not write-bound:
+    // plain loads, static tiles, 3 CTAs/SM (sweep_jit.py fkg).  Below kSchedMinBatch the static tiles are kept as well,
+    // without the constant-row fill and its second launch (profiles/ab_sched.py --sizes).
+    // KIN_JIT_EPOCH_MB / KIN_JIT_PF_DIST / KIN_JIT_SCHED_MIN_N: sweep knobs.
+    if (h.n_dof > 0 && !o.coll && c->n >= env_ll("KIN_JIT_SCHED_MIN_N", kSchedMinBatch)) {
         const size_t rs = o.precision ? sizeof(float) : sizeof(double);
-        size_t budget = std::min<size_t>((size_t)(m ? m->dev_smem : 227 * 1024), 200 * 1024);
-        if (o.layout == KIN_LAYOUT_AOS) budget -= std::min<size_t>(budget, 24 * 1024);     // room for the output stages
-        if (o.bulk) budget -= std::min<size_t>(budget, (size_t)o.block * 24 * rs);         // two [12][32] stages per warp
-        // measured (profiles/sweep_jit.py, 2^24 configurations): 128 threads x 12 tiles per batch, one CTA per SM:
-        // 8.72 -> 7.78 ms (0.84 -> 0.94 of the HBM peak); the collision kernels need their shared memory for the
-        // per-configuration scratch and are not write-bound: no batching there unless asked for (KIN_JIT_QBATCH_COLL)
-        long long qb = (long long)(budget / (2 * (size_t)h.n_dof * o.block * rs));
-        qb = std::min<long long>(qb, 16);
-        // ... and a call that writes little per configuration (the gripper transform + its Jacobian: 480 B) is not
-        // write-bound either: plain loads, 3 CTAs/SM: 1.76 -> 1.68 ms per 2^24, tiled 1.84 -> 1.62 (sweep_jit.py fkg)
         const size_t out_bytes = rs * ((o.want_T ? (size_t)12 * h.n_fk : 0) + (o.want_J ? (size_t)(o.with_rot ? 6 : 3) * h.n_dof * h.n_jac : 0));
-        if (out_bytes < 1024) qb = 0;
-        // ... nor is a short launch: the grid-wide barriers cost more than they save below 2^18 configurations
-        // (profiles/sweep_qbatch_min.py, fk + jac: 2^16: 42.7 us with / 36.8 without; 2^17: 70.2 / 68.5; 2^18: 130.7 / 134.3;
-        // 2^20: 486 / 541; 2^23: 3843 / 4413)
-        if (c->n < env_ll("KIN_JIT_QBATCH_MIN_N", kQbatchMinBatch)) qb = 0;
-        qb = o.coll ? env_ll("KIN_JIT_QBATCH_COLL", 0) : env_ll("KIN_JIT_QBATCH", qb);
-        if (qb >= 1 && (qb >= 2 || o.coll)) { o.qbatch = (int)qb; o.min_blocks = 1; }
+        // AoS: the claimed tiles measured slower than the input batches (2^22 configurations: 2.44 against 1.89 ms,
+        // DESIGN 4.4), so that layout keeps them: the configurations of as many tiles as fit twice in ~176 KB fetched
+        // per batch with cp.async, behind a grid-wide barrier (one CTA per SM, cooperative launch)
+        const long long qb = std::min<long long>(16, (long long)((std::min<size_t>((size_t)(m ? m->dev_smem : 227 * 1024), 200 * 1024) - 24 * 1024) /
+                                                                 (2 * (size_t)h.n_dof * o.block * rs)));
+        if (out_bytes >= 1024 && o.layout == KIN_LAYOUT_AOS && qb >= 2) {
+            o.qbatch = (int)qb;
+            o.min_blocks = 1;
+        } else if (out_bytes >= 1024) {
+            o.sched = 1;
+            o.epoch = (int)std::max<long long>(1, (env_ll("KIN_JIT_EPOCH_MB", 8) << 20) / ((long long)o.block * h.n_dof * rs));
+            o.pf_dist = (int)env_ll("KIN_JIT_PF_DIST", 1);
+        }
     }
     // ... whose rows that do not depend on the configuration (175 of the 348 of FK-all + gripper Jacobian for Fetch) are
     // then written by a second, fill-shaped kernel instead of one store per configuration (kin_gen_skeleton.cuh:
     // kin_const_fill_kernel; DESIGN 4.4).  SoA only: a constant row is one contiguous run there, not in the tiled / AoS
     // layouts.  (KIN_JIT_CONST_FILL=0 stores every row per thread, for A/B measurements.)
-    if (o.layout == KIN_LAYOUT_SOA && o.qbatch > 0 && !o.coll && (o.want_T || o.want_J))
+    if (o.layout == KIN_LAYOUT_SOA && o.sched && (o.want_T || o.want_J))
         o.const_fill = (int)env_ll("KIN_JIT_CONST_FILL", 1) ? 1 : 0;
     return o;
 }
@@ -601,6 +600,7 @@ std::shared_ptr<JitKernel> get_jit_with(KinModel *m, DeviceProgram *dp, const ki
     }
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&k->occ, (const void *)k->kern, k->block, smem);
     if (e != cudaSuccess || k->occ < 1) { k->log = "occupancy query failed"; cudaGetLastError(); g_jit_failures.fetch_add(1); return nullptr; }
+    k->sched = o.sched != 0;
     k->cooperative = o.qbatch > 0;
     k->fill_rows = g.config.find("#define KCFILL 1") != std::string::npos ? (int)(g.const_T.size() + g.const_J.size()) : 0;
     if (k->fill_rows > 0 && cudaLibraryGetKernel(&k->fill, k->lib, "kin_const_fill_kernel") != cudaSuccess) {
@@ -634,7 +634,16 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
     if (o.warp) grid = (c->n + k.block / 32 - 1) / (k.block / 32);        // one warp per configuration, not persistent
     if (grid < 1) return KIN_OK;
     void *args[] = {&a};
-    if (k.cooperative) {
+    if (k.sched) {
+        // a zero-initialised tile counter per launch (stream-ordered, so concurrent launches have their own)
+        unsigned *next = nullptr;
+        CUDA_TRY(cudaMallocFromPoolAsync((void **)&next, sizeof(unsigned), m->pool, stream));
+        a.tile_next = next;
+        cudaError_t e = cudaMemsetAsync(next, 0, sizeof(unsigned), stream);
+        if (e == cudaSuccess) e = cudaLaunchKernel((const void *)k.kern, dim3((unsigned)grid), dim3((unsigned)k.block), args, jit_smem(o, h, k), stream);
+        cudaFreeAsync(next, stream);
+        if (e != cudaSuccess) return fail_cuda(e, "launching the specialised kernel");
+    } else if (k.cooperative) {
         // two zero-initialised barrier words per launch (stream-ordered, so concurrent launches have their own)
         unsigned *sync = nullptr;
         CUDA_TRY(cudaMallocFromPoolAsync((void **)&sync, 2 * sizeof(unsigned), m->pool, stream));
@@ -774,7 +783,7 @@ int kin_codegen_dump(const KinModelDesc *d, const KinCall *c, int32_t compile, c
     if (!kin::compile_program(hm, fk, jac, want_coll, want_stale, kin::JF_REGS, dp.prog, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
     kin::GenOptions o = gen_options(nullptr, c, &dp);
     if (std::getenv("KIN_DUMP_IK")) {          // development aid: the batched-IK kernel of this link instead
-        o.ik = 1; o.rpy_jac = o.with_rot; o.qbatch = 0; o.ksync = 0; o.coll = false; o.block = 128; o.min_blocks = 1;
+        o.ik = 1; o.rpy_jac = o.with_rot; o.ksync = 0; o.coll = false; o.block = 128; o.min_blocks = 1;
     }
     kin::GenSource g;
     if (!kin::generate_source(dp.prog, o, g, err)) return fail(KIN_ERR_INVALID_ARGUMENT, "codegen: " + err);

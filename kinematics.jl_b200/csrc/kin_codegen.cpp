@@ -11,8 +11,8 @@ namespace kin {
 
 std::string GenOptions::key() const {
     char b[200];
-    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d", precision, layout, (int)want_T, (int)want_J,
-                  (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, (int)ws, block, min_blocks, qbatch,
+    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d S%d.%d.%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d", precision, layout, (int)want_T, (int)want_J,
+                  (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, (int)ws, block, min_blocks, qbatch, sched, epoch, pf_dist,
                   ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min, const_fill);
     return b;
 }
@@ -419,6 +419,8 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
       << "\n#define KTILED " << (o.layout == 2 ? 1 : 0) << "\n#define KAOS " << (o.layout == 1 ? 1 : 0) << "\n#define KWS " << (o.ws ? 1 : 0) << "\n";
     c << "#define KBS " << o.block << "\n#define KMINB " << o.min_blocks << "\n#define KWARP " << o.warp << "\n#define KIK " << o.ik << "\n#define KQB " << o.qbatch << "\n#define KSYNC_ON "
       << o.ksync << "\n#define KES32 " << o.es32 << "\n";
+    const bool sched = o.sched && !o.coll && !o.warp && !o.ik && !o.ws;
+    c << "#define KSCHED " << (sched ? 1 : 0) << "\n#define KEPOCH " << (sched ? std::max(1, o.epoch) : 1) << "\n#define KPFD " << (sched ? o.pf_dist : 0) << "\n";
     // the configuration-independent outputs as a table of rows (kin_gen_skeleton.cuh: kin_const_fill_kernel): component (T: k,
     // J: -1 - k) and value, written as the literals phase 1 stores -- the outputs keep their bits, sign of zero included
     // -- and, for the store macros, which components the table holds.  Phase 1 keeps every KST_* line (kin_eval_host and

@@ -32,7 +32,10 @@ struct GenOptions {
     bool want_grads = false, want_argmin = false, stale = false;
     bool ws = false;            // warp-specialised skeleton (producer = phase 1, consumers = phase 2)
     int block = 128, min_blocks = 1;
-    int qbatch = 0;             // > 0: tiles per input batch (cp.async into shared memory behind a grid-wide barrier)
+    int qbatch = 0;             // > 0 (AoS): tiles per input batch (cp.async into shared memory behind a grid-wide barrier)
+    int sched = 0;              // 1: FK / Jacobian only: tiles claimed from a counter, inputs prefetched into L2 one epoch at a time
+    int epoch = 0;              //    sched: tiles per epoch
+    int pf_dist = 0;            //    sched: epochs the L2 prefetch runs ahead (0: none)
     int warp = 0;               // 1: small-batch kernel, one WARP per configuration (lane = sphere in phase 2)
     int ik = 0;                 // 1: the batched Levenberg-Marquardt IK kernel around phase 1 (one link: T + rpy-Jacobian)
     int grad_mode = -1;         // >= 0: the gradient mode as a compile-time constant (only that code path is compiled in)

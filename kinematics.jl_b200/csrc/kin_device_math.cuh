@@ -433,6 +433,7 @@ struct GenArgs {
     int32_t *argmin_out;
     const void *boxes;           // device: n_box rows of BOX_REALS reals (rewritten in place by kin_model_set_boxes)
     void *ws_ring;               // warp-specialised variant: global hand-over ring
+    unsigned *tile_next;         // claimed tiles (KSCHED): the tile counter, zeroed before every launch
     unsigned *sync;              // input batching (KQB > 0): two zero-initialised words of the grid-wide barrier
     long long n, ld;
     int n_box, grad_mode;

@@ -215,17 +215,24 @@ __device__ __forceinline__ void phase2b_group(const int s0, const int ge, const 
 // =====================================================================================================================
 // Monolithic kernel: phase 1 and phase 2 in the same thread.
 // Dynamic shared memory: [box table n_box * BOX_REALS][radii KS] then the per-thread scratch [slot][thread]:
-//   3 KS sphere-centre coordinates, 3 KND stale-Jacobian columns (KSTALE), 2 SPH_GROUP hand-over slots;
-// then (KQB > 0) the input batches [2][KQB][KND][BS].
+//   3 KS sphere-centre coordinates, 3 KND stale-Jacobian columns (KSTALE), 2 SPH_GROUP hand-over slots.
 //
-// KQB > 0: INPUT BATCHING.  The kernels are bound by the DRAM write path (2784 B of results per configuration against
-// 64 B of input), and on HBM3e a trickle of small reads in the middle of a saturated write stream is disproportionately
-// expensive: a store-only kernel with this output pattern sustains 6.05 TB/s, the same kernel reading its 8 inputs per
-// thread 5.22 TB/s (profiles/probe_store.cu) -- every read interrupts the write drain of the channels it touches.
-// So the configurations of KQB tiles per CTA are fetched at once with cp.async into shared memory, one batch ahead
-// (double buffered), and ALL CTAs issue the fetch of a batch at the same moment, behind a grid-wide barrier: the DRAM
-// sees one read burst per batch (about every 100 us) instead of 4 reads per microsecond.  The probe recovers 5.93 TB/s
-// that way.  The grid is launched cooperatively (all CTAs resident), the barrier words live in A.sync.
+// KSCHED: CLAIMED TILES, INPUTS STAGED THROUGH L2 IN ONE BURST PER EPOCH (the FK / Jacobian-only kernels).  They are bound
+// by the DRAM write path (2784 B of results per configuration against 64 B of input), and on HBM3e a trickle of small
+// reads in the middle of a saturated write stream is disproportionately expensive (a store-only probe with this output
+// pattern sustains 6.05 TB/s, the same probe reading its 8 inputs per thread 5.22 TB/s; profiles/probe_store.cu): every
+// read interrupts the write drain of the channels it touches.  So the reads are clustered in time without lock-stepping
+// the grid: the tiles are taken in ascending order (CTA b starts with the tiles b and b + grid, then claims 2 grid,
+// 2 grid + 1, ... from the counter A.tile_next), in epochs of KEPOCH tiles; whoever takes tile t with t mod KEPOCH < P
+// (P = min(grid, KEPOCH)) issues piece t mod KEPOCH of epoch t / KEPOCH + KPFD -- one cp.async.bulk.prefetch.L2 of that
+// piece's tiles per input row (SoA) or of its one contiguous block (tiled, AoS), evict_last -- so the q of a whole
+// epoch enters L2 in one burst, KPFD epochs ahead, and the per-thread loads hit L2.  No grid-wide barrier, no
+// cooperative launch: an SM whose writes drain faster takes more tiles (DESIGN 4.4).
+//
+// KQB > 0 (AoS, where the claimed tiles measured slower): INPUT BATCHING.  The configurations of KQB tiles per CTA are
+// fetched at once with cp.async into shared memory ([2][KQB][KND][BS] after the output stages), one batch ahead, and ALL
+// CTAs issue the fetch of a batch at the same moment, behind a grid-wide barrier: one read burst per batch.  The grid
+// is launched cooperatively (all CTAs resident), the barrier words live in A.sync.
 // =====================================================================================================================
 #if KIK
 // =====================================================================================================================
@@ -517,6 +524,32 @@ __device__ __forceinline__ void kin_grid_barrier(unsigned *sync, unsigned n_cta)
     __syncthreads();
 }
 #endif
+#if KSCHED
+// bytes [lo, hi) of q into L2, evict_last; the 16-byte-aligned part only (the size of a bulk copy is a multiple of 16 and
+// nothing outside q is touched), the few bytes at the ends are left to the loads
+__device__ __forceinline__ void l2_prefetch(const void *lo, const void *hi, const unsigned long long pol) {
+    const unsigned long long a = ((unsigned long long)lo + 15) & ~15ull, b = (unsigned long long)hi & ~15ull;
+    if (b > a) asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(a), "r"((unsigned)(b - a)), "l"(pol) : "memory");
+}
+// piece p of epoch e: tiles [e E + p E / P, e E + (p + 1) E / P), configurations below n only
+__device__ __forceinline__ void prefetch_piece(const kin::GenArgs &A, const long long n_tiles, const long long e, const int p, const int P) {
+    using namespace kin;
+    const long long t0 = e * KEPOCH + (long long)p * KEPOCH / P, t1 = min(n_tiles, e * KEPOCH + (long long)(p + 1) * KEPOCH / P);
+    if (t0 >= t1) return;
+    const long long c0 = t0 * KBS, c1 = min(t1 * KBS, A.n);
+    const real *q = reinterpret_cast<const real *>(A.q);
+    unsigned long long pol;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+    if (KAOS) {
+        l2_prefetch(q + c0 * KND, q + c1 * KND, pol);
+    } else if (KTILED) {
+        l2_prefetch(q + (c0 >> 5) * (KND * 32), q + ((c1 - 1) >> 5) * (KND * 32) + (KND - 1) * 32 + ((c1 - 1) & 31) + 1, pol);
+    } else {
+        #pragma unroll 1
+        for (int c = 0; c < KND; ++c) l2_prefetch(q + c * A.ld + c0, q + c * A.ld + c1, pol);
+    }
+}
+#endif
 
 #if KBULK
 // ---- tiled layout, FK / Jacobian-only kernels: outputs leave through the TMA engine.  In the tiled layout the
@@ -632,7 +665,45 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
         const long long n_ = min(tile_ * BS + tid, (long long)A.n - 1);
         return reinterpret_cast<const real *>(A.q) + (KAOS ? n_ * KND : KTILED ? (n_ >> 5) * ((long long)KND * 32) + (n_ & 31) : n_);
     };
-#if KQB > 0
+#if KSCHED
+    // claimed tiles (see above): tile is computed, the inputs of tile_nxt are loaded meanwhile, and thread 0 claims the
+    // one after (claim_s[i & 1], read by every thread after the barrier that ends tile i)
+    __shared__ long long claim_s[2];
+    const int pf_pieces = min((int)gridDim.x, KEPOCH);
+    long long tile = blockIdx.x, tile_nxt = tile + gridDim.x;
+    auto took = [&](const long long t) {
+        if (KPFD > 0 && t < n_tiles && t % KEPOCH < pf_pieces) prefetch_piece(A, n_tiles, t / KEPOCH + KPFD, (int)(t % KEPOCH), pf_pieces);
+    };
+    if (tid == 0) {
+        if (KPFD > 0 && (int)blockIdx.x < pf_pieces) {
+            #pragma unroll 1
+            for (int e = 0; e < KPFD; ++e) prefetch_piece(A, n_tiles, e, blockIdx.x, pf_pieces);
+        }
+        took(tile);
+        took(tile_nxt);
+    }
+    real qcur[KND > 0 ? KND : 1];
+    if (tile < n_tiles) {
+        const real *qp = q_ptr(tile);
+        #pragma unroll
+        for (int c = 0; c < KND; ++c) qcur[c] = KAOS ? __ldg(qp + c) : __ldcs(qp + (size_t)c * es);
+    }
+    {
+        #pragma unroll 1
+        for (int claim_i = 0; tile < n_tiles; ++claim_i) {
+            if (tid == 0) {
+                const long long t = 2ll * gridDim.x + atomicAdd(A.tile_next, 1u);
+                claim_s[claim_i & 1] = t;
+                took(t);
+            }
+            real qnxt[KND > 0 ? KND : 1];
+            {
+                const real *qp = q_ptr(tile_nxt < n_tiles ? tile_nxt : tile);
+                #pragma unroll
+                for (int c = 0; c < KND; ++c) qnxt[c] = KAOS ? __ldg(qp + c) : __ldcs(qp + (size_t)c * es);
+            }
+            #define KQ(c) qcur[c]
+#elif KQB > 0
     real *sq = smem_next;                                     // [2][KQB][KND][BS]
     const long long my_tiles = (long long)blockIdx.x < n_tiles ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     const long long max_tiles = (n_tiles + gridDim.x - 1) / gridDim.x, max_batches = (max_tiles + KQB - 1) / KQB;
@@ -762,7 +833,15 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
 #include "kin_gen_phase2.inc"
 #endif
             }
-#if KQB > 0
+#if KSCHED
+            __syncthreads();
+            tile = tile_nxt;
+            tile_nxt = claim_s[claim_i & 1];
+            #pragma unroll
+            for (int c = 0; c < KND; ++c) qcur[c] = qnxt[c];
+        }
+    }
+#elif KQB > 0
         }
         __syncthreads();                                      // the batch buffer is refilled two iterations later
     }

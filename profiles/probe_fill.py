@@ -3,7 +3,9 @@
 Runs, in one process tree on one GPU: the card's name / power limit / max SM clock (nvidia-smi, read-only), torch.fill_
 of 8 GiB (the 7.5 TB/s figure of probe_write_bw.py), then `probe_store fill` (contiguous 8 GiB fills with each store
 form, and the 348-row SoA pattern at 2^22 configurations with its 175 constant rows as contiguous fills), then torch.fill_
-again.  Usage: python profiles/probe_fill.py [rounds]"""
+again.  `python profiles/probe_fill.py sched [rounds]` instead runs `probe_store sched`: the 173 varying rows under the
+static / barrier schedule against claimed tiles with and without epoch L2 prefetches, and short-lived CTAs (DESIGN 4.4).
+Usage: python profiles/probe_fill.py [sched] [rounds]"""
 import os
 import shutil
 import subprocess
@@ -37,7 +39,11 @@ def torch_fill(rounds):
 
 
 def main():
-    rounds = int(sys.argv[1]) if len(sys.argv) > 1 else 7
+    args = sys.argv[1:]
+    sched = bool(args) and args[0] == "sched"
+    if sched:
+        args = args[1:]
+    rounds = int(args[0]) if args else 7
     print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv"],
                          capture_output=True, text=True).stdout, flush=True)
     with tempfile.TemporaryDirectory() as tmp:
@@ -45,6 +51,9 @@ def main():
         nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
         subprocess.check_call([nvcc, "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-o", exe,
                                os.path.join(HERE, "probe_store.cu")])
+        if sched:
+            subprocess.check_call([exe, "sched", str(rounds)])
+            return
         torch_fill(rounds)
         subprocess.check_call([exe, "fill", str(rounds)])
         torch_fill(rounds)

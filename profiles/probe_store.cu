@@ -16,6 +16,7 @@
 #include <cstring>
 #include <algorithm>
 #include <functional>
+#include <string>
 #include <vector>
 
 #define CK(x) do { cudaError_t e = (x); if (e != cudaSuccess) { printf("CUDA error %s at %s:%d\n", cudaGetErrorString(e), __FILE__, __LINE__); exit(1); } } while (0)
@@ -464,6 +465,83 @@ __global__ void __launch_bounds__(BS) k_mix(double *x, const double *q, long lon
     }
 }
 
+// ---- schedule section (`probe_store sched`): k_mix MODE 3 (the 173 varying rows, 8 SoA inputs per thread) with the
+//      grid-wide barrier replaced by tiles claimed from a counter, and the input reads clustered by bulk L2 prefetches.
+// A CTA starts with the tiles b and b + grid and then claims 2 grid, 2 grid + 1, ... from g_tile_next (zeroed before
+// every launch), one tile ahead of the one whose inputs it loads into registers, which is one tile ahead of the one it
+// computes.  Epoch prefetch (D > 0): tiles are taken in ascending order, in epochs of E tiles; whoever takes tile t
+// with t mod E < P issues piece t mod E of epoch t / E + D: cp.async.bulk.prefetch.L2 of that piece's tile range in
+// each of the 8 rows of q, evict_last; the CTAs b < P prefetch piece b of the epochs 0 .. D - 1 first.
+__device__ unsigned g_tile_next = 0;
+__device__ __forceinline__ void prefetch_piece(const double *q, long long N, long long n_tiles, long long e, int p, int E, int P) {
+    const long long t0 = e * E + (long long)p * E / P, t1 = min(n_tiles, e * E + (long long)(p + 1) * E / P);
+    if (t0 >= t1) return;
+    unsigned long long pol;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+    #pragma unroll
+    for (int c = 0; c < 8; ++c)
+        asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(q + (long long)c * N + t0 * BS),
+                     "r"((unsigned)((t1 - t0) * BS * 8)), "l"(pol) : "memory");
+}
+__device__ __forceinline__ void took_tile(const double *q, long long N, long long n_tiles, long long t, int E, int D, int P) {
+    if (D > 0 && t < n_tiles && t % E < P) prefetch_piece(q, N, n_tiles, t / E + D, (int)(t % E), E, P);
+}
+template <bool CS>
+__device__ __forceinline__ void mix_varying_rows(double *x, long long N, long long n, double v) {
+    double *p = x + n;
+    #pragma unroll
+    for (int c = 0; c < REC; ++c)
+        if (!mix_const(c)) { if (CS) __stcs(p + (size_t)c * N, v + c); else p[(size_t)c * N] = v + c; }
+}
+// (b) D = 0 / (c) D > 0: persistent CTAs, claimed tiles
+template <bool CS> __global__ void __launch_bounds__(BS) k_sched(double *x, const double *q, long long N, int E, int D, int P) {
+    __shared__ long long s_claim[2];
+    const long long n_tiles = N / BS;
+    long long cur = blockIdx.x, nxt = blockIdx.x + gridDim.x;
+    if (threadIdx.x == 0) {
+        if (D > 0 && (int)blockIdx.x < P)
+            for (int e = 0; e < D; ++e) prefetch_piece(q, N, n_tiles, e, blockIdx.x, E, P);
+        took_tile(q, N, n_tiles, cur, E, D, P);
+        took_tile(q, N, n_tiles, nxt, E, D, P);
+    }
+    double qc[8], qn[8];
+    #pragma unroll
+    for (int c = 0; c < 8; ++c) qc[c] = cur < n_tiles ? __ldcs(q + (long long)c * N + cur * BS + threadIdx.x) : 0.0;
+    for (int k = 0; cur < n_tiles; ++k) {
+        if (threadIdx.x == 0) {
+            const long long t = 2ll * gridDim.x + atomicAdd(&g_tile_next, 1u);
+            s_claim[k & 1] = t;
+            took_tile(q, N, n_tiles, t, E, D, P);
+        }
+        const long long tn = nxt < n_tiles ? nxt : cur;
+        #pragma unroll
+        for (int c = 0; c < 8; ++c) qn[c] = __ldcs(q + (long long)c * N + tn * BS + threadIdx.x);
+        const long long n = cur * BS + threadIdx.x;
+        double v = (double)n;
+        #pragma unroll
+        for (int c = 0; c < 8; ++c) v += qc[c];
+        mix_varying_rows<CS>(x, N, n, v);
+        __syncthreads();
+        cur = nxt; nxt = s_claim[k & 1];
+        #pragma unroll
+        for (int c = 0; c < 8; ++c) qc[c] = qn[c];
+    }
+}
+// (d) short-lived CTAs: one tile per CTA, the hardware schedules them (in ascending order); P = pieces per epoch
+template <bool CS> __global__ void __launch_bounds__(BS) k_sched_np(double *x, const double *q, long long N, int E, int D, int P) {
+    const long long n_tiles = N / BS, t = blockIdx.x;
+    if (threadIdx.x == 0) {
+        if (D > 0 && (int)blockIdx.x < P)
+            for (int e = 0; e < D; ++e) prefetch_piece(q, N, n_tiles, e, blockIdx.x, E, P);
+        took_tile(q, N, n_tiles, t, E, D, P);
+    }
+    const long long n = t * BS + threadIdx.x;
+    double v = (double)n;
+    #pragma unroll
+    for (int c = 0; c < 8; ++c) v += __ldcs(q + (long long)c * N + n);
+    mix_varying_rows<CS>(x, N, n, v);
+}
+
 template <typename F> float timeit(F launch, int reps) {
     cudaEvent_t a, b;
     CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b));
@@ -558,8 +636,71 @@ int fill_main(int rounds) {
     return 0;
 }
 
+// `probe_store sched [rounds]`: the 173 varying rows of the mix (k_mix MODE 3) at 2^22 and 2^24 configurations under
+// each schedule, at several CTA shapes and epoch sizes (q of an epoch 4 / 8 / 16 MB), prefetch distance D = 0 (control:
+// claimed tiles, no prefetch), 1, 2.  GB/s counts the varying rows' bytes plus q.
+int sched_main(int rounds) {
+    int n_sm; CK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, 0));
+    const long long NMAX = 1ll << 24, RT = 12;
+    double *x, *q;
+    CK(cudaMalloc(&x, (size_t)NMAX * REC * 8));
+    CK(cudaMalloc(&q, (size_t)NMAX * 8 * 8));
+    CK(cudaMemset(q, 0, (size_t)NMAX * 8 * 8));
+    {
+        int rows[175];
+        for (int c = 0, k = 0; c < REC; ++c) if (mix_const(c)) rows[k++] = c;
+        CK(cudaMemcpyToSymbol(c_const_rows, rows, sizeof rows));
+    }
+    unsigned *d_tile;
+    CK(cudaGetSymbolAddress((void **)&d_tile, g_tile_next));
+    const size_t smem = (size_t)2 * RT * 8 * BS * 8;
+    CK(cudaFuncSetAttribute(k_mix<3, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(cudaFuncSetAttribute(k_mix<3, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    struct V { std::string name; double gb; std::function<void()> run; std::vector<float> ms; };
+    std::vector<V> vs;
+    for (int lg : {22, 24}) {
+        const long long N = 1ll << lg, n_tiles = N / BS;
+        const double gb = (N * 173 * 8 + N * 64) / 1e9;
+        char nm[128];
+        snprintf(nm, sizeof nm, "2^%d (a) static + smem batches + grid barrier", lg);
+        vs.push_back({nm, gb, [=] { k_mix<3, 8, false><<<n_sm, BS, smem>>>(x, q, N, (int)RT); }, {}});
+        snprintf(nm, sizeof nm, "2^%d (a) ... , .cs stores", lg);
+        vs.push_back({nm, gb, [=] { k_mix<3, 8, true><<<n_sm, BS, smem>>>(x, q, N, (int)RT); }, {}});
+        for (int occ : {1, 2, 4}) {
+            const int g = n_sm * occ;
+            for (int mb : {4, 8, 16}) {
+                const int E = (int)((mb << 20) / (BS * 64));
+                for (int D : {0, 1, 2}) {
+                    if (D == 0 && mb != 8) continue;               // the control does not depend on E
+                    snprintf(nm, sizeof nm, "2^%d (%s) claimed, %d/SM, %2d MB epochs, D=%d", lg, D ? "c" : "b", occ, mb, D);
+                    vs.push_back({nm, gb, [=] { cudaMemsetAsync(d_tile, 0, 4); k_sched<true><<<g, BS>>>(x, q, N, E, D, std::min(g, E)); }, {}});
+                }
+            }
+        }
+        for (int mb : {4, 8, 16})
+            for (int D : {0, 1, 2}) {
+                if (D == 0 && mb != 8) continue;
+                const int E = (int)((mb << 20) / (BS * 64)), P = std::min(n_sm * 4, E);
+                snprintf(nm, sizeof nm, "2^%d (d) short-lived, %2d MB epochs, D=%d", lg, mb, D);
+                vs.push_back({nm, gb, [=] { k_sched_np<true><<<(unsigned)n_tiles, BS>>>(x, q, N, E, D, P); }, {}});
+            }
+    }
+    for (int r = 0; r < rounds; ++r)
+        for (auto &v : vs) v.ms.push_back(timeit(v.run, 5));
+    printf("%-56s %9s %9s %9s %9s   (%d rounds of 5 launches each, variants alternating)\n", "variant", "med ms", "min ms", "max ms", "med GB/s", rounds);
+    for (auto &v : vs) {
+        std::vector<float> s = v.ms;
+        std::sort(s.begin(), s.end());
+        const float med = s[s.size() / 2];
+        printf("%-56s %9.4f %9.4f %9.4f %9.1f\n", v.name.c_str(), med, s.front(), s.back(), v.gb / (med * 1e-3));
+    }
+    CK(cudaFree(x)); CK(cudaFree(q));
+    return 0;
+}
+
 int main(int argc, char **argv) {
     if (argc > 1 && !strcmp(argv[1], "fill")) return fill_main(argc > 2 ? atoi(argv[2]) : 7);
+    if (argc > 1 && !strcmp(argv[1], "sched")) return sched_main(argc > 2 ? atoi(argv[2]) : 7);
     const long long N = argc > 1 ? atoll(argv[1]) : (1ll << 22);
     const long long total = N * REC;
     double *x;
