@@ -362,6 +362,20 @@ typedef struct {
     void *dmin_out;            /* DEVICE [n], nullable: min over spheres of the UNtruncated signed distance at q_out */
 } KinIkCall;
 KIN_API int kin_ik_solve(KinModel *model, const KinIkCall *call);
+/* kin_ik_solve with the extra hard constraint d_p(q) - self_margin >= 0 for every pair p of the model's self-collision
+ * table (kin_model_set_self_pairs; d_p as kin_self_collision).  Everything else as kin_ik_solve with the AL loop:
+ * with call->collision != 0 the sphere-vs-box constraint applies too; with call->collision == 0 only the pairs do,
+ * and the model needs spheres + a pair table but no boxes.  self_dmin_out: DEVICE [n], nullable: min over pairs of
+ * the untruncated d_p at q_out.
+ * Per iteration: kin_eval (pose, + spheres with collision), ONE kin_self_collision launch over the same active list
+ * (pair values and gradients, truncated at self_margin + 0.05), the step kernel; the pairs share the penalty parameter
+ * coll_weight with the spheres, and a problem stops when f < ftol and every sphere and pair holds to ctol.  The
+ * constraint-free pose-only solve is never used here.  Errors, before anything is launched: no pair table or a NaN
+ * self_margin (KIN_ERR_INVALID_ARGUMENT), collision != 0 without spheres / boxes (as kin_ik_solve), n_dof > 20
+ * (KIN_ERR_LIMIT).  Workspace: on top of kin_ik_solve's, P (n_dof + 2) * 8 bytes of stream-ordered scratch per problem
+ * (pair values, gradients and multipliers) -- 23.2 KB on a model of 18 columns and 145 pairs, i.e. 6.1 GB at 2^18
+ * problems and 24.3 GB at 2^20; a pool allocation that fails is returned as KIN_ERR_CUDA. */
+KIN_API int kin_ik_solve_self(KinModel *model, const KinIkCall *call, double self_margin, void *self_dmin_out);
 
 /* Diagnostics for bench.py / tests: kernel launches issued by this library since load, and the
  * static resources of the kernel a call would use (registers / thread, dynamic shared memory bytes /

@@ -326,21 +326,29 @@ pose_constraint(dm::DeviceMechanism, links::Vector{<:Link}, Q::CuMatrix{Float64}
 # for the spheres / boxes the DeviceMechanism was created with, from the warm start q0 (pass the result of a
 # collision=false solve for the reference's two-stage scheme, :8-13).  Returns (q (n_dof, N), f (N,), iterations (N,),
 # dmin (N,) -- the smallest signed sphere distance at q; all zeros without collision).
+# self_margin (extension, kin_ik_solve_self): also keep every pair of the self-collision table (set_self_pairs!) at least
+# self_margin apart, with or without collision; then a fifth result, self_dmin (N,), the smallest pair distance at q.
 function inverse_kinematics_batch(dm::DeviceMechanism, link::Link, targets::CuMatrix{Float64}, q0::CuMatrix{Float64},
                                   joints::Vector{<:Joint}; with_rot=true, iters=100, ftol=1e-10, collision=false, margin=0.02,
-                                  coll_weight=100.0, ctol=1e-6, with_base=false)
+                                  coll_weight=100.0, ctol=1e-6, with_base=false, self_margin=nothing)
     N = size(q0, 2)
     @assert size(targets) == (6, N) && size(q0, 1) == dm.n_dof
     lo = Cdouble[lower_limit(j) for j in joints]; hi = Cdouble[upper_limit(j) for j in joints]     # inverse_kinematics.jl:54-55
     with_base && (append!(lo, fill(-Inf, 3)); append!(hi, fill(Inf, 3)))
     q = similar(q0); f = CuArray{Float64}(undef, N); its = CuArray{Cint}(undef, N); dmin = CUDA.zeros(Float64, N)
+    self_dmin = self_margin === nothing ? nothing : CuArray{Float64}(undef, N)
     vp(x) = reinterpret(CuPtr{Cvoid}, pointer(x))
     GC.@preserve lo hi begin
         call = KinIkCall(N, link.id, with_rot, iters, ftol, 1e-2, vp(targets), vp(q0), pointer(lo), pointer(hi), vp(q), vp(f),
                          pointer(its), cuda_stream(), collision, 0, margin, coll_weight, ctol, vp(dmin))
-        check(ccall((:kin_ik_solve, libkin), Cint, (Ptr{Cvoid}, Ref{KinIkCall}), dm.handle, call))
+        if self_margin === nothing
+            check(ccall((:kin_ik_solve, libkin), Cint, (Ptr{Cvoid}, Ref{KinIkCall}), dm.handle, call))
+        else
+            check(ccall((:kin_ik_solve_self, libkin), Cint, (Ptr{Cvoid}, Ref{KinIkCall}, Cdouble, CuPtr{Cvoid}),
+                        dm.handle, call, Float64(self_margin), pointer(self_dmin)))
+        end
     end
-    return q, f, its, dmin
+    return self_margin === nothing ? (q, f, its, dmin) : (q, f, its, dmin, self_dmin)
 end
 
 # Reductions of compute_coll_dists per configuration (extension): smallest sphere distance, the sphere attaining it

@@ -1415,11 +1415,60 @@ int kin_pose_residual(KinModel *m, int32_t precision, int32_t layout, const void
 }  // extern "C"
 namespace {
 
-template <int ND>
-void launch_ik_coll_step(const kin::IkCollArgs &a, bool rot, cudaStream_t stream, int dev_smem) {
+// One launch of the self-collision kernel (kin_eval_kernel<..., SELF = true>) over `pairs`: n configurations, SoA rows
+// of stride ld (the other layouts ignore it).  kin_self_collision calls it with ld = n; kin_ik_solve_self with the
+// stride of its workspace over the active list.
+int self_collision_launch(KinModel *m, const DevicePairs &pairs, int32_t precision, int32_t layout, const void *q, long long n,
+                          long long ld, double truncation_dist, double vals_offset, void *vals_out, void *grads_out,
+                          void *dmin_out, int32_t *amin_out, cudaStream_t stream) {
+    // phase 1 of a collision call computes the sphere centres and joint frames: the self-collision kernels run the
+    // program of a plain collision call (no links requested, clean scratch); only the pointer's presence matters
+    KinCall c;
+    std::memset(&c, 0, sizeof c);
+    c.precision = precision; c.layout = layout; c.n = n; c.q = q;
+    c.vals_out = vals_out ? vals_out : dmin_out; c.scratch_mode = KIN_SCRATCH_CLEAN;
+    std::shared_ptr<DeviceProgram> dp;
+    int rc = get_program(m, &c, dp);
+    if (rc != KIN_OK) return rc;
+    const int pi = precision == KIN_F32 ? 1 : 0, li = layout;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        if (dp->self_block[pi][li] == 0 && (rc = configure(m, dp.get(), pi, li, true)) != KIN_OK) return rc;
+    }
+    kin::KernelArgs a;
+    std::memset(&a, 0, sizeof a);
+    a.h = dp->prog.h;
+    a.tab_i = dp->d_int;
+    a.tab_r = pi ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
+    a.q = q;
+    a.vals_out = vals_out; a.grads_out = grads_out;
+    a.n = n; a.ld = ld;
+    a.truncation_dist = truncation_dist; a.vals_offset = vals_offset;
+    a.self_pairs = pairs.d; a.n_self_pairs = pairs.n;
+    a.dmin_out = dmin_out; a.amin_out = amin_out;
+    const int block = dp->self_block[pi][li];
+    const long long tiles = (n + block - 1) / block;
+    long long grid = (long long)dp->self_occ[pi][li] * m->n_sm;
+    if (grid > tiles) grid = tiles;
+    const int jr = dp->prog.h.n_dof <= kin::JF_REGS ? 1 : 0;
+    kSelfKernels[pi][li][dp->self_bs_index[pi][li]][jr]<<<(unsigned)grid, block, dp->self_smem[pi][li], stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    g_launches.fetch_add(1);
+    return KIN_OK;
+}
+
+// The pair block of kin_ik_solve_self: the table (kept alive for the whole solve) and the margin.
+struct IkSelfBlock {
+    std::shared_ptr<DevicePairs> pairs;
+    double margin = 0.0;
+    void *dmin_out = nullptr;
+};
+
+template <int ND, bool SELF>
+void launch_ik_coll_step(const kin::IkcArgsT<SELF> &a, bool rot, cudaStream_t stream, int dev_smem) {
     int block = 128;
     size_t smem = 0;
-    auto kern = rot ? kin::ik_coll_step_kernel<ND, true> : kin::ik_coll_step_kernel<ND, false>;
+    auto kern = rot ? kin::ik_coll_step_kernel<ND, true, SELF> : kin::ik_coll_step_kernel<ND, false, SELF>;
     if (ND == 0) {
         // run-time-sized instance (13 .. IKC_MAX_DOF columns): the normal equations of a problem live in shared memory,
         // [slot][thread]; the largest CTA whose slots fit (18 columns: 1800 B per thread, 128 threads = 225 KB; 20 columns: 96 threads)
@@ -1432,26 +1481,51 @@ void launch_ik_coll_step(const kin::IkCollArgs &a, bool rot, cudaStream_t stream
     kern<<<grid, block, smem, stream>>>(a);
 }
 
+template <bool SELF>
+void launch_ik_coll_step_any(const kin::IkcArgsT<SELF> &a, int nd, int rows, cudaStream_t stream, int dev_smem) {
+    // KIN_IK_STEP=warp sends the step through the one-warp-per-problem kernel (kin_ik_coll.cuh: an independent
+    // parallelisation with bit-identical iterates, kept as a cross-check; measured slower than one thread per problem
+    // at every list length: 18 columns, 42 k problems 1.7 against 1.06 ms, 262 k problems 9.3 against 4.6 ms)
+    const char *step_mode = std::getenv("KIN_IK_STEP");
+    if (step_mode && !std::strcmp(step_mode, "warp")) {
+        const unsigned grid = (unsigned)((a.n_act + 3) / 4);                 // 4 warps = 4 problems per CTA
+        if (rows == 6) kin::ik_coll_step_warp_kernel<true, SELF><<<grid, 128, 0, stream>>>(a);
+        else kin::ik_coll_step_warp_kernel<false, SELF><<<grid, 128, 0, stream>>>(a);
+    } else switch (nd) {
+#define KIN_IKC_CASE(N_) case N_: launch_ik_coll_step<N_, SELF>(a, rows == 6, stream, dev_smem); break;
+        KIN_IKC_CASE(1) KIN_IKC_CASE(2) KIN_IKC_CASE(3) KIN_IKC_CASE(4) KIN_IKC_CASE(5) KIN_IKC_CASE(6)
+        KIN_IKC_CASE(7) KIN_IKC_CASE(8) KIN_IKC_CASE(9) KIN_IKC_CASE(10) KIN_IKC_CASE(11) KIN_IKC_CASE(12)
+#undef KIN_IKC_CASE
+        default: launch_ik_coll_step<0, SELF>(a, rows == 6, stream, dev_smem); break;       // 13 .. IKC_MAX_DOF columns: run-time-sized instance
+    }
+}
+
 // The collision-constrained solve of kin_ik_solve (csrc/kin_ik_coll.cuh): a loop of (kin_eval, step kernel) pairs on the
 // caller's stream over a stream-ordered workspace.  At iterations 1, 2, 3, 4, 6, 8, 12, 16, 24, ... the still-running
 // problems are compacted into an active list and its length (8 bytes) is read back -- the only host synchronisations --
 // so that the following pairs cover only those problems (KIN_IK_NO_COMPACT=1: every pair covers the whole batch and
 // nothing is read back).
 // With c->collision == 0 (the pose-only problem when the run-time compiler is unavailable) no sphere is evaluated.
-int ik_solve_coll(KinModel *m, const KinIkCall *c) {
+// With sb (kin_ik_solve_self) every iteration also evaluates the self-collision pairs at the trial points (one
+// kin_self_collision launch over the same active list, between kin_eval and the step) and the step kernels run their
+// SELF instances; pair values and gradients are indexed by list position like V and G, the pair multipliers by problem
+// like mult, so the compaction carries nothing new.
+int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullptr) {
     const int nd = m->hm.n_dof(), S = c->collision ? m->hm.n_sph : 0, rows = c->with_rot ? 6 : 3;
+    const int P = sb ? sb->pairs->n : 0;
     if (c->collision && (S < 1 || m->hm.n_box < 1))
         return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: collision requested but the model has no spheres / no boxes");
     if (c->collision && !(c->margin == c->margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: margin is NaN");
     DeviceGuard guard(m->device);
     cudaStream_t stream = (cudaStream_t)c->stream;
     const long long n = c->n, ld = (n + 31) / 32 * 32;
-    // workspace (doubles per problem): q_try, T, J, V, G | q, H, g, phi, fpose, damp, viol, mult | Vfin ; then int32 status, its
+    // workspace (doubles per problem): q_try, T, J, V, G | q, H, g, phi, fpose, damp, viol, mult | Vfin | q_try_b
+    // | VP, GP, multP (pairs only) ; then int32 status, its, two lists
     const long long nh = (long long)nd * (nd + 1) / 2;
-    const long long per = nd + 12 + (long long)rows * nd + S + (long long)S * nd + nd + nh + nd + 4 + S + S + nd;
+    const long long per = nd + 12 + (long long)rows * nd + S + (long long)S * nd + nd + nh + nd + 4 + S + S + nd + (long long)P * (nd + 2);
     double *ws = nullptr;
     CUDA_TRY(cudaMallocFromPoolAsync((void **)&ws, sizeof(double) * (size_t)(per * ld + 2) + 4 * sizeof(int32_t) * (size_t)ld, m->pool, stream));
-    kin::IkCollArgs a;
+    kin::IkCollSelfArgs a;
     std::memset(&a, 0, sizeof a);
     double *p = ws;
     auto take = [&](long long k) { double *r = p; p += k * ld; return r; };
@@ -1463,6 +1537,8 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c) {
     a.phi = take(1); a.fpose = take(1); a.damp = take(1); a.viol = take(1); a.mult = take(S);
     double *Vfin = take(S);
     double *q_try_b = take(nd);                                  // second trial-point buffer (compaction ping-pong)
+    double *VP = take(P), *GP = take((long long)P * nd);
+    a.VP = VP; a.GP = GP; a.multP = take(P);
     unsigned long long *d_count = (unsigned long long *)p;
     p += 2;
     a.status = (int32_t *)p; a.its = a.status + ld;
@@ -1477,9 +1553,15 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c) {
         a.lo[j] = c->lower ? c->lower[j] : -INFINITY;
         a.hi[j] = c->upper ? c->upper[j] : INFINITY;
     }
+    a.n_pairs = P;
+    if (sb) { a.self_margin = sb->margin; a.self_trunc = sb->margin + 0.05; }      // as the sphere block (planning.jl:56)
     int rc = KIN_OK;
     kin::ik_coll_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(a, (const double *)c->q0, nd);
     g_launches.fetch_add(1);
+    if (sb) {
+        cudaError_t le = cudaMemsetAsync(a.multP, 0, sizeof(double) * (size_t)P * (size_t)ld, stream);      // multipliers 0
+        if (le != cudaSuccess) { cudaFreeAsync(ws, stream); return fail_cuda(le, "clearing the pair multipliers of kin_ik_solve_self"); }
+    }
     KinCall ec;
     std::memset(&ec, 0, sizeof ec);
     ec.precision = KIN_F64; ec.layout = KIN_LAYOUT_SOA; ec.n = n; ec.batch_stride = ld; ec.q = a.q_try;
@@ -1511,22 +1593,14 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c) {
         }
         rc = kin_eval(m, &ec);
         if (rc != KIN_OK) break;
-        a.it = it;
-        // KIN_IK_STEP=warp sends the step through the one-warp-per-problem kernel (kin_ik_coll.cuh: an independent
-        // parallelisation with bit-identical iterates, kept as a cross-check; measured slower than one thread per problem
-        // at every list length: 18 columns, 42 k problems 1.7 against 1.06 ms, 262 k problems 9.3 against 4.6 ms)
-        const char *step_mode = std::getenv("KIN_IK_STEP");
-        if (step_mode && !std::strcmp(step_mode, "warp")) {
-            const unsigned grid = (unsigned)((a.n_act + 3) / 4);                 // 4 warps = 4 problems per CTA
-            if (rows == 6) kin::ik_coll_step_warp_kernel<true><<<grid, 128, 0, stream>>>(a);
-            else kin::ik_coll_step_warp_kernel<false><<<grid, 128, 0, stream>>>(a);
-        } else switch (nd) {
-#define KIN_IKC_CASE(N_) case N_: launch_ik_coll_step<N_>(a, rows == 6, stream, m->dev_smem); break;
-            KIN_IKC_CASE(1) KIN_IKC_CASE(2) KIN_IKC_CASE(3) KIN_IKC_CASE(4) KIN_IKC_CASE(5) KIN_IKC_CASE(6)
-            KIN_IKC_CASE(7) KIN_IKC_CASE(8) KIN_IKC_CASE(9) KIN_IKC_CASE(10) KIN_IKC_CASE(11) KIN_IKC_CASE(12)
-#undef KIN_IKC_CASE
-            default: launch_ik_coll_step<0>(a, rows == 6, stream, m->dev_smem); break;       // 13 .. IKC_MAX_DOF columns: run-time-sized instance
+        if (sb) {           // the pairs at the same trial points, SoA FP64 of stride ld, truncated like the spheres
+            rc = self_collision_launch(m, *sb->pairs, KIN_F64, KIN_LAYOUT_SOA, a.q_try, a.n_act, ld, a.self_trunc, 0.0, VP, GP,
+                                       nullptr, nullptr, stream);
+            if (rc != KIN_OK) break;
         }
+        a.it = it;
+        if (sb) launch_ik_coll_step_any<true>(a, nd, rows, stream, m->dev_smem);
+        else launch_ik_coll_step_any<false>(a, nd, rows, stream, m->dev_smem);
         cudaError_t le = cudaGetLastError();
         if (le != cudaSuccess) { rc = fail_cuda(le, "launching ik_coll_step_kernel"); break; }
         g_launches.fetch_add(1);
@@ -1540,6 +1614,10 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c) {
             fc.truncation_dist = INFINITY; fc.vals_out = Vfin; fc.stream = c->stream;
             rc = kin_eval(m, &fc);
         }
+        // ... and the smallest untruncated pair distance (a dmin-only self-collision launch at q)
+        if (rc == KIN_OK && sb && sb->dmin_out)
+            rc = self_collision_launch(m, *sb->pairs, KIN_F64, KIN_LAYOUT_SOA, a.q, n, ld, INFINITY, 0.0, nullptr, nullptr,
+                                       sb->dmin_out, nullptr, stream);
         if (rc == KIN_OK) {
             kin::ik_coll_finish_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(a, Vfin, nd, (double *)c->q_out, (double *)c->f_out,
                                                                                      c->iters_out, S > 0 ? (double *)c->dmin_out : nullptr);
@@ -1662,6 +1740,31 @@ int kin_ik_solve(KinModel *m, const KinIkCall *c) {
     cudaFreeAsync(ws, stream);
     if (le != cudaSuccess) return fail_cuda(le, "staged kin_ik_solve");
     return KIN_OK;
+}
+
+// kin_ik_solve plus the self-collision pairs as a hard constraint: always the augmented-Lagrangian loop of ik_solve_coll.
+// Every argument is checked before anything is launched.
+int kin_ik_solve_self(KinModel *m, const KinIkCall *c, double self_margin, void *self_dmin_out) {
+    if (!m || !c) return fail(KIN_ERR_INVALID_ARGUMENT, "null model or call");
+    if (c->n < 0 || (c->n > 0 && (!c->targets || !c->q0 || !c->q_out || !c->f_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
+    if (c->iters < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative iteration count");
+    const int nd = m->hm.n_dof();
+    if (nd < 1 || nd > kin::IKC_MAX_DOF) return fail(KIN_ERR_LIMIT, "kin_ik_solve_self: 1..20 configuration columns");
+    if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
+    if (std::isnan(self_margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_self: self_margin is NaN");
+    IkSelfBlock sb;
+    {
+        std::lock_guard<std::mutex> lock(m->mu);
+        sb.pairs = m->self_pairs;
+    }
+    if (!sb.pairs) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_self: the model has no pair table (kin_model_set_self_pairs)");
+    if (c->collision && (m->hm.n_sph < 1 || m->hm.n_box < 1))
+        return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: collision requested but the model has no spheres / no boxes");
+    if (c->collision && std::isnan(c->margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: margin is NaN");
+    if (c->n == 0) return KIN_OK;
+    sb.margin = self_margin;
+    sb.dmin_out = self_dmin_out;
+    return ik_solve_coll(m, c, &sb);
 }
 
 // FP64 peak probe (the denominator of the "FP64 pipe" column of the rooflines): every thread runs 8 independent
@@ -1826,40 +1929,8 @@ int kin_self_collision(KinModel *m, int32_t precision, int32_t layout, const voi
     }
     if (!pairs) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: the model has no pair table (kin_model_set_self_pairs)");
     if (n == 0) return KIN_OK;
-    // phase 1 of a collision call computes the sphere centres and joint frames: the self-collision kernels run the
-    // program of a plain collision call (no links requested, clean scratch); only the pointer's presence matters
-    KinCall c;
-    std::memset(&c, 0, sizeof c);
-    c.precision = precision; c.layout = layout; c.n = n; c.q = q;
-    c.vals_out = vals_out ? vals_out : dmin_out; c.scratch_mode = KIN_SCRATCH_CLEAN;
-    std::shared_ptr<DeviceProgram> dp;
-    int rc = get_program(m, &c, dp);
-    if (rc != KIN_OK) return rc;
-    const int pi = precision == KIN_F32 ? 1 : 0, li = layout;
-    {
-        std::lock_guard<std::mutex> lock(m->mu);
-        if (dp->self_block[pi][li] == 0 && (rc = configure(m, dp.get(), pi, li, true)) != KIN_OK) return rc;
-    }
-    kin::KernelArgs a;
-    std::memset(&a, 0, sizeof a);
-    a.h = dp->prog.h;
-    a.tab_i = dp->d_int;
-    a.tab_r = pi ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
-    a.q = q;
-    a.vals_out = vals_out; a.grads_out = grads_out;
-    a.n = n; a.ld = n;
-    a.truncation_dist = truncation_dist; a.vals_offset = vals_offset;
-    a.self_pairs = pairs->d; a.n_self_pairs = pairs->n;
-    a.dmin_out = dmin_out; a.amin_out = amin_out;
-    const int block = dp->self_block[pi][li];
-    const long long tiles = (n + block - 1) / block;
-    long long grid = (long long)dp->self_occ[pi][li] * m->n_sm;
-    if (grid > tiles) grid = tiles;
-    const int jr = dp->prog.h.n_dof <= kin::JF_REGS ? 1 : 0;
-    kSelfKernels[pi][li][dp->self_bs_index[pi][li]][jr]<<<(unsigned)grid, block, dp->self_smem[pi][li], (cudaStream_t)stream>>>(a);
-    CUDA_TRY(cudaGetLastError());
-    g_launches.fetch_add(1);
-    return KIN_OK;
+    return self_collision_launch(m, *pairs, precision, layout, q, n, n, truncation_dist, vals_offset, vals_out, grads_out,
+                                 dmin_out, amin_out, (cudaStream_t)stream);
 }
 
 }  // extern "C"

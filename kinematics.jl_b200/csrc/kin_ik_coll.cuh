@@ -19,9 +19,12 @@
 // its length (8 bytes, one stream synchronisation) and the following launches cover only that many problems: the trial
 // points / kin_eval outputs are then indexed by list position i, the solver state by problem act[i].  Between two
 // compactions a problem that stops stays in the list (its evaluation is repeated, results ignored).
+// SELF-COLLISION (kin_ik_solve_self): a kin_self_collision launch between 1. and 2. evaluates the model's sphere pairs at
+// the same trial points, and the SELF instances of the step kernels add the pairs as a second constraint block.
 #pragma once
 
 #include <cstdint>
+#include <type_traits>
 
 namespace kin {
 
@@ -43,6 +46,19 @@ struct IkCollArgs {
     int32_t *its;                    // iterations used
     double lo[IKC_MAX_DOF], hi[IKC_MAX_DOF];
 };
+
+// The self-collision block of kin_ik_solve_self (SELF instances of the step kernels): the hard constraint
+// d_p(q) - self_margin >= 0 for every pair p of the model's table, from the kin_self_collision launch of the same
+// iteration.  A derived struct, so that the fields of IkCollArgs keep their offsets and the init / compact / finish
+// kernels, which take further parameters behind an IkCollArgs, keep theirs.
+struct IkCollSelfArgs : IkCollArgs {
+    int n_pairs;
+    double self_margin, self_trunc;
+    const double *VP, *GP;           // pair values [P][ld] and gradients [P][ND][ld] at the trial points (list position)
+    double *multP;                   // pair multipliers [P][ld] (problem)
+};
+template <bool SELF>
+using IkcArgsT = typename std::conditional<SELF, IkCollSelfArgs, IkCollArgs>::type;
 
 // q0 (AoS, caller's) -> q_try and q (SoA); merit +inf so that the first evaluation is accepted
 __global__ void __launch_bounds__(256) ik_coll_init_kernel(const IkCollArgs A, const double *__restrict__ q0, int nd) {
@@ -93,8 +109,11 @@ struct IkcStore<0> {
 };
 __host__ __device__ inline size_t ikc_dyn_smem_per_thread(int nd) { return sizeof(double) * (size_t)(nd * (nd + 1) / 2 + 3 * nd); }
 
-template <int NDT, bool ROT>
-__global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkCollArgs A) {
+// SELF (kin_ik_solve_self): a second constraint block over the self-collision pairs, the same operations per entry as
+// the sphere block (merit term mu psi_p^2, multiplier update, rank-one update of H and g where psi_p > 0, viol) and the
+// same weight mu, after it.  Written with `if constexpr`: the instances without it are the code they were before.
+template <int NDT, bool ROT, bool SELF = false>
+__global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> A) {
     extern __shared__ double ikc_smem[];
     constexpr int NDA = NDT > 0 ? NDT : IKC_MAX_DOF;
     const int ND = NDT > 0 ? NDT : A.nd;
@@ -138,6 +157,14 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkCollArgs A) {
         const double d = A.V[s * ld + i];
         const double psi = d >= A.trunc ? 0.0 : fmax(0.0, margin - d + A.mult[s * ld + n] / mu);
         phi_t = fma(mu * psi, psi, phi_t);
+    }
+    if constexpr (SELF) {
+        #pragma unroll 1
+        for (int p = 0; p < A.n_pairs; ++p) {
+            const double d = A.VP[p * ld + i];
+            const double psi = d >= A.self_trunc ? 0.0 : fmax(0.0, A.self_margin - d + A.multP[p * ld + n] / mu);
+            phi_t = fma(mu * psi, psi, phi_t);
+        }
     }
     const bool ok = phi_t < A.phi[n];
     double damp = A.damp[n];
@@ -193,6 +220,34 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkCollArgs A) {
                     for (int b = 0; b <= a; ++b) W.H(a, b) = fma(ma, W.v(b), W.H(a, b));
                 }
                 phi_n = fma(w, psi, phi_n);
+            }
+        }
+        if constexpr (SELF) {
+            const double sm = A.self_margin;
+            #pragma unroll 1
+            for (int p = 0; p < A.n_pairs; ++p) {
+                const double d = A.VP[p * ld + i];
+                double lam = 0.0, psi = 0.0;
+                if (d < A.self_trunc) {
+                    viol = fmax(viol, sm - d);
+                    lam = mu * fmax(0.0, sm - d + A.multP[p * ld + n] / mu);
+                    psi = fmax(0.0, sm - d + lam / mu);
+                }
+                A.multP[p * ld + n] = lam;
+                if (psi > 0.0) {                     // only active pairs load their gradient row
+                    #pragma unroll
+                    for (int a = 0; a < ND; ++a) W.v(a) = A.GP[(long long)(p * ND + a) * ld + i];
+                    const double w = mu * psi;
+                    #pragma unroll
+                    for (int a = 0; a < ND; ++a) {
+                        const double ga = W.v(a);
+                        W.g(a) = fma(-w, ga, W.g(a));
+                        const double ma = mu * ga;
+                        #pragma unroll
+                        for (int b = 0; b <= a; ++b) W.H(a, b) = fma(ma, W.v(b), W.H(a, b));
+                    }
+                    phi_n = fma(w, psi, phi_n);
+                }
             }
         }
         #pragma unroll
@@ -275,8 +330,9 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkCollArgs A) {
 // written to cut the latency of the run-time-sized instance and does not: a warp per problem leaves 12+ lanes idle and
 // touches one sector per matrix entry (the state is SoA over problems), measured 1.7 ms against 1.06 ms per launch on
 // 42 k problems of 18 columns, 9.3 against 4.6 ms on 262 k.
-template <bool ROT>
-__global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkCollArgs A) {
+// SELF: the pair block of ik_coll_step_kernel<., ., true>, with the same operations per entry in the same order.
+template <bool ROT, bool SELF = false>
+__global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<SELF> A) {
     constexpr int MAXC = IKC_MAX_DOF, ROWS = ROT ? 6 : 3;
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -319,6 +375,14 @@ __global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkCollArgs
         const double d = A.V[s * ld + i];
         const double psi = d >= A.trunc ? 0.0 : fmax(0.0, margin - d + A.mult[s * ld + n] / mu);
         phi_t = fma(mu * psi, psi, phi_t);
+    }
+    if constexpr (SELF) {
+        #pragma unroll 1
+        for (int p = 0; p < A.n_pairs; ++p) {
+            const double d = A.VP[p * ld + i];
+            const double psi = d >= A.self_trunc ? 0.0 : fmax(0.0, A.self_margin - d + A.multP[p * ld + n] / mu);
+            phi_t = fma(mu * psi, psi, phi_t);
+        }
     }
     const bool ok = phi_t < A.phi[n];
     double damp = A.damp[n];
@@ -368,6 +432,33 @@ __global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkCollArgs
                     if (b <= lane) Hrow[b] = fma(ma, gb, Hrow[b]);
                 }
                 phi_n = fma(w, psi, phi_n);
+            }
+        }
+        if constexpr (SELF) {
+            const double sm = A.self_margin;
+            #pragma unroll 1
+            for (int p = 0; p < A.n_pairs; ++p) {
+                const double d = A.VP[p * ld + i];
+                double lam = 0.0, psi = 0.0;
+                if (d < A.self_trunc) {
+                    viol = fmax(viol, sm - d);
+                    lam = mu * fmax(0.0, sm - d + A.multP[p * ld + n] / mu);
+                    psi = fmax(0.0, sm - d + lam / mu);
+                }
+                __syncwarp();                                                   // every lane has read the old multiplier
+                if (lane == 0) A.multP[p * ld + n] = lam;
+                if (psi > 0.0) {
+                    const double ga = mine ? A.GP[(long long)(p * ND + a) * ld + i] : 0.0;
+                    const double w = mu * psi;
+                    g_a = fma(-w, ga, g_a);
+                    const double ma = mu * ga;
+                    #pragma unroll
+                    for (int b = 0; b < MAXC; ++b) {
+                        const double gb = __shfl_sync(FULL, ga, b);
+                        if (b <= lane) Hrow[b] = fma(ma, gb, Hrow[b]);
+                    }
+                    phi_n = fma(w, psi, phi_n);
+                }
             }
         }
         if (mine) {

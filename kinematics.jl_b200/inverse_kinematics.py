@@ -78,7 +78,7 @@ def ik_objective(m: Mechanism, link, joints, target_pose, with_rot=True):
 
 
 def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iters=100, ftol=1e-10, lambda0=1e-2,
-                    sscc=None, sdf=None, margin=0.02, coll_weight=100.0, ctol=1e-6):
+                    sscc=None, sdf=None, margin=0.02, coll_weight=100.0, ctol=1e-6, self_margin=None, self_pairs=None):
     """The device-resident batched solve (``kin_ik_solve``).  ``targets`` (N, 6), ``q0`` (N, n_dof) CUDA tensors.
 
     Without ``sscc`` / ``sdf``: the whole pose-only Levenberg-Marquardt solve in ONE kernel launch around the generated
@@ -88,8 +88,21 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
     With ``sscc`` and ``sdf``: the reference's constrained problem (inverse_kinematics.jl:14-19: the same objective
     subject to ``dists - margin >= 0``) from the warm start ``q0``, by an augmented-Lagrangian Levenberg-Marquardt
     iteration that issues one fused ``kin_eval`` and one step kernel per iteration over the still-running problems (active list)
-    (csrc/kin_ik_coll.cuh) -> (q, f, iterations, dmin) with dmin (N,) the smallest signed sphere distance at q."""
+    (csrc/kin_ik_coll.cuh) -> (q, f, iterations, dmin) with dmin (N,) the smallest signed sphere distance at q.
+
+    With ``self_margin`` (extension; ``kin_ik_solve_self``): also ``d_p - self_margin >= 0`` for every self-collision
+    pair of the table ``self_pairs`` ((P, 2) 1-based sphere ids, default ``self_collision_pairs(sscc, joints)``), in
+    the same loop with one more launch per iteration.  ``sscc`` is required, ``sdf`` optional (without it only the pairs
+    constrain the solve).  Returns (q, f, iterations[, dmin], self_dmin), self_dmin (N,) the smallest pair distance at
+    q.  On the Fetch sphere fixture the default policy keeps a pair of constant distance that overlaps by 5.5 mm in
+    every configuration, which no solver can satisfy: pass ``self_collision_pairs(sscc, joints,
+    ignore=[("wrist_flex_link", "elbow_flex_link")])`` (64 pairs) there."""
     import torch
+    if self_margin is not None:
+        if sscc is None:
+            raise ValueError("ik_solve_device: self_margin needs the collision checker sscc (its spheres form the pairs)")
+        if not np.isfinite(float(self_margin)):
+            raise ValueError("ik_solve_device: self_margin must be finite")
     collide = sscc is not None and sdf is not None
     q0 = torch.as_tensor(q0, dtype=torch.float64, device="cuda").contiguous()
     set_joint_angles(m, joints, q0)            # defines the configuration columns (and the device model) as every caller does
@@ -98,6 +111,9 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
         _, dm = _prepare(sscc, joints, sdf)
     else:
         dm = device_model(m)
+    if self_margin is not None:
+        from .collision import _prepare_self
+        _, dm = _prepare_self(sscc, joints, self_pairs)
     nb = 3 if m.with_base else 0
     lo = np.ascontiguousarray([j.lower_limit for j in joints] + [-np.inf] * nb, dtype=np.float64)
     hi = np.ascontiguousarray([j.upper_limit for j in joints] + [np.inf] * nb, dtype=np.float64)
@@ -116,8 +132,13 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
     if collide:
         dmin = torch.empty(N, dtype=torch.float64, device="cuda")
         c.collision, c.margin, c.coll_weight, c.ctol, c.dmin_out = 1, float(margin), float(coll_weight), float(ctol), dmin.data_ptr()
-    _lib.check(_lib.lib().kin_ik_solve(dm.h, C.byref(c)))
-    return (q, f, its, dmin) if collide else (q, f, its)
+    if self_margin is None:
+        _lib.check(_lib.lib().kin_ik_solve(dm.h, C.byref(c)))
+        return (q, f, its, dmin) if collide else (q, f, its)
+    c.coll_weight, c.ctol = float(coll_weight), float(ctol)
+    self_dmin = torch.empty(N, dtype=torch.float64, device="cuda")
+    _lib.check(_lib.lib().kin_ik_solve_self(dm.h, C.byref(c), float(self_margin), self_dmin.data_ptr()))
+    return (q, f, its, dmin, self_dmin) if collide else (q, f, its, self_dmin)
 
 
 def _seed_limits(m, joints):
@@ -132,7 +153,7 @@ def _seed_limits(m, joints):
 
 def inverse_kinematics_batch(m: Mechanism, link, joints, targets, q0, with_rot=True, iters=100, ftol=1e-10,
                              sscc=None, sdf=None, margin=0.02, coll_weight=100.0, use_bistage=True, restarts=0, tol=1e-3, seed=0,
-                             coll_iters=60, ctol=1e-6, return_dmin=False):
+                             coll_iters=60, ctol=1e-6, return_dmin=False, self_margin=None, self_pairs=None):
     """Batched IK for N independent pose targets (config 4 of BASELINE.json) on the reference's objective
     f = |[p - p_t; rpy - rpy_t]|^2 (inverse_kinematics.jl:38-50), iterates clamped to the joint limits (:52-63).
 
@@ -148,9 +169,19 @@ def inverse_kinematics_batch(m: Mechanism, link, joints, targets, q0, with_rot=T
     at most ``coll_iters`` (fused evaluation, step kernel) launch pairs over the still-running problems (the active list is re-compacted about ten times per solve).  ``restarts``
     re-seeds the problems that end with pose error > ``tol`` or a distance below ``margin - ctol`` (a local method can
     end pressed against the obstacle on the wrong side of it).
+    ``self_margin`` (extension, ``kin_ik_solve_self``; needs ``sscc``, ``sdf`` optional): the solve also keeps every
+    self-collision pair of ``self_pairs`` (default ``self_collision_pairs(sscc, joints)``) at least ``self_margin``
+    apart; the warm start stays pose-only, a problem counts as solved only with its smallest pair distance
+    >= ``self_margin - 10 ctol``, and restarts re-seed the others too.  On the Fetch sphere fixture pass
+    ``self_collision_pairs(sscc, joints, ignore=[("wrist_flex_link", "elbow_flex_link")])``: the default table keeps a
+    pair that overlaps by 5.5 mm in every configuration.
     ``targets`` (N, 6) [x y z roll pitch yaw], ``q0`` (N, n_dof).  Returns (q, f) with f the pose objective
-    (and the smallest signed sphere distance per problem with ``return_dmin``)."""
+    (and the smallest signed sphere distance per problem with ``return_dmin``; with ``self_margin`` and ``return_dmin``:
+    (q, f, dmin or None, self_dmin))."""
     import torch
+    selfc = self_margin is not None
+    if selfc and sscc is None:
+        raise ValueError("inverse_kinematics_batch: self_margin needs the collision checker sscc")
     collide = sscc is not None and sdf is not None
     targets = torch.as_tensor(targets, dtype=torch.float64, device="cuda")
     q0 = torch.as_tensor(q0, dtype=torch.float64, device="cuda")
@@ -159,18 +190,27 @@ def inverse_kinematics_batch(m: Mechanism, link, joints, targets, q0, with_rot=T
         return ik_solve_device(m, link, joints, tg, qs, with_rot=with_rot, iters=iters, ftol=ftol)[:2]
 
     def solve(tg, qs):
-        """-> q, f, good (N,) bool"""
-        if not collide:
+        """-> q, f, dmin, self_dmin, good (N,) bool"""
+        if not collide and not selfc:
             q, f = pose_only(tg, qs)
-            return q, f, None, f <= tol * tol
+            return q, f, None, None, f <= tol * tol
         if use_bistage:
             qs, _ = pose_only(tg, qs)
-        q, f, _, dmin = ik_solve_device(m, link, joints, tg, qs, with_rot=with_rot, iters=coll_iters, ftol=ftol, sscc=sscc, sdf=sdf,
-                                        margin=margin, coll_weight=coll_weight, ctol=ctol)
+        out = ik_solve_device(m, link, joints, tg, qs, with_rot=with_rot, iters=coll_iters, ftol=ftol, sscc=sscc,
+                              sdf=sdf if collide else None, margin=margin, coll_weight=coll_weight, ctol=ctol,
+                              self_margin=self_margin, self_pairs=self_pairs)
+        q, f = out[0], out[1]
+        dmin = out[3] if collide else None
+        sdmin = out[-1] if selfc else None
         # f = sum of squared residuals: max |e| <= tol is implied by f <= tol^2
-        return q, f, dmin, (f <= tol * tol) & (dmin >= margin - 10 * ctol)
+        good = f <= tol * tol
+        if collide:
+            good = good & (dmin >= margin - 10 * ctol)
+        if selfc:
+            good = good & (sdmin >= self_margin - 10 * ctol)
+        return q, f, dmin, sdmin, good
 
-    q, f, dmin, good = solve(targets, q0)
+    q, f, dmin, sdmin, good = solve(targets, q0)
     if restarts > 0:
         lo, hi = _seed_limits(m, joints)
         gen = torch.Generator(device="cuda").manual_seed(seed)
@@ -179,31 +219,39 @@ def inverse_kinematics_batch(m: Mechanism, link, joints, targets, q0, with_rot=T
             if bad.numel() == 0:
                 break
             qs = lo + (hi - lo) * torch.rand((bad.numel(), q.shape[1]), generator=gen, device="cuda", dtype=torch.float64)
-            q2, f2, d2, g2 = solve(targets[bad], qs)
+            q2, f2, d2, s2, g2 = solve(targets[bad], qs)
             # a restart replaces a failed problem when it succeeds, or (pose only) when it is closer
-            better = g2 if collide else (f2 < f[bad])
+            better = g2 if (collide or selfc) else (f2 < f[bad])
             q[bad[better]] = q2[better]
             f[bad[better]] = f2[better]
             if collide:
                 dmin[bad[better]] = d2[better]
+            if selfc:
+                sdmin[bad[better]] = s2[better]
             good[bad[better]] = g2[better]
     set_joint_angles(m, joints, q)
+    if selfc and return_dmin:
+        return q, f, dmin, sdmin
     if collide and return_dmin:
         return q, f, dmin
     return q, f
 
 
 def inverse_kinematics(m: Mechanism, link, joints, target_pose, sscc=None, sdf=None, use_bistage=True, ftol=1e-5,
-                       with_rot=True, margin=0.02):
+                       with_rot=True, margin=0.02, self_margin=None, self_pairs=None):
     """``inverse_kinematics!`` (inverse_kinematics.jl:1-30) for ONE target, driven by SLSQP as in the reference.
     The reference calls NLopt's LD_SLSQP; NLopt is not installed here, scipy's SLSQP (the same Kraft routine, which
     the reference itself uses as its SCIPY back-end in planning.jl:388-394) drives the same callbacks: the objective
     ``f_objective`` (:38-50, ``ik_objective``), the joint-limit bounds (:52-63) and, with ``sscc`` / ``sdf``, the HARD
     inequality constraint ``dists - margin >= 0`` of ``IneqConst(sscc, joints, sdf, 1, 0.02)`` (:14-19) after the
-    collision-free warm start (:8-13).  Every evaluation runs on the GPU (N = 1).  Returns (q, scipy result); the
+    collision-free warm start (:8-13).  ``self_margin`` (extension): also the self-collision constraint
+    ``SelfIneqConst(sscc, joints, 1, self_margin, self_pairs)`` as a second inequality, as ``plan_trajectory`` adds it;
+    the warm start stays unconstrained.  Every evaluation runs on the GPU (N = 1).  Returns (q, scipy result); the
     mechanism is left at the solution like the reference leaves it."""
     from scipy.optimize import minimize
-    from .planning import IneqConst, scipynize
+    from .planning import IneqConst, SelfIneqConst, scipynize
+    if self_margin is not None and sscc is None:
+        raise ValueError("inverse_kinematics: self_margin needs the collision checker sscc")
     nb = 3 if m.with_base else 0
     lo = [j.lower_limit for j in joints] + [-np.inf] * nb
     hi = [j.upper_limit for j in joints] + [np.inf] * nb
@@ -218,12 +266,18 @@ def inverse_kinematics(m: Mechanism, link, joints, target_pose, sscc=None, sdf=N
                         options={"ftol": ftol, "maxiter": 200})
 
     x0 = np.array([m.angles[j.id - 1] for j in joints] + (list(m.base_pose) if m.with_base else []))
-    if sscc is None or sdf is None:
+    cons = []
+    if sscc is not None and sdf is not None:
+        g, dg = scipynize(IneqConst(sscc, joints, sdf, 1, margin))
+        cons.append({"type": "ineq", "fun": g, "jac": dg})
+    if self_margin is not None:
+        gs, dgs = scipynize(SelfIneqConst(sscc, joints, 1, self_margin, self_pairs))
+        cons.append({"type": "ineq", "fun": gs, "jac": dgs})
+    if not cons:
         res = solve(x0, ())
     else:
         if use_bistage:
             x0 = solve(x0, ()).x
-        g, dg = scipynize(IneqConst(sscc, joints, sdf, 1, margin))
-        res = solve(x0, [{"type": "ineq", "fun": g, "jac": dg}])
+        res = solve(x0, cons)
     set_joint_angles(m, joints, res.x)
     return res.x, res
