@@ -376,6 +376,22 @@ KIN_API int kin_ik_solve(KinModel *model, const KinIkCall *call);
  * (pair values, gradients and multipliers) -- 23.2 KB on a model of 18 columns and 145 pairs, i.e. 6.1 GB at 2^18
  * problems and 24.3 GB at 2^20; a pool allocation that fails is returned as KIN_ERR_CUDA. */
 KIN_API int kin_ik_solve_self(KinModel *model, const KinIkCall *call, double self_margin, void *self_dmin_out);
+/* Several links per problem (extension: the reference's inverse_kinematics! places one link).  The objective is
+ * f = sum_l |e_l|^2 with e_l = [p_l - p_t,l ; rpy_l - rpy_t,l] (angles wrapped to (-pi, pi]); a link with
+ * with_rots[l] == 0 contributes its 3 position rows only -- the stacked pose constraint of kin_pose_residual_multi.
+ * link_ids / with_rots: HOST [n_links], 1-based distinct ids.  call->link_id and call->with_rot are not read;
+ * call->targets is DEVICE [n][6 n_links], the 6 values of each link in link order (the angles of a position-only link
+ * are not read).  Everything else as kin_ik_solve (self_collision == 0: the pose-only solve, or the AL loop with
+ * call->collision) or kin_ik_solve_self (self_collision != 0; self_dmin_out nullable); f_out is the sum over the
+ * links.  n_links == 1 is bit for bit the call of kin_ik_solve / kin_ik_solve_self.  Errors, before anything is
+ * launched: n_links outside 1..KIN_IK_MAX_LINKS, a null array, an id out of range or repeated, a NaN self_margin
+ * (KIN_ERR_INVALID_ARGUMENT); self_collision without a pair table, collision without spheres / boxes
+ * (KIN_ERR_INVALID_ARGUMENT, as the two single-link calls); n_dof > 20 (KIN_ERR_LIMIT).  Workspace of the AL loop: on
+ * top of the single-link solve's, (n_links - 1)(12 + rows n_dof) * 8 bytes of stream-ordered scratch per problem
+ * (rows = 6 when any link has rotation, else 3): the links' transforms and Jacobians. */
+#define KIN_IK_MAX_LINKS 4
+KIN_API int kin_ik_solve_links(KinModel *model, const KinIkCall *call, int32_t n_links, const int32_t *link_ids,
+                               const int32_t *with_rots, int32_t self_collision, double self_margin, void *self_dmin_out);
 
 /* Diagnostics for bench.py / tests: kernel launches issued by this library since load, and the
  * static resources of the kernel a call would use (registers / thread, dynamic shared memory bytes /

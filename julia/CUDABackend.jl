@@ -351,6 +351,33 @@ function inverse_kinematics_batch(dm::DeviceMechanism, link::Link, targets::CuMa
     return self_margin === nothing ? (q, f, its, dmin) : (q, f, its, dmin, self_dmin)
 end
 
+# Several links per problem (extension, kin_ik_solve_links; the reference's inverse_kinematics! places one link):
+# `targets` (6 L, N), the 6 values of each link in link order; the objective is the sum of the links' f_objective, a link
+# whose with_rots entry is false contributing its 3 position rows.  Everything else and the results as above.
+function inverse_kinematics_batch(dm::DeviceMechanism, links::AbstractVector{<:Link}, targets::CuMatrix{Float64},
+                                  q0::CuMatrix{Float64}, joints::Vector{<:Joint}; with_rots=fill(true, length(links)),
+                                  iters=100, ftol=1e-10, collision=false, margin=0.02, coll_weight=100.0, ctol=1e-6,
+                                  with_base=false, self_margin=nothing)
+    N = size(q0, 2); L = length(links)
+    @assert 1 <= L <= 4 && length(with_rots) == L && size(targets) == (6L, N) && size(q0, 1) == dm.n_dof
+    lo = Cdouble[lower_limit(j) for j in joints]; hi = Cdouble[upper_limit(j) for j in joints]
+    with_base && (append!(lo, fill(-Inf, 3)); append!(hi, fill(Inf, 3)))
+    ids = Cint[l.id for l in links]; rots = Cint[w ? 1 : 0 for w in with_rots]
+    q = similar(q0); f = CuArray{Float64}(undef, N); its = CuArray{Cint}(undef, N); dmin = CUDA.zeros(Float64, N)
+    self_dmin = self_margin === nothing ? CUDA.zeros(Float64, 1) : CuArray{Float64}(undef, N)
+    vp(x) = reinterpret(CuPtr{Cvoid}, pointer(x))
+    GC.@preserve lo hi ids rots begin
+        call = KinIkCall(N, 0, 0, iters, ftol, 1e-2, vp(targets), vp(q0), pointer(lo), pointer(hi), vp(q), vp(f),
+                         pointer(its), cuda_stream(), collision, 0, margin, coll_weight, ctol, vp(dmin))
+        check(ccall((:kin_ik_solve_links, libkin), Cint,
+                    (Ptr{Cvoid}, Ref{KinIkCall}, Cint, Ptr{Cint}, Ptr{Cint}, Cint, Cdouble, CuPtr{Cvoid}),
+                    dm.handle, call, Cint(L), ids, rots, Cint(self_margin === nothing ? 0 : 1),
+                    Float64(self_margin === nothing ? 0.0 : self_margin),
+                    self_margin === nothing ? CuPtr{Cvoid}(0) : pointer(self_dmin)))
+    end
+    return self_margin === nothing ? (q, f, its, dmin) : (q, f, its, dmin, self_dmin)
+end
+
 # Reductions of compute_coll_dists per configuration (extension): smallest sphere distance, the sphere attaining it
 # (1-based, first minimum), hinge cost sum_s max(0, margin - d_s)^2
 function collision_summary(dm::DeviceMechanism, Q::CuMatrix{Float64}; layout::Symbol=:soa, margin::Float64=0.0)

@@ -782,8 +782,10 @@ int kin_codegen_dump(const KinModelDesc *d, const KinCall *c, int32_t compile, c
     std::string err;
     if (!kin::compile_program(hm, fk, jac, want_coll, want_stale, kin::JF_REGS, dp.prog, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
     kin::GenOptions o = gen_options(nullptr, c, &dp);
-    if (std::getenv("KIN_DUMP_IK")) {          // development aid: the batched-IK kernel of this link instead
+    if (const char *ik = std::getenv("KIN_DUMP_IK")) {   // development aid: the batched-IK kernel of this link instead
         o.ik = 1; o.rpy_jac = o.with_rot; o.ksync = 0; o.coll = false; o.block = 128; o.min_blocks = 1;
+        // several links (kin_ik_solve_links): the value is the rotation mask (bit l: link l has rotation rows)
+        if (dp.prog.h.n_fk > 1) o.ik_rot = (unsigned)std::strtoul(ik, nullptr, 0);
     }
     kin::GenSource g;
     if (!kin::generate_source(dp.prog, o, g, err)) return fail(KIN_ERR_INVALID_ARGUMENT, "codegen: " + err);
@@ -1457,6 +1459,23 @@ int self_collision_launch(KinModel *m, const DevicePairs &pairs, int32_t precisi
     return KIN_OK;
 }
 
+// The links a solve places (kin_ik_solve / kin_ik_solve_self: the call's one link; kin_ik_solve_links: up to
+// KIN_IK_MAX_LINKS), in the order of the targets.  rows: residual rows per link in the kin_eval Jacobian (6 when any
+// link has rotation).
+static_assert(kin::IKC_MAX_LINKS == KIN_IK_MAX_LINKS, "the step kernels hold KIN_IK_MAX_LINKS residual blocks");
+struct IkLinks {
+    int n = 1;
+    int32_t ids[KIN_IK_MAX_LINKS] = {};
+    unsigned rot_mask = 0;
+    int rows() const { return rot_mask ? 6 : 3; }
+};
+IkLinks ik_one_link(const KinIkCall *c) {
+    IkLinks lk;
+    lk.ids[0] = c->link_id;
+    lk.rot_mask = c->with_rot ? 1u : 0u;
+    return lk;
+}
+
 // The pair block of kin_ik_solve_self: the table (kept alive for the whole solve) and the margin.
 struct IkSelfBlock {
     std::shared_ptr<DevicePairs> pairs;
@@ -1464,11 +1483,11 @@ struct IkSelfBlock {
     void *dmin_out = nullptr;
 };
 
-template <int ND, bool SELF>
-void launch_ik_coll_step(const kin::IkcArgsT<SELF> &a, bool rot, cudaStream_t stream, int dev_smem) {
+template <int ND, bool SELF, bool LINKS>
+void launch_ik_coll_step(const kin::IkcArgsT<SELF, LINKS> &a, bool rot, cudaStream_t stream, int dev_smem) {
     int block = 128;
     size_t smem = 0;
-    auto kern = rot ? kin::ik_coll_step_kernel<ND, true, SELF> : kin::ik_coll_step_kernel<ND, false, SELF>;
+    auto kern = rot ? kin::ik_coll_step_kernel<ND, true, SELF, LINKS> : kin::ik_coll_step_kernel<ND, false, SELF, LINKS>;
     if (ND == 0) {
         // run-time-sized instance (13 .. IKC_MAX_DOF columns): the normal equations of a problem live in shared memory,
         // [slot][thread]; the largest CTA whose slots fit (18 columns: 1800 B per thread, 128 threads = 225 KB; 20 columns: 96 threads)
@@ -1481,22 +1500,22 @@ void launch_ik_coll_step(const kin::IkcArgsT<SELF> &a, bool rot, cudaStream_t st
     kern<<<grid, block, smem, stream>>>(a);
 }
 
-template <bool SELF>
-void launch_ik_coll_step_any(const kin::IkcArgsT<SELF> &a, int nd, int rows, cudaStream_t stream, int dev_smem) {
+template <bool SELF, bool LINKS>
+void launch_ik_coll_step_any(const kin::IkcArgsT<SELF, LINKS> &a, int nd, int rows, cudaStream_t stream, int dev_smem) {
     // KIN_IK_STEP=warp sends the step through the one-warp-per-problem kernel (kin_ik_coll.cuh: an independent
     // parallelisation with bit-identical iterates, kept as a cross-check; measured slower than one thread per problem
     // at every list length: 18 columns, 42 k problems 1.7 against 1.06 ms, 262 k problems 9.3 against 4.6 ms)
     const char *step_mode = std::getenv("KIN_IK_STEP");
     if (step_mode && !std::strcmp(step_mode, "warp")) {
         const unsigned grid = (unsigned)((a.n_act + 3) / 4);                 // 4 warps = 4 problems per CTA
-        if (rows == 6) kin::ik_coll_step_warp_kernel<true, SELF><<<grid, 128, 0, stream>>>(a);
-        else kin::ik_coll_step_warp_kernel<false, SELF><<<grid, 128, 0, stream>>>(a);
+        if (rows == 6) kin::ik_coll_step_warp_kernel<true, SELF, LINKS><<<grid, 128, 0, stream>>>(a);
+        else kin::ik_coll_step_warp_kernel<false, SELF, LINKS><<<grid, 128, 0, stream>>>(a);
     } else switch (nd) {
-#define KIN_IKC_CASE(N_) case N_: launch_ik_coll_step<N_, SELF>(a, rows == 6, stream, dev_smem); break;
+#define KIN_IKC_CASE(N_) case N_: launch_ik_coll_step<N_, SELF, LINKS>(a, rows == 6, stream, dev_smem); break;
         KIN_IKC_CASE(1) KIN_IKC_CASE(2) KIN_IKC_CASE(3) KIN_IKC_CASE(4) KIN_IKC_CASE(5) KIN_IKC_CASE(6)
         KIN_IKC_CASE(7) KIN_IKC_CASE(8) KIN_IKC_CASE(9) KIN_IKC_CASE(10) KIN_IKC_CASE(11) KIN_IKC_CASE(12)
 #undef KIN_IKC_CASE
-        default: launch_ik_coll_step<0, SELF>(a, rows == 6, stream, dev_smem); break;       // 13 .. IKC_MAX_DOF columns: run-time-sized instance
+        default: launch_ik_coll_step<0, SELF, LINKS>(a, rows == 6, stream, dev_smem); break;       // 13 .. IKC_MAX_DOF columns: run-time-sized instance
     }
 }
 
@@ -1510,8 +1529,10 @@ void launch_ik_coll_step_any(const kin::IkcArgsT<SELF> &a, int nd, int rows, cud
 // kin_self_collision launch over the same active list, between kin_eval and the step) and the step kernels run their
 // SELF instances; pair values and gradients are indexed by list position like V and G, the pair multipliers by problem
 // like mult, so the compaction carries nothing new.
-int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullptr) {
-    const int nd = m->hm.n_dof(), S = c->collision ? m->hm.n_sph : 0, rows = c->with_rot ? 6 : 3;
+// With several links (kin_ik_solve_links) kin_eval returns every link's transform and Euler-rate Jacobian, T and J
+// grow by (n_links - 1)(12 + rows n_dof) doubles per problem, and the step kernels run their LINKS instances.
+int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkLinks &lk, const IkSelfBlock *sb = nullptr) {
+    const int nd = m->hm.n_dof(), S = c->collision ? m->hm.n_sph : 0, rows = lk.rows(), NL = lk.n;
     const int P = sb ? sb->pairs->n : 0;
     if (c->collision && (S < 1 || m->hm.n_box < 1))
         return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: collision requested but the model has no spheres / no boxes");
@@ -1522,16 +1543,16 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullp
     // workspace (doubles per problem): q_try, T, J, V, G | q, H, g, phi, fpose, damp, viol, mult | Vfin | q_try_b
     // | VP, GP, multP (pairs only) ; then int32 status, its, two lists
     const long long nh = (long long)nd * (nd + 1) / 2;
-    const long long per = nd + 12 + (long long)rows * nd + S + (long long)S * nd + nd + nh + nd + 4 + S + S + nd + (long long)P * (nd + 2);
+    const long long per = nd + 12LL * NL + (long long)NL * rows * nd + S + (long long)S * nd + nd + nh + nd + 4 + S + S + nd + (long long)P * (nd + 2);
     double *ws = nullptr;
     CUDA_TRY(cudaMallocFromPoolAsync((void **)&ws, sizeof(double) * (size_t)(per * ld + 2) + 4 * sizeof(int32_t) * (size_t)ld, m->pool, stream));
-    kin::IkCollSelfArgs a;
+    kin::IkCollLinksArgs a;
     std::memset(&a, 0, sizeof a);
     double *p = ws;
     auto take = [&](long long k) { double *r = p; p += k * ld; return r; };
     a.n = n; a.ld = ld; a.n_sph = S;
     a.q_try = take(nd);
-    double *T = take(12), *J = take((long long)rows * nd), *V = take(S), *G = take((long long)S * nd);
+    double *T = take(12LL * NL), *J = take((long long)NL * rows * nd), *V = take(S), *G = take((long long)S * nd);
     a.T = T; a.J = J; a.V = V; a.G = G;
     a.q = take(nd); a.H = take(nh); a.g = take(nd);
     a.phi = take(1); a.fpose = take(1); a.damp = take(1); a.viol = take(1); a.mult = take(S);
@@ -1554,6 +1575,7 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullp
         a.hi[j] = c->upper ? c->upper[j] : INFINITY;
     }
     a.n_pairs = P;
+    a.n_links = NL; a.rot_mask = lk.rot_mask;
     if (sb) { a.self_margin = sb->margin; a.self_trunc = sb->margin + 0.05; }      // as the sphere block (planning.jl:56)
     int rc = KIN_OK;
     kin::ik_coll_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(a, (const double *)c->q0, nd);
@@ -1565,8 +1587,8 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullp
     KinCall ec;
     std::memset(&ec, 0, sizeof ec);
     ec.precision = KIN_F64; ec.layout = KIN_LAYOUT_SOA; ec.n = n; ec.batch_stride = ld; ec.q = a.q_try;
-    ec.n_fk_links = 1; ec.fk_links = &c->link_id; ec.T_out = T;
-    ec.n_jac_links = 1; ec.jac_links = &c->link_id; ec.with_rot = c->with_rot ? 1 : 0; ec.rpy_jac = 1; ec.J_out = J;
+    ec.n_fk_links = NL; ec.fk_links = lk.ids; ec.T_out = T;
+    ec.n_jac_links = NL; ec.jac_links = lk.ids; ec.with_rot = lk.rot_mask ? 1 : 0; ec.rpy_jac = 1; ec.J_out = J;
     ec.truncation_dist = a.trunc; ec.grad_mode = KIN_GRAD_FD; ec.scratch_mode = KIN_SCRATCH_CLEAN;
     if (S > 0) { ec.vals_out = V; ec.grads_out = G; }
     ec.stream = c->stream;
@@ -1599,8 +1621,10 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullp
             if (rc != KIN_OK) break;
         }
         a.it = it;
-        if (sb) launch_ik_coll_step_any<true>(a, nd, rows, stream, m->dev_smem);
-        else launch_ik_coll_step_any<false>(a, nd, rows, stream, m->dev_smem);
+        if (NL > 1 && sb) launch_ik_coll_step_any<true, true>(a, nd, rows, stream, m->dev_smem);
+        else if (NL > 1) launch_ik_coll_step_any<false, true>(a, nd, rows, stream, m->dev_smem);
+        else if (sb) launch_ik_coll_step_any<true, false>(a, nd, rows, stream, m->dev_smem);
+        else launch_ik_coll_step_any<false, false>(a, nd, rows, stream, m->dev_smem);
         cudaError_t le = cudaGetLastError();
         if (le != cudaSuccess) { rc = fail_cuda(le, "launching ik_coll_step_kernel"); break; }
         g_launches.fetch_add(1);
@@ -1630,35 +1654,28 @@ int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkSelfBlock *sb = nullp
     return rc;
 }
 
-}  // namespace
-extern "C" {
-
-int kin_ik_solve(KinModel *m, const KinIkCall *c) {
-    if (!m || !c) return fail(KIN_ERR_INVALID_ARGUMENT, "null model or call");
-    if (c->n < 0 || (c->n > 0 && (!c->targets || !c->q0 || !c->q_out || !c->f_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
-    if (c->iters < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative iteration count");
+// The pose-only solve: the generated one-launch kernel (kin_gen_skeleton.cuh: kin_ik_kernel) around the links'
+// straight-line FK + Euler-rate Jacobians, staged over the still-running problems for large batches.  Without the
+// run-time compiler: the loop of ik_solve_coll without spheres.
+int ik_solve_pose(KinModel *m, const KinIkCall *c, const IkLinks &lk) {
     const int nd = m->hm.n_dof();
-    if (nd < 1 || nd > kin::IKC_MAX_DOF) return fail(KIN_ERR_LIMIT, "kin_ik_solve: 1..20 configuration columns");
-    if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
-    if (c->n == 0) return KIN_OK;
-    if (c->collision) return ik_solve_coll(m, c);
-    if (std::getenv("KIN_DISABLE_JIT")) return ik_solve_coll(m, c);      // no run-time compiler: (kin_eval, step kernel) pairs
+    if (std::getenv("KIN_DISABLE_JIT")) return ik_solve_coll(m, c, lk);      // no run-time compiler: (kin_eval, step kernel) pairs
     DeviceGuard guard(m->device);
-    // the program of (this link's transform + its Euler-rate Jacobian)
+    // the program of (the links' transforms + their Euler-rate Jacobians)
     KinCall pc;
     std::memset(&pc, 0, sizeof pc);
     pc.precision = KIN_F64; pc.layout = KIN_LAYOUT_SOA; pc.n = c->n; pc.q = c->q0;
-    pc.n_fk_links = 1; pc.fk_links = &c->link_id; pc.T_out = (void *)c->q_out;
-    pc.n_jac_links = 1; pc.jac_links = &c->link_id; pc.J_out = (void *)c->q_out; pc.with_rot = c->with_rot ? 1 : 0; pc.rpy_jac = 1;
+    pc.n_fk_links = lk.n; pc.fk_links = lk.ids; pc.T_out = (void *)c->q_out;
+    pc.n_jac_links = lk.n; pc.jac_links = lk.ids; pc.J_out = (void *)c->q_out; pc.with_rot = lk.rot_mask ? 1 : 0; pc.rpy_jac = 1;
     pc.truncation_dist = INFINITY;
     std::shared_ptr<DeviceProgram> dp;
     int rc = get_program(m, &pc, dp);
     if (rc != KIN_OK) return rc;
     kin::GenOptions o;
     o.precision = 0; o.layout = 0; o.want_T = true; o.want_J = true; o.with_rot = pc.with_rot; o.rpy_jac = 1;
-    o.ik = 1; o.block = (int)env_ll("KIN_IK_BLOCK", 128); o.min_blocks = (int)env_ll("KIN_IK_MINB", 1);
+    o.ik = 1; o.ik_rot = lk.n > 1 ? lk.rot_mask : 0u; o.block = (int)env_ll("KIN_IK_BLOCK", 128); o.min_blocks = (int)env_ll("KIN_IK_MINB", 1);
     std::shared_ptr<JitKernel> k = get_jit_with(m, dp.get(), o, "kin_ik_kernel");
-    if (!k) return ik_solve_coll(m, c);
+    if (!k) return ik_solve_coll(m, c, lk);
     kin::IkArgs a;
     std::memset(&a, 0, sizeof a);
     a.targets = c->targets; a.q0 = c->q0; a.q_out = c->q_out; a.f_out = c->f_out; a.iters_out = c->iters_out;
@@ -1742,29 +1759,78 @@ int kin_ik_solve(KinModel *m, const KinIkCall *c) {
     return KIN_OK;
 }
 
-// kin_ik_solve plus the self-collision pairs as a hard constraint: always the augmented-Lagrangian loop of ik_solve_coll.
-// Every argument is checked before anything is launched.
-int kin_ik_solve_self(KinModel *m, const KinIkCall *c, double self_margin, void *self_dmin_out) {
+// The checks every solve makes before anything is launched (collision and pair table: ik_solve_checked).
+int ik_check_call(KinModel *m, const KinIkCall *c, const char *what) {
     if (!m || !c) return fail(KIN_ERR_INVALID_ARGUMENT, "null model or call");
     if (c->n < 0 || (c->n > 0 && (!c->targets || !c->q0 || !c->q_out || !c->f_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
     if (c->iters < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative iteration count");
     const int nd = m->hm.n_dof();
-    if (nd < 1 || nd > kin::IKC_MAX_DOF) return fail(KIN_ERR_LIMIT, "kin_ik_solve_self: 1..20 configuration columns");
-    if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
-    if (std::isnan(self_margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_self: self_margin is NaN");
+    if (nd < 1 || nd > kin::IKC_MAX_DOF) return fail(KIN_ERR_LIMIT, std::string(what) + ": 1..20 configuration columns");
+    return KIN_OK;
+}
+
+// kin_ik_solve_self / kin_ik_solve_links: the pair table (self_collision != 0) and the sphere / box tables
+// (collision != 0) are checked before anything is launched, then the common path.
+int ik_solve_checked(KinModel *m, const KinIkCall *c, const IkLinks &lk, bool self_collision, double self_margin,
+                     void *self_dmin_out, const char *what) {
+    if (self_collision && std::isnan(self_margin)) return fail(KIN_ERR_INVALID_ARGUMENT, std::string(what) + ": self_margin is NaN");
     IkSelfBlock sb;
-    {
-        std::lock_guard<std::mutex> lock(m->mu);
-        sb.pairs = m->self_pairs;
+    if (self_collision) {
+        {
+            std::lock_guard<std::mutex> lock(m->mu);
+            sb.pairs = m->self_pairs;
+        }
+        if (!sb.pairs) return fail(KIN_ERR_INVALID_ARGUMENT, std::string(what) + ": the model has no pair table (kin_model_set_self_pairs)");
     }
-    if (!sb.pairs) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_self: the model has no pair table (kin_model_set_self_pairs)");
     if (c->collision && (m->hm.n_sph < 1 || m->hm.n_box < 1))
         return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: collision requested but the model has no spheres / no boxes");
     if (c->collision && std::isnan(c->margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: margin is NaN");
     if (c->n == 0) return KIN_OK;
+    if (!self_collision) return c->collision ? ik_solve_coll(m, c, lk) : ik_solve_pose(m, c, lk);
     sb.margin = self_margin;
     sb.dmin_out = self_dmin_out;
-    return ik_solve_coll(m, c, &sb);
+    return ik_solve_coll(m, c, lk, &sb);
+}
+
+}  // namespace
+extern "C" {
+
+int kin_ik_solve(KinModel *m, const KinIkCall *c) {
+    int rc = ik_check_call(m, c, "kin_ik_solve");
+    if (rc != KIN_OK) return rc;
+    if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
+    if (c->n == 0) return KIN_OK;
+    if (c->collision) return ik_solve_coll(m, c, ik_one_link(c));
+    return ik_solve_pose(m, c, ik_one_link(c));
+}
+
+// kin_ik_solve plus the self-collision pairs as a hard constraint: always the augmented-Lagrangian loop of ik_solve_coll.
+// Every argument is checked before anything is launched.
+int kin_ik_solve_self(KinModel *m, const KinIkCall *c, double self_margin, void *self_dmin_out) {
+    int rc = ik_check_call(m, c, "kin_ik_solve_self");
+    if (rc != KIN_OK) return rc;
+    if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
+    return ik_solve_checked(m, c, ik_one_link(c), true, self_margin, self_dmin_out, "kin_ik_solve_self");
+}
+
+// Several links at once (extension): kin_ik_solve / kin_ik_solve_self on f = sum_l |e_l|^2.  One link is exactly the
+// call of those two.  Every argument is checked before anything is launched.
+int kin_ik_solve_links(KinModel *m, const KinIkCall *c, int32_t n_links, const int32_t *link_ids, const int32_t *with_rots,
+                       int32_t self_collision, double self_margin, void *self_dmin_out) {
+    int rc = ik_check_call(m, c, "kin_ik_solve_links");
+    if (rc != KIN_OK) return rc;
+    if (n_links < 1 || n_links > KIN_IK_MAX_LINKS) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_links: 1..KIN_IK_MAX_LINKS links");
+    if (!link_ids || !with_rots) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_links: null link_ids / with_rots");
+    IkLinks lk;
+    lk.n = n_links;
+    for (int l = 0; l < n_links; ++l) {
+        if (link_ids[l] < 1 || link_ids[l] > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
+        for (int k = 0; k < l; ++k)
+            if (link_ids[k] == link_ids[l]) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve_links: repeated link id");
+        lk.ids[l] = link_ids[l];
+        if (with_rots[l]) lk.rot_mask |= 1u << l;
+    }
+    return ik_solve_checked(m, c, lk, self_collision != 0, self_margin, self_dmin_out, "kin_ik_solve_links");
 }
 
 // FP64 peak probe (the denominator of the "FP64 pipe" column of the rooflines): every thread runs 8 independent

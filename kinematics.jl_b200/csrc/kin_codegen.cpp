@@ -11,9 +11,9 @@ namespace kin {
 
 std::string GenOptions::key() const {
     char b[200];
-    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d S%d.%d.%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d", precision, layout, (int)want_T, (int)want_J,
+    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d S%d.%d.%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d Q%x", precision, layout, (int)want_T, (int)want_J,
                   (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, (int)ws, block, min_blocks, qbatch, sched, epoch, pf_dist,
-                  ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min, const_fill);
+                  ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min, const_fill, ik_rot);
     return b;
 }
 
@@ -427,6 +427,7 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
     // the tests read the generated text); the skeleton drops the listed ones at compile time.
     const bool cfill = o.const_fill && o.layout == 0 && !o.warp && !o.ik && !o.ws && (!out.const_T.empty() || !out.const_J.empty());
     c << "#define KCFILL " << (cfill ? 1 : 0) << "\n";
+    if (o.ik && h.n_fk > 1) c << "#define KIKROT 0x" << std::hex << o.ik_rot << std::dec << "u\n";
     c << "namespace kin {\n";
     for (int a = 0; a < 2; ++a) {
         const std::vector<std::pair<int, double>> &tab = a ? out.const_J : out.const_T;

@@ -38,6 +38,7 @@ struct GenOptions {
     int pf_dist = 0;            //    sched: epochs the L2 prefetch runs ahead (0: none)
     int warp = 0;               // 1: small-batch kernel, one WARP per configuration (lane = sphere in phase 2)
     int ik = 0;                 // 1: the batched Levenberg-Marquardt IK kernel around phase 1 (one link: T + rpy-Jacobian)
+    unsigned ik_rot = 0;        //    ik with several links: bit l = link l has its rotation rows (KIKROT; unused for one link)
     int grad_mode = -1;         // >= 0: the gradient mode as a compile-time constant (only that code path is compiled in)
     int fd_cold = 0;            // 1: the rare direct-FD fallback of the series gradient is an out-of-line call
     int ksync = 0;              // 1: CTA-wide barrier after every node of phase 1 (the warps of a CTA then fetch the

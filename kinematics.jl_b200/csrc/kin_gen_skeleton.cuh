@@ -245,22 +245,29 @@ __device__ __forceinline__ void phase2b_group(const int s0, const int ge, const 
 // (inverse_kinematics.jl:52-63), accept / reject with the damping scaled by 0.3 / 4.  Angle residuals are wrapped to
 // (-pi, pi].  A problem stops on its own when f < ftol.  The reference drives the same evaluations with NLopt SLSQP
 // (third party); this replaces the per-iteration host round trips of a solver callback by a device-resident loop.
+// SEVERAL LINKS (kin_ik_solve_links, extension): phase 1 gives the KNFK link transforms and Jacobians, the objective
+// is f = sum_l |e_l|^2 and H = sum_l J_l'J_l, g = sum_l J_l'e_l, accumulated link by link and row by row; the targets are
+// [n][6 KNFK].  Bit l of KIKROT (generated for more than one link; one link: KROWS decides) gives link l its rotation
+// rows; the others contribute their 3 position rows.
 // =====================================================================================================================
+#ifndef KIKROT
+#define KIKROT (KROWS == 6 ? 1u : 0u)
+#endif
 extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_ik_kernel(const __grid_constant__ kin::IkArgs A) {
     using namespace kin;
-    constexpr int BS = KBS, ND = KND, ROWS = KROWS;
+    constexpr int BS = KBS, ND = KND, ROWS = KROWS, NL = KNFK;
     const long long li = (long long)blockIdx.x * BS + threadIdx.x;      // position in the active list
     if (li >= A.n) return;
     const long long n = A.idx ? A.idx[li] : li;                         // problem
     const real PI = real(3.14159265358979323846);
-    real q[ND], qt[ND], g[ND], tg[6], H[ND][ND];
+    real q[ND], qt[ND], g[ND], tg[6 * NL], H[ND][ND];
     {
         const real *q0 = reinterpret_cast<const real *>(A.q0) + n * ND;
-        const real *tp = reinterpret_cast<const real *>(A.targets) + n * 6;
+        const real *tp = reinterpret_cast<const real *>(A.targets) + n * 6 * NL;
         #pragma unroll
         for (int c = 0; c < ND; ++c) { q[c] = q0[c]; qt[c] = q0[c]; g[c] = real(0); }
         #pragma unroll
-        for (int i = 0; i < 6; ++i) tg[i] = tp[i];
+        for (int i = 0; i < 6 * NL; ++i) tg[i] = tp[i];
         #pragma unroll
         for (int a = 0; a < ND; ++a)
             #pragma unroll
@@ -270,10 +277,11 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_ik_kernel(const __g
     int it = 0;
     #pragma unroll 1
     for (;; ++it) {
-        // ---- evaluate at qt: link transform Tl (3x4 column-major) and Euler-rate Jacobian Jm[j * ROWS + r] ----
-        real Tl[12], Jm[ROWS * ND];
+        // ---- evaluate at qt: link transforms Tl[12 l + .] (3x4 column-major) and Euler-rate Jacobians
+        //      Jm[(l ND + j) ROWS + r] ----
+        real Tl[12 * NL], Jm[ROWS * ND * NL];
         #pragma unroll
-        for (int k = 0; k < ROWS * ND; ++k) Jm[k] = real(0);
+        for (int k = 0; k < ROWS * ND * NL; ++k) Jm[k] = real(0);
         {
             #define KQ(c) qt[c]
             #define KST_T(k, v) Tl[k] = (v)
@@ -283,26 +291,32 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_ik_kernel(const __g
             #define KSYNC()
 #include "kin_gen_phase1.inc"
         }
-        real e[ROWS];
+        real e[6 * NL];
         #pragma unroll
-        for (int i = 0; i < 3; ++i) e[i] = Tl[9 + i] - tg[i];
-        if (ROWS == 6) {   // rpy(T), transform.jl:45-48 (RotZYX): R[r][c] = Tl[c*3 + r]
-            const real yaw = atan2_(Tl[1], Tl[0]);
-            real s1, c1;
-            sincos_(yaw, &s1, &c1);
-            const real pitch = atan2_(-Tl[2], sqrt_(fma_(Tl[5], Tl[5], Tl[8] * Tl[8])));
-            const real roll = atan2_(fma_(Tl[6], s1, -(Tl[7] * c1)), fma_(Tl[4], c1, -(Tl[3] * s1)));
-            const real ang[3] = {roll - tg[3], pitch - tg[4], yaw - tg[5]};
+        for (int l = 0; l < NL; ++l) {
+            const real *T = Tl + 12 * l, *t = tg + 6 * l;
             #pragma unroll
-            for (int i = 0; i < 3; ++i) {            // wrap to (-pi, pi]
-                real a = ang[i];
-                a = a - real(2) * PI * floor((a + PI) / (real(2) * PI));
-                e[3 + i] = a;
+            for (int i = 0; i < 3; ++i) e[6 * l + i] = T[9 + i] - t[i];
+            if ((KIKROT >> l) & 1u) {   // rpy(T), transform.jl:45-48 (RotZYX): R[r][c] = T[c*3 + r]
+                const real yaw = atan2_(T[1], T[0]);
+                real s1, c1;
+                sincos_(yaw, &s1, &c1);
+                const real pitch = atan2_(-T[2], sqrt_(fma_(T[5], T[5], T[8] * T[8])));
+                const real roll = atan2_(fma_(T[6], s1, -(T[7] * c1)), fma_(T[4], c1, -(T[3] * s1)));
+                const real ang[3] = {roll - t[3], pitch - t[4], yaw - t[5]};
+                #pragma unroll
+                for (int i = 0; i < 3; ++i) {            // wrap to (-pi, pi]
+                    real a = ang[i];
+                    a = a - real(2) * PI * floor((a + PI) / (real(2) * PI));
+                    e[6 * l + 3 + i] = a;
+                }
             }
         }
         real ft = real(0);
         #pragma unroll
-        for (int r = 0; r < ROWS; ++r) ft = fma_(e[r], e[r], ft);
+        for (int l = 0; l < NL; ++l)
+            #pragma unroll
+            for (int r = 0; r < (((KIKROT >> l) & 1u) ? 6 : 3); ++r) ft = fma_(e[6 * l + r], e[6 * l + r], ft);
         const bool ok = ft < f;
         if (it > 0) {
             lam *= ok ? real(0.3) : real(4.0);
@@ -315,13 +329,18 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_ik_kernel(const __g
                 q[a] = qt[a];
                 real ga = real(0);
                 #pragma unroll
-                for (int r = 0; r < ROWS; ++r) ga = fma_(Jm[a * ROWS + r], e[r], ga);
+                for (int l = 0; l < NL; ++l)
+                    #pragma unroll
+                    for (int r = 0; r < (((KIKROT >> l) & 1u) ? 6 : 3); ++r) ga = fma_(Jm[(l * ND + a) * ROWS + r], e[6 * l + r], ga);
                 g[a] = ga;
                 #pragma unroll
                 for (int b = 0; b <= a; ++b) {
                     real hab = real(0);
                     #pragma unroll
-                    for (int r = 0; r < ROWS; ++r) hab = fma_(Jm[a * ROWS + r], Jm[b * ROWS + r], hab);
+                    for (int l = 0; l < NL; ++l)
+                        #pragma unroll
+                        for (int r = 0; r < (((KIKROT >> l) & 1u) ? 6 : 3); ++r)
+                            hab = fma_(Jm[(l * ND + a) * ROWS + r], Jm[(l * ND + b) * ROWS + r], hab);
                     H[a][b] = hab;
                 }
             }

@@ -21,6 +21,8 @@
 // compactions a problem that stops stays in the list (its evaluation is repeated, results ignored).
 // SELF-COLLISION (kin_ik_solve_self): a kin_self_collision launch between 1. and 2. evaluates the model's sphere pairs at
 // the same trial points, and the SELF instances of the step kernels add the pairs as a second constraint block.
+// SEVERAL LINKS (kin_ik_solve_links): kin_eval returns every link's transform and Euler-rate Jacobian, and the LINKS
+// instances of the step kernels sum the links' residual blocks into the objective and the normal equations.
 #pragma once
 
 #include <cstdint>
@@ -57,8 +59,40 @@ struct IkCollSelfArgs : IkCollArgs {
     const double *VP, *GP;           // pair values [P][ld] and gradients [P][ND][ld] at the trial points (list position)
     double *multP;                   // pair multipliers [P][ld] (problem)
 };
-template <bool SELF>
-using IkcArgsT = typename std::conditional<SELF, IkCollSelfArgs, IkCollArgs>::type;
+// The multi-link pose block of kin_ik_solve_links (LINKS instances of the step kernels): the objective is
+// f = sum_l |e_l|^2 over n_links links.  T holds 12 rows per link and J ROWS n_dof rows per link (ROWS = 6 when any link
+// has rotation, as kin_eval writes them); a link whose bit of rot_mask is clear contributes its 3 position rows only.
+// The targets are [n][6 n_links].  Derived from IkCollSelfArgs so that one struct carries both blocks.
+constexpr int IKC_MAX_LINKS = 4;        // KIN_IK_MAX_LINKS
+struct IkCollLinksArgs : IkCollSelfArgs {
+    int n_links;
+    unsigned rot_mask;
+};
+template <bool SELF, bool LINKS = false>
+using IkcArgsT = typename std::conditional<LINKS, IkCollLinksArgs,
+                                           typename std::conditional<SELF, IkCollSelfArgs, IkCollArgs>::type>::type;
+
+// e_l = [p - p_t; rpy - rpy_t] of one link (planning.jl:114-138 sign), angles wrapped; Tn points at the link's 12 rows
+// of stride ld, tg at its 6 target values.  The same operations as the residual block of the single-link kernels.
+__device__ __forceinline__ void ikc_link_residual(const double *Tn, long long ld, const double *tg, bool rot, double e[6]) {
+    const double PI = 3.14159265358979323846;
+    #pragma unroll
+    for (int k = 0; k < 3; ++k) e[k] = Tn[(9 + k) * ld] - tg[k];
+    if (rot) {
+        const double r00 = Tn[0], r10 = Tn[ld], r20 = Tn[2 * ld], r01 = Tn[3 * ld], r11 = Tn[4 * ld], r21 = Tn[5 * ld],
+                     r02 = Tn[6 * ld], r12 = Tn[7 * ld], r22 = Tn[8 * ld];
+        const double yaw = atan2(r10, r00);
+        double s1, c1;
+        sincos(yaw, &s1, &c1);
+        const double pitch = atan2(-r20, sqrt(fma(r21, r21, r22 * r22)));
+        const double roll = atan2(fma(r02, s1, -(r12 * c1)), fma(r11, c1, -(r01 * s1)));
+        const double ang[3] = {roll - tg[3], pitch - tg[4], yaw - tg[5]};
+        #pragma unroll
+        for (int k = 0; k < 3; ++k) e[3 + k] = ang[k] - 2.0 * PI * floor((ang[k] + PI) / (2.0 * PI));
+    } else {
+        e[3] = e[4] = e[5] = 0.0;
+    }
+}
 
 // q0 (AoS, caller's) -> q_try and q (SoA); merit +inf so that the first evaluation is accepted
 __global__ void __launch_bounds__(256) ik_coll_init_kernel(const IkCollArgs A, const double *__restrict__ q0, int nd) {
@@ -112,8 +146,10 @@ __host__ __device__ inline size_t ikc_dyn_smem_per_thread(int nd) { return sizeo
 // SELF (kin_ik_solve_self): a second constraint block over the self-collision pairs, the same operations per entry as
 // the sphere block (merit term mu psi_p^2, multiplier update, rank-one update of H and g where psi_p > 0, viol) and the
 // same weight mu, after it.  Written with `if constexpr`: the instances without it are the code they were before.
-template <int NDT, bool ROT, bool SELF = false>
-__global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> A) {
+// LINKS (kin_ik_solve_links, n_links >= 2): the residual and the J'J / J'e accumulation run over the links, link by
+// link and row by row, in the order the one-warp kernel uses too.
+template <int NDT, bool ROT, bool SELF = false, bool LINKS = false>
+__global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF, LINKS> A) {
     extern __shared__ double ikc_smem[];
     constexpr int NDA = NDT > 0 ? NDT : IKC_MAX_DOF;
     const int ND = NDT > 0 ? NDT : A.nd;
@@ -129,8 +165,12 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> 
     IkcStore<NDT> W(ikc_smem, (int)threadIdx.x, (int)blockDim.x, ND);
 
     // ---- residual at the trial point: e = [p - p_t; rpy - rpy_t] (planning.jl:114-138 sign), angles wrapped ----
-    double e[ROWS];
-    {
+    double e[LINKS ? 6 * IKC_MAX_LINKS : ROWS];
+    if constexpr (LINKS) {
+        #pragma unroll
+        for (int l = 0; l < IKC_MAX_LINKS; ++l)
+            if (l < A.n_links) ikc_link_residual(A.T + 12 * l * ld + i, ld, A.targets + n * 6 * A.n_links + 6 * l, (A.rot_mask >> l) & 1u, e + 6 * l);
+    } else {
         const double *Tn = A.T + i, *tg = A.targets + n * 6;
         #pragma unroll
         for (int i = 0; i < 3; ++i) e[i] = Tn[(9 + i) * ld] - tg[i];
@@ -148,8 +188,19 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> 
         }
     }
     double ft = 0.0;
-    #pragma unroll
-    for (int r = 0; r < ROWS; ++r) ft = fma(e[r], e[r], ft);
+    if constexpr (LINKS) {
+        #pragma unroll
+        for (int l = 0; l < IKC_MAX_LINKS; ++l)
+            if (l < A.n_links) {
+                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
+                #pragma unroll
+                for (int r = 0; r < 6; ++r)
+                    if (r < rl) ft = fma(e[6 * l + r], e[6 * l + r], ft);
+            }
+    } else {
+        #pragma unroll
+        for (int r = 0; r < ROWS; ++r) ft = fma(e[r], e[r], ft);
+    }
 
     // ---- merit under the CURRENT multipliers ----
     double phi_t = ft;
@@ -184,16 +235,44 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> 
             #pragma unroll
             for (int b = 0; b <= a; ++b) W.H(a, b) = 0.0;
         }
-        #pragma unroll
-        for (int r = 0; r < ROWS; ++r) {
+        if constexpr (LINKS) {
             #pragma unroll
-            for (int a = 0; a < ND; ++a) W.v(a) = A.J[(long long)(a * ROWS + r) * ld + i];
-            #pragma unroll
-            for (int a = 0; a < ND; ++a) {
-                const double ja = W.v(a);
-                W.g(a) = fma(ja, e[r], W.g(a));
+            for (int l = 0; l < IKC_MAX_LINKS; ++l) {
+                if (l >= A.n_links) break;
+                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
+                const double *Jl = A.J + (long long)l * ROWS * ND * ld;
+                double el[6];
                 #pragma unroll
-                for (int b = 0; b <= a; ++b) W.H(a, b) = fma(ja, W.v(b), W.H(a, b));
+                for (int r = 0; r < 6; ++r) el[r] = e[6 * l + r];
+                #pragma unroll 1
+                for (int r = 0; r < rl; ++r) {
+                    #pragma unroll
+                    for (int a = 0; a < ND; ++a) W.v(a) = Jl[(long long)(a * ROWS + r) * ld + i];
+                    double er = el[0];
+                    #pragma unroll
+                    for (int k = 1; k < 6; ++k)
+                        if (r == k) er = el[k];
+                    #pragma unroll
+                    for (int a = 0; a < ND; ++a) {
+                        const double ja = W.v(a);
+                        W.g(a) = fma(ja, er, W.g(a));
+                        #pragma unroll
+                        for (int b = 0; b <= a; ++b) W.H(a, b) = fma(ja, W.v(b), W.H(a, b));
+                    }
+                }
+            }
+        } else {
+            #pragma unroll
+            for (int r = 0; r < ROWS; ++r) {
+                #pragma unroll
+                for (int a = 0; a < ND; ++a) W.v(a) = A.J[(long long)(a * ROWS + r) * ld + i];
+                #pragma unroll
+                for (int a = 0; a < ND; ++a) {
+                    const double ja = W.v(a);
+                    W.g(a) = fma(ja, e[r], W.g(a));
+                    #pragma unroll
+                    for (int b = 0; b <= a; ++b) W.H(a, b) = fma(ja, W.v(b), W.H(a, b));
+                }
             }
         }
         double phi_n = ft, viol = -CUDART_INF;
@@ -331,8 +410,9 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF> 
 // touches one sector per matrix entry (the state is SoA over problems), measured 1.7 ms against 1.06 ms per launch on
 // 42 k problems of 18 columns, 9.3 against 4.6 ms on 262 k.
 // SELF: the pair block of ik_coll_step_kernel<., ., true>, with the same operations per entry in the same order.
-template <bool ROT, bool SELF = false>
-__global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<SELF> A) {
+// LINKS: the multi-link pose block of ik_coll_step_kernel<., ., ., true>, likewise.
+template <bool ROT, bool SELF = false, bool LINKS = false>
+__global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<SELF, LINKS> A) {
     constexpr int MAXC = IKC_MAX_DOF, ROWS = ROT ? 6 : 3;
     constexpr unsigned FULL = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -349,8 +429,12 @@ __global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<S
     const int a = mine ? lane : 0;
 
     // ---- residual and merit at the trial point: every lane computes them (broadcast loads), as the one-thread kernel does ----
-    double e[ROWS];
-    {
+    double e[LINKS ? 6 * IKC_MAX_LINKS : ROWS];
+    if constexpr (LINKS) {
+        #pragma unroll
+        for (int l = 0; l < IKC_MAX_LINKS; ++l)
+            if (l < A.n_links) ikc_link_residual(A.T + 12 * l * ld + i, ld, A.targets + n * 6 * A.n_links + 6 * l, (A.rot_mask >> l) & 1u, e + 6 * l);
+    } else {
         const double *Tn = A.T + i, *tg = A.targets + n * 6;
         #pragma unroll
         for (int k = 0; k < 3; ++k) e[k] = Tn[(9 + k) * ld] - tg[k];
@@ -368,8 +452,19 @@ __global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<S
         }
     }
     double ft = 0.0;
-    #pragma unroll
-    for (int r = 0; r < ROWS; ++r) ft = fma(e[r], e[r], ft);
+    if constexpr (LINKS) {
+        #pragma unroll
+        for (int l = 0; l < IKC_MAX_LINKS; ++l)
+            if (l < A.n_links) {
+                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
+                #pragma unroll
+                for (int r = 0; r < 6; ++r)
+                    if (r < rl) ft = fma(e[6 * l + r], e[6 * l + r], ft);
+            }
+    } else {
+        #pragma unroll
+        for (int r = 0; r < ROWS; ++r) ft = fma(e[r], e[r], ft);
+    }
     double phi_t = ft;
     for (int s = 0; s < S; ++s) {
         const double d = A.V[s * ld + i];
@@ -399,14 +494,40 @@ __global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<S
         g_a = 0.0;
         #pragma unroll
         for (int b = 0; b < MAXC; ++b) Hrow[b] = 0.0;
-        #pragma unroll
-        for (int r = 0; r < ROWS; ++r) {
-            const double ja = mine ? A.J[(long long)(a * ROWS + r) * ld + i] : 0.0;
-            g_a = fma(ja, e[r], g_a);
+        if constexpr (LINKS) {
             #pragma unroll
-            for (int b = 0; b < MAXC; ++b) {
-                const double jb = __shfl_sync(FULL, ja, b);
-                if (b <= lane) Hrow[b] = fma(ja, jb, Hrow[b]);
+            for (int l = 0; l < IKC_MAX_LINKS; ++l) {
+                if (l >= A.n_links) break;
+                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
+                const double *Jl = A.J + (long long)l * ROWS * ND * ld;
+                double el[6];
+                #pragma unroll
+                for (int r = 0; r < 6; ++r) el[r] = e[6 * l + r];
+                #pragma unroll 1
+                for (int r = 0; r < rl; ++r) {
+                    const double ja = mine ? Jl[(long long)(a * ROWS + r) * ld + i] : 0.0;
+                    double er = el[0];
+                    #pragma unroll
+                    for (int k = 1; k < 6; ++k)
+                        if (r == k) er = el[k];
+                    g_a = fma(ja, er, g_a);
+                    #pragma unroll
+                    for (int b = 0; b < MAXC; ++b) {
+                        const double jb = __shfl_sync(FULL, ja, b);
+                        if (b <= lane) Hrow[b] = fma(ja, jb, Hrow[b]);
+                    }
+                }
+            }
+        } else {
+            #pragma unroll
+            for (int r = 0; r < ROWS; ++r) {
+                const double ja = mine ? A.J[(long long)(a * ROWS + r) * ld + i] : 0.0;
+                g_a = fma(ja, e[r], g_a);
+                #pragma unroll
+                for (int b = 0; b < MAXC; ++b) {
+                    const double jb = __shfl_sync(FULL, ja, b);
+                    if (b <= lane) Hrow[b] = fma(ja, jb, Hrow[b]);
+                }
             }
         }
         double phi_n = ft, viol = -CUDART_INF;

@@ -77,6 +77,25 @@ def ik_objective(m: Mechanism, link, joints, target_pose, with_rot=True):
     return f, g
 
 
+MAX_LINKS = 4      # KIN_IK_MAX_LINKS
+
+
+def _link_list(link, with_rot, what):
+    """``link``: one Link (-> None: the single-link calls) or a list of links (extension, ``kin_ik_solve_links``) with
+    ``with_rot`` a bool or one bool per link -> (links, with_rots).  Checked before anything touches a device."""
+    if not isinstance(link, (list, tuple)):
+        return None
+    links = list(link)
+    if not 1 <= len(links) <= MAX_LINKS:
+        raise ValueError("%s: 1..%d links, got %d" % (what, MAX_LINKS, len(links)))
+    if len({id(l) for l in links}) != len(links) or len({getattr(l, "id", None) for l in links}) != len(links):
+        raise ValueError("%s: the links must be distinct" % what)
+    rots = list(with_rot) if isinstance(with_rot, (list, tuple)) else [with_rot] * len(links)
+    if len(rots) != len(links):
+        raise ValueError("%s: %d links but %d with_rot flags" % (what, len(links), len(rots)))
+    return links, [bool(w) for w in rots]
+
+
 def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iters=100, ftol=1e-10, lambda0=1e-2,
                     sscc=None, sdf=None, margin=0.02, coll_weight=100.0, ctol=1e-6, self_margin=None, self_pairs=None):
     """The device-resident batched solve (``kin_ik_solve``).  ``targets`` (N, 6), ``q0`` (N, n_dof) CUDA tensors.
@@ -96,8 +115,13 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
     constrain the solve).  Returns (q, f, iterations[, dmin], self_dmin), self_dmin (N,) the smallest pair distance at
     q.  On the Fetch sphere fixture the default policy keeps a pair of constant distance that overlaps by 5.5 mm in
     every configuration, which no solver can satisfy: pass ``self_collision_pairs(sscc, joints,
-    ignore=[("wrist_flex_link", "elbow_flex_link")])`` (64 pairs) there."""
+    ignore=[("wrist_flex_link", "elbow_flex_link")])`` (64 pairs) there.
+
+    Several links (extension; ``kin_ik_solve_links``): ``link`` a list of up to 4 distinct links, ``with_rot`` a bool
+    or one bool per link, ``targets`` (N, 6 L) with the 6 values of each link in link order; the objective is the sum
+    of the links' |e_l|^2 and everything else works as above.  A single Link keeps the single-link calls."""
     import torch
+    multi = _link_list(link, with_rot, "ik_solve_device")
     if self_margin is not None:
         if sscc is None:
             raise ValueError("ik_solve_device: self_margin needs the collision checker sscc (its spheres form the pairs)")
@@ -119,12 +143,14 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
     hi = np.ascontiguousarray([j.upper_limit for j in joints] + [np.inf] * nb, dtype=np.float64)
     tg = torch.as_tensor(targets, dtype=torch.float64, device="cuda").contiguous()
     N, nd = q0.shape
-    assert tg.shape == (N, 6) and nd == dm.n_dof
+    assert tg.shape == (N, 6 * (len(multi[0]) if multi else 1)) and nd == dm.n_dof
     q = torch.empty_like(q0)
     f = torch.empty(N, dtype=torch.float64, device="cuda")
     its = torch.empty(N, dtype=torch.int32, device="cuda")
     c = _lib.KinIkCall()
-    c.n, c.link_id, c.with_rot, c.iters, c.ftol, c.lambda0 = N, link.id, int(with_rot), int(iters), float(ftol), float(lambda0)
+    c.n, c.iters, c.ftol, c.lambda0 = N, int(iters), float(ftol), float(lambda0)
+    if not multi:
+        c.link_id, c.with_rot = link.id, int(with_rot)
     c.targets, c.q0 = tg.data_ptr(), q0.data_ptr()
     c.lower, c.upper = lo.ctypes.data_as(C.POINTER(C.c_double)), hi.ctypes.data_as(C.POINTER(C.c_double))
     c.q_out, c.f_out, c.iters_out = q.data_ptr(), f.data_ptr(), its.data_ptr()
@@ -132,12 +158,22 @@ def ik_solve_device(m: Mechanism, link, joints, targets, q0, with_rot=True, iter
     if collide:
         dmin = torch.empty(N, dtype=torch.float64, device="cuda")
         c.collision, c.margin, c.coll_weight, c.ctol, c.dmin_out = 1, float(margin), float(coll_weight), float(ctol), dmin.data_ptr()
-    if self_margin is None:
+    if self_margin is not None:
+        c.coll_weight, c.ctol = float(coll_weight), float(ctol)
+        self_dmin = torch.empty(N, dtype=torch.float64, device="cuda")
+    if multi:
+        ids = np.ascontiguousarray([l.id for l in multi[0]], dtype=np.int32)
+        rots = np.ascontiguousarray(multi[1], dtype=np.int32)
+        ip = C.POINTER(C.c_int32)
+        _lib.check(_lib.lib().kin_ik_solve_links(dm.h, C.byref(c), len(ids), ids.ctypes.data_as(ip), rots.ctypes.data_as(ip),
+                                                 int(self_margin is not None), float(self_margin or 0.0),
+                                                 self_dmin.data_ptr() if self_margin is not None else None))
+    elif self_margin is None:
         _lib.check(_lib.lib().kin_ik_solve(dm.h, C.byref(c)))
+    else:
+        _lib.check(_lib.lib().kin_ik_solve_self(dm.h, C.byref(c), float(self_margin), self_dmin.data_ptr()))
+    if self_margin is None:
         return (q, f, its, dmin) if collide else (q, f, its)
-    c.coll_weight, c.ctol = float(coll_weight), float(ctol)
-    self_dmin = torch.empty(N, dtype=torch.float64, device="cuda")
-    _lib.check(_lib.lib().kin_ik_solve_self(dm.h, C.byref(c), float(self_margin), self_dmin.data_ptr()))
     return (q, f, its, dmin, self_dmin) if collide else (q, f, its, self_dmin)
 
 
@@ -177,14 +213,20 @@ def inverse_kinematics_batch(m: Mechanism, link, joints, targets, q0, with_rot=T
     pair that overlaps by 5.5 mm in every configuration.
     ``targets`` (N, 6) [x y z roll pitch yaw], ``q0`` (N, n_dof).  Returns (q, f) with f the pose objective
     (and the smallest signed sphere distance per problem with ``return_dmin``; with ``self_margin`` and ``return_dmin``:
-    (q, f, dmin or None, self_dmin))."""
+    (q, f, dmin or None, self_dmin)).
+    Several links (extension, ``kin_ik_solve_links``): ``link`` a list, ``with_rot`` a bool or a per-link list,
+    ``targets`` (N, 6 L); f is the sum over the links, and a problem is solved when f <= tol^2 (every residual of
+    every link within tol) and the constraints hold."""
     import torch
+    multi = _link_list(link, with_rot, "inverse_kinematics_batch")
     selfc = self_margin is not None
     if selfc and sscc is None:
         raise ValueError("inverse_kinematics_batch: self_margin needs the collision checker sscc")
     collide = sscc is not None and sdf is not None
     targets = torch.as_tensor(targets, dtype=torch.float64, device="cuda")
     q0 = torch.as_tensor(q0, dtype=torch.float64, device="cuda")
+    if targets.dim() != 2 or targets.shape != (q0.shape[0], 6 * (len(multi[0]) if multi else 1)):
+        raise ValueError("inverse_kinematics_batch: targets must be (N, 6 * number of links), got %s" % (tuple(targets.shape),))
 
     def pose_only(tg, qs):
         return ik_solve_device(m, link, joints, tg, qs, with_rot=with_rot, iters=iters, ftol=ftol)[:2]
@@ -247,9 +289,15 @@ def inverse_kinematics(m: Mechanism, link, joints, target_pose, sscc=None, sdf=N
     collision-free warm start (:8-13).  ``self_margin`` (extension): also the self-collision constraint
     ``SelfIneqConst(sscc, joints, 1, self_margin, self_pairs)`` as a second inequality, as ``plan_trajectory`` adds it;
     the warm start stays unconstrained.  Every evaluation runs on the GPU (N = 1).  Returns (q, scipy result); the
-    mechanism is left at the solution like the reference leaves it."""
+    mechanism is left at the solution like the reference leaves it.
+    Several links (extension): ``link`` a list of links, ``target_pose`` a list of as many poses (Transform or
+    6-vector), ``with_rot`` a bool or one per link; the objective is the sum of the links' f_objective, the stacked
+    ``_pose_residual`` of ``kin_pose_residual_multi``."""
     from scipy.optimize import minimize
     from .planning import IneqConst, SelfIneqConst, scipynize
+    multi = _link_list(link, with_rot, "inverse_kinematics")
+    if multi and (not isinstance(target_pose, (list, tuple)) or len(target_pose) != len(multi[0])):
+        raise ValueError("inverse_kinematics: one target pose per link")
     if self_margin is not None and sscc is None:
         raise ValueError("inverse_kinematics: self_margin needs the collision checker sscc")
     nb = 3 if m.with_base else 0
@@ -259,6 +307,9 @@ def inverse_kinematics(m: Mechanism, link, joints, target_pose, sscc=None, sdf=N
 
     def fun(x):
         set_joint_angles(m, joints, np.asarray(x, dtype=np.float64))
+        if multi:
+            f, g = _pose_residual(m, multi[0], joints, list(target_pose), multi[1], _lib.POSE_IK_OBJECTIVE)
+            return float(f[0]), g[0].double().cpu().numpy()
         return ik_objective(m, link, joints, target_pose, with_rot)
 
     def solve(x0, constraints):

@@ -66,7 +66,8 @@ EXPORTS = ["kin_last_error", "kin_abi_version", "kin_build_id", "kin_debug_build
            "kin_eval_host", "kin_fk_links", "kin_fk_jacobian", "kin_collision", "kin_launch_count",
            "kin_query_launch", "kin_sdf_points", "kin_program_dump", "kin_pose_residual", "kin_pose_residual_multi", "kin_probe_fp64",
            "kin_jit_status", "kin_jit_stats", "kin_codegen_dump", "kin_ik_solve", "kin_host_transfer_bytes",
-           "kin_model_set_self_pairs", "kin_model_n_self_pairs", "kin_self_collision", "kin_ik_solve_self"]
+           "kin_model_set_self_pairs", "kin_model_n_self_pairs", "kin_self_collision", "kin_ik_solve_self",
+           "kin_ik_solve_links"]
 
 
 def source_files():
@@ -218,6 +219,8 @@ def lib():
         L.kin_probe_fp64.argtypes = [_dp, _dp, _dp]
         L.kin_ik_solve.argtypes = [C.c_void_p, C.POINTER(KinIkCall)]
         L.kin_ik_solve_self.argtypes = [C.c_void_p, C.POINTER(KinIkCall), C.c_double, C.c_void_p]
+        L.kin_ik_solve_links.argtypes = [C.c_void_p, C.POINTER(KinIkCall), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+                                         C.c_int32, C.c_double, C.c_void_p]
         L.kin_jit_status.restype = C.c_char_p
         _lp = C.POINTER(C.c_int64)
         L.kin_jit_stats.argtypes = [_lp, _lp, _lp, _lp]
