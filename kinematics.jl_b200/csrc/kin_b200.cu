@@ -403,7 +403,6 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     o.want_grads = o.coll && c->grads_out != nullptr;
     o.want_argmin = o.coll && c->argmin_out != nullptr;
     o.stale = o.want_grads && c->scratch_mode == KIN_SCRATCH_REFERENCE;
-    o.ws = false;
     // Launch shape and code-shape switches, from the sweeps in profiles/ (sweep_jit.py; ms per 2^22 fused configurations):
     //   collision, SoA:   128 threads x 2 CTAs/SM with a CTA-wide barrier after every node of the straight-line phase 1
     //                     (the warps of a CTA then share instruction fetches: the fused kernel is 90 KB of code, far
@@ -414,7 +413,7 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     // small batches: one warp per configuration (kin_gen_skeleton.cuh, KWARP)
     o.warp = use_warp_kernel(c, h) ? 1 : 0;
     if (o.warp) {
-        o.block = 128; o.min_blocks = 1; o.ksync = 0; o.es32 = 0; o.fd_cold = 0;
+        o.block = 128; o.min_blocks = 1; o.ksync = 0; o.es32 = 0;
         o.grad_mode = o.want_grads ? c->grad_mode : -1;
         return o;
     }
@@ -425,7 +424,6 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     o.block = (int)env_ll("KIN_JIT_BLOCK", ((o.coll && tiled) || f32c) ? 256 : 128);
     o.min_blocks = (int)env_ll("KIN_JIT_MINB", o.coll ? ((tiled && !f32c) ? 1 : 2) : 1);
     o.grad_mode = o.want_grads ? c->grad_mode : -1;
-    o.fd_cold = (int)env_ll("KIN_JIT_FD_COLD", 0);
     o.ksync = (int)env_ll("KIN_JIT_KSYNC", (o.coll && !tiled) ? 1 : 0);
     o.es32 = (o.layout == KIN_LAYOUT_SOA && (c->batch_stride ? c->batch_stride : c->n) < (1ll << 32)) ? (int)env_ll("KIN_JIT_ES32", 1) : 0;
     // Models with many columns / spheres (a dual-arm mechanism with the planar base: 18 columns, 19 spheres = 952 B of
@@ -434,18 +432,9 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     // threads per SM -- 96 x 2: 3.27, 128 x 1: 4.87, 160 x 1: 3.88, 192 x 1: 3.28, 224 x 1: 2.84 (interpreting kernel: 6.91);
     // FP32 256 x 1: 2.41, 192 x 2: 1.61, 224 x 2: 1.84, 384 x 1: 1.59, 448 x 1: 1.47 -- so the shape with the most threads
     // that fits is taken (up to what the register file holds: 256 threads at 255 registers, 512 at 128 in FP32).
-    // The joint frames of phase 2 stay in registers at any column count: parking them in the shared scratch instead
-    // (jf_smem, opt-in through KIN_JIT_JF_REGS_MAX) costs threads and measured 4.15 against 2.52 ms at 15 columns,
-    // 6.21 against 2.84 at 18.
-    o.jf_smem = (o.coll && h.n_dof > env_ll("KIN_JIT_JF_REGS_MAX", 32)) ? 1 : 0;
-    // phase 2b: one instance per distinct relevance mask (0, default), or one instance testing the mask at run time (1; -1: when
-    // there are more than KIN_JIT_RTMASK_MIN masks).  Dual-arm model, 13 masks, 18-column loops: the code shrinks from 15.7 k
-    // to 6.4 k instructions, the time does not follow (2^21 configurations, ms per-mask / run-time: 15 columns collision-only
-    // 2.57 / 2.60, fused 3.29 / 3.04; 18 columns 2.84 / 2.99, 3.66 / 3.67): the node barriers already make a CTA share its
-    // instruction fetches.  Kept as a knob.
-    o.rtmask = (int)env_ll("KIN_JIT_RTMASK", 0);
-    o.rtmask_min = (int)env_ll("KIN_JIT_RTMASK_MIN", 6);
-    if (o.coll && (!std::getenv("KIN_JIT_BLOCK") || o.jf_smem)) {
+    // The joint frames of phase 2 stay in registers at any column count: parking them in the shared scratch costs
+    // threads and measured slower (DESIGN 7, round 2d).
+    if (o.coll && !std::getenv("KIN_JIT_BLOCK")) {
         const size_t cta_max = (size_t)(m ? m->dev_smem : 227 * 1024), sm_total = cta_max + 1024;   // 228 KB per SM, 1 KB reserved per CTA
         auto fits = [&](int block, int minb) {
             JitKernel probe;
@@ -536,7 +525,7 @@ kin::JitHeaders jit_headers(const kin::GenSource &g) {
 // per-thread scratch slots of the generated kernel (kin_gen_skeleton.cuh)
 int jit_slots(const kin::GenOptions &o, const kin::ProgHeader &h) {
     if (!o.coll) return 0;
-    return 3 * h.n_sph + (o.stale ? 3 * h.n_dof : 0) + 2 * kin::SPH_GROUP + (o.jf_smem ? 6 * h.n_dof : 0);
+    return 3 * h.n_sph + (o.stale ? 3 * h.n_dof : 0) + 2 * kin::SPH_GROUP;
 }
 
 size_t jit_smem(const kin::GenOptions &o, const kin::ProgHeader &h, const JitKernel &k) {
@@ -1502,15 +1491,7 @@ void launch_ik_coll_step(const kin::IkcArgsT<SELF, LINKS> &a, bool rot, cudaStre
 
 template <bool SELF, bool LINKS>
 void launch_ik_coll_step_any(const kin::IkcArgsT<SELF, LINKS> &a, int nd, int rows, cudaStream_t stream, int dev_smem) {
-    // KIN_IK_STEP=warp sends the step through the one-warp-per-problem kernel (kin_ik_coll.cuh: an independent
-    // parallelisation with bit-identical iterates, kept as a cross-check; measured slower than one thread per problem
-    // at every list length: 18 columns, 42 k problems 1.7 against 1.06 ms, 262 k problems 9.3 against 4.6 ms)
-    const char *step_mode = std::getenv("KIN_IK_STEP");
-    if (step_mode && !std::strcmp(step_mode, "warp")) {
-        const unsigned grid = (unsigned)((a.n_act + 3) / 4);                 // 4 warps = 4 problems per CTA
-        if (rows == 6) kin::ik_coll_step_warp_kernel<true, SELF, LINKS><<<grid, 128, 0, stream>>>(a);
-        else kin::ik_coll_step_warp_kernel<false, SELF, LINKS><<<grid, 128, 0, stream>>>(a);
-    } else switch (nd) {
+    switch (nd) {
 #define KIN_IKC_CASE(N_) case N_: launch_ik_coll_step<N_, SELF, LINKS>(a, rows == 6, stream, dev_smem); break;
         KIN_IKC_CASE(1) KIN_IKC_CASE(2) KIN_IKC_CASE(3) KIN_IKC_CASE(4) KIN_IKC_CASE(5) KIN_IKC_CASE(6)
         KIN_IKC_CASE(7) KIN_IKC_CASE(8) KIN_IKC_CASE(9) KIN_IKC_CASE(10) KIN_IKC_CASE(11) KIN_IKC_CASE(12)

@@ -11,9 +11,9 @@ namespace kin {
 
 std::string GenOptions::key() const {
     char b[200];
-    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d w%d b%d m%d q%d S%d.%d.%d y%d e%d G%d C%d I%d W%d P%d B%d F%d R%d.%d K%d Q%x", precision, layout, (int)want_T, (int)want_J,
-                  (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, (int)ws, block, min_blocks, qbatch, sched, epoch, pf_dist,
-                  ksync, es32, grad_mode, fd_cold, ik, warp, prims, bulk, jf_smem, rtmask, rtmask_min, const_fill, ik_rot);
+    std::snprintf(b, sizeof b, "p%d l%d T%d J%d c%d r%d y%d k%d g%d a%d s%d b%d m%d q%d S%d.%d.%d y%d e%d G%d I%d W%d P%d B%d K%d Q%x", precision, layout, (int)want_T, (int)want_J,
+                  (int)coll, with_rot, rpy_jac, keep_irrelevant, (int)want_grads, (int)want_argmin, (int)stale, block, min_blocks, qbatch, sched, epoch, pf_dist,
+                  ksync, es32, grad_mode, ik, warp, prims, bulk, const_fill, ik_rot);
     return b;
 }
 
@@ -207,11 +207,6 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
                 for (int i = 0; i < 3; ++i) f.a[i] = E.fma(Aj.r[i * 3 + 0], x, E.fma(Aj.r[i * 3 + 1], y, E.mul(Aj.r[i * 3 + 2], z)));
             }
             frames[qcol] = f;
-            if (o.ws || (o.jf_smem && o.coll))       // frames handed over / parked in the shared scratch as they are computed
-                for (int i = 0; i < 6; ++i) {
-                    const Val &v = i < 3 ? f.o[i] : f.a[i - 3];
-                    if (!v.c || o.jf_smem) E.os << "KJF_OUT(" << qcol << ", " << i << ", " << E.str(v) << ");\n";
-                }
             const Val qa = Emitter::V("q" + std::to_string(qcol));
             T = Aj;
             if (jtype == 2) {          // prismatic: pose * Trans(axis * a), mechanism.jl:100-103
@@ -358,10 +353,9 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
 
     // ------------------------------------------------------------------ phase 2: one call per run of equal masks
     std::ostringstream p2;
-    bool rt_mask = false;       // phase 2b tests the relevance mask at run time (one instance) instead of one instance per mask
     if (o.coll) {
         // joint frames of the columns as the consumers of phase 2 see them
-        p2 << "#ifndef KJFR_DEFINED\nconst JFrame<real> jfr[KND] = {\n";
+        p2 << "const JFrame<real> jfr[KND] = {\n";
         for (int j = 0; j < ND; ++j) {
             const Frame &f = frames[j];
             p2 << "  {{";
@@ -369,7 +363,7 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
             for (int i = 0; i < 3; ++i) p2 << (f.set ? E.str(f.a[i]) : std::string("real(0)")) << (i < 2 ? ", " : "}}");
             p2 << (j + 1 < ND ? ",\n" : "\n");
         }
-        p2 << "};\n#endif\n";
+        p2 << "};\n";
         // runs of consecutive spheres with equal relevance mask; groups of up to SPH_GROUP spheres inside a run
         struct Run { int sb, se; unsigned mask; };
         std::vector<Run> runs;
@@ -387,23 +381,18 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
             for (unsigned mk : masks) seen |= mk == r.mask;
             if (!seen) masks.push_back(r.mask);
         }
-        rt_mask = o.rtmask == 1 || (o.rtmask < 0 && (int)masks.size() > o.rtmask_min);
-        p2 << "#if !KWARP\n#pragma unroll 1\nfor (int s0 = 0; s0 < KS;) {\n    int se, mi;\n    unsigned mk;\n";
+        p2 << "#if !KWARP\n#pragma unroll 1\nfor (int s0 = 0; s0 < KS;) {\n    int se, mi;\n";
         for (size_t r = 0; r < runs.size(); ++r) {
             size_t mi = 0;
             while (masks[mi] != runs[r].mask) ++mi;
             p2 << "    " << (r ? "else " : "") << (r + 1 < runs.size() ? "if (s0 < " + std::to_string(runs[r].se) + ") " : "") << "{ se = " << runs[r].se
-               << "; mi = " << mi << "; mk = 0x" << std::hex << runs[r].mask << std::dec << "u; }\n";
+               << "; mi = " << mi << "; }\n";
         }
         p2 << "    const int ge = min(s0 + SPH_GROUP, se);\n    phase2a_group<real>(s0, ge, KP2AARGS);\n";
-        if (rt_mask) {
-            p2 << "    (void)mi;\n    phase2b_group<real, KND, 0u>(s0, ge, KP2BARGS);\n";
-        } else {
-            p2 << "    switch (mi) {\n";
-            for (size_t mi = 0; mi < masks.size(); ++mi)
-                p2 << "        case " << mi << ": phase2b_group<real, KND, 0x" << std::hex << masks[mi] << std::dec << "u>(s0, ge, KP2BARGS); break;\n";
-            p2 << "        default: break;\n    }\n";
-        }
+        p2 << "    switch (mi) {\n";
+        for (size_t mi = 0; mi < masks.size(); ++mi)
+            p2 << "        case " << mi << ": phase2b_group<real, KND, 0x" << std::hex << masks[mi] << std::dec << "u>(s0, ge, KP2BARGS); break;\n";
+        p2 << "        default: break;\n    }\n";
         p2 << "    s0 = ge;\n}\n#endif\n";
     }
     out.phase2 = p2.str();
@@ -411,21 +400,18 @@ bool generate_source(const Program &p, const GenOptions &o, GenSource &out, std:
     // ------------------------------------------------------------------ constants of the model + options
     std::ostringstream c;
     c << "#define KREAL " << (f32 ? "float" : "double") << "\n";
-    if (o.fd_cold) c << "#define KIN_FD_COLD 1\n";
-    c << "#define KP2RTMASK " << (rt_mask ? 1 : 0) << "\n";
-    c << "#define KJFSMEM " << ((o.jf_smem && o.coll && !o.warp && !o.ik) ? 1 : 0) << "\n";
     c << "#define KPRIMS " << o.prims << "\n#define KBULK " << ((o.bulk && o.layout == 2 && !o.warp && !o.ik) ? 1 : 0) << "\n";
     c << "#define KWANT_T " << (o.want_T ? 1 : 0) << "\n#define KWANT_J " << (o.want_J ? 1 : 0) << "\n#define KCOLL " << (o.coll ? 1 : 0)
-      << "\n#define KTILED " << (o.layout == 2 ? 1 : 0) << "\n#define KAOS " << (o.layout == 1 ? 1 : 0) << "\n#define KWS " << (o.ws ? 1 : 0) << "\n";
+      << "\n#define KTILED " << (o.layout == 2 ? 1 : 0) << "\n#define KAOS " << (o.layout == 1 ? 1 : 0) << "\n";
     c << "#define KBS " << o.block << "\n#define KMINB " << o.min_blocks << "\n#define KWARP " << o.warp << "\n#define KIK " << o.ik << "\n#define KQB " << o.qbatch << "\n#define KSYNC_ON "
       << o.ksync << "\n#define KES32 " << o.es32 << "\n";
-    const bool sched = o.sched && !o.coll && !o.warp && !o.ik && !o.ws;
+    const bool sched = o.sched && !o.coll && !o.warp && !o.ik;
     c << "#define KSCHED " << (sched ? 1 : 0) << "\n#define KEPOCH " << (sched ? std::max(1, o.epoch) : 1) << "\n#define KPFD " << (sched ? o.pf_dist : 0) << "\n";
     // the configuration-independent outputs as a table of rows (kin_gen_skeleton.cuh: kin_const_fill_kernel): component (T: k,
     // J: -1 - k) and value, written as the literals phase 1 stores -- the outputs keep their bits, sign of zero included
     // -- and, for the store macros, which components the table holds.  Phase 1 keeps every KST_* line (kin_eval_host and
     // the tests read the generated text); the skeleton drops the listed ones at compile time.
-    const bool cfill = o.const_fill && o.layout == 0 && !o.warp && !o.ik && !o.ws && (!out.const_T.empty() || !out.const_J.empty());
+    const bool cfill = o.const_fill && o.layout == 0 && !o.warp && !o.ik && (!out.const_T.empty() || !out.const_J.empty());
     c << "#define KCFILL " << (cfill ? 1 : 0) << "\n";
     if (o.ik && h.n_fk > 1) c << "#define KIKROT 0x" << std::hex << o.ik_rot << std::dec << "u\n";
     c << "namespace kin {\n";

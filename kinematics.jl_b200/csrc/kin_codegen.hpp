@@ -30,7 +30,6 @@ struct GenOptions {
     bool want_T = false, want_J = false, coll = false;
     int with_rot = 0, rpy_jac = 0, keep_irrelevant = 0;
     bool want_grads = false, want_argmin = false, stale = false;
-    bool ws = false;            // warp-specialised skeleton (producer = phase 1, consumers = phase 2)
     int block = 128, min_blocks = 1;
     int qbatch = 0;             // > 0 (AoS): tiles per input batch (cp.async into shared memory behind a grid-wide barrier)
     int sched = 0;              // 1: FK / Jacobian only: tiles claimed from a counter, inputs prefetched into L2 one epoch at a time
@@ -40,13 +39,8 @@ struct GenOptions {
     int ik = 0;                 // 1: the batched Levenberg-Marquardt IK kernel around phase 1 (one link: T + rpy-Jacobian)
     unsigned ik_rot = 0;        //    ik with several links: bit l = link l has its rotation rows (KIKROT; unused for one link)
     int grad_mode = -1;         // >= 0: the gradient mode as a compile-time constant (only that code path is compiled in)
-    int fd_cold = 0;            // 1: the rare direct-FD fallback of the series gradient is an out-of-line call
     int ksync = 0;              // 1: CTA-wide barrier after every node of phase 1 (the warps of a CTA then fetch the
                                 //    straight-line code together: one instruction-cache fill serves all of them)
-    int rtmask = 0;             // phase 2b: 1 = one instance testing the relevance mask at run time, 0 = one instance per distinct mask,
-                                //   -1 = by the number of distinct masks (more than rtmask_min: run time)
-    int rtmask_min = 6;
-    int jf_smem = 0;            // 1: the joint frames of phase 2 live in the per-thread shared scratch, not in registers (opt-in, KIN_JIT_JF_REGS_MAX: measured slower)
     int bulk = 0;               // 1: tiled layout, FK / Jacobian only: outputs staged per warp and written with cp.async.bulk (TMA)
     int prims = 0;              // 1: the SDF table holds rows other than boxes (sphere / cylinder): the row loops test the kind
     int es32 = 0;               // 1: SoA component stride held in 32 bits (ld < 2^32): one IMAD.WIDE per store address

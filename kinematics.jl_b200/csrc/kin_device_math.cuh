@@ -201,13 +201,6 @@ __device__ __forceinline__ void box_gradient_fd_direct(const BoxRow<real> &b, re
     for (int i = 0; i < 3; ++i) g[i] = (key_to_dist(k[i]) - dmin) * ieps;
 }
 
-// out-of-line copy for the rare fallback of the series form (keeps the hot code small: the instruction cache is a
-// limiter of the fused kernels)
-template <typename real>
-__device__ __noinline__ void box_gradient_fd_direct_cold(const BoxRow<real> &b, real px, real py, real pz, real dmin, real g[3]) {
-    box_gradient_fd_direct(b, px, py, pz, dmin, g);
-}
-
 // The same forward-difference QUOTIENT from the closed form of the box distance (FP64 only).
 // With l = inv_pose * p, q_k = |l_k| - h_k, sigma_k = sign(l_k) and away from every kink of the SDF (no l_k
 // changes sign, no q_k crosses zero, the arg-max of q does not change within eps):
@@ -357,11 +350,7 @@ __device__ __forceinline__ void box_gradient(const BoxRow<real> &b, int grad_mod
     if (grad_mode == 1) { box_grad_analytic(b, px, py, pz, dmin, g); return; }
     if (grad_mode == 0) {
         if (box_gradient_fd_series(b, px, py, pz, dmin, g)) return;
-#ifdef KIN_FD_COLD
-        box_gradient_fd_direct_cold(b, px, py, pz, dmin, g);     // rare (within 2 eps of a kink): kept out of line
-#else
         box_gradient_fd_direct(b, px, py, pz, dmin, g);
-#endif
         return;
     }
     box_gradient_fd_direct(b, px, py, pz, dmin, g);

@@ -3,7 +3,7 @@
 //     #include "kin_gen_config.h"      generated: KREAL, KND, KS, KREV, KSTALE, ..., KRADIUS[]
 //     #include "kin_device_math.cuh"   the shared arithmetic (same functions as the interpreting kernels)
 //     #include "kin_gen_skeleton.cuh"  this file; it includes
-//         "kin_gen_phase1.inc"         generated straight-line phase 1 (uses KQ, KST_T, KST_J, KCEN_SET, KJF_OUT)
+//         "kin_gen_phase1.inc"         generated straight-line phase 1 (uses KQ, KST_T, KST_J, KCEN_SET)
 //         "kin_gen_phase2.inc"         generated: joint frames + one phase2_run<MASK> call per run of spheres
 // One thread = one configuration, persistent CTAs, SoA or tiled layout (kin_b200.h).  No table is interpreted: the
 // only run-time tables left are the boxes (kin_model_set_boxes moves them without recompiling) and the radii.
@@ -127,16 +127,9 @@ __device__ __forceinline__ void phase2b_group(const int s0, const int ge, const 
 #if KAOS && !KWARP && !KIK
                                               , real_ *stw, const int nvalid
 #endif
-                                              , const real_ *jfs     // KJFSMEM: this thread's joint frames in the shared scratch, [6 j + i][thread]
-                                              , const unsigned rmask // KP2RTMASK: the relevance mask of this run of spheres at run time
                                               ) {
     typedef real_ real;
     constexpr int BS = KBS;
-    // One instance per distinct relevance mask (MASK: the column loop below keeps only what that mask needs) -- or (opt-in,
-    // KIN_JIT_RTMASK: for models with many distinct masks, e.g. 13 instances of an 18-column loop on a dual-arm mechanism)
-    // ONE instance that tests the mask of the run at run time: warp-uniform branches, 2.4 x less code, measured within
-    // +-8 % of the per-mask instances (kin_b200.cu: gen_options)
-    const unsigned mask_ = KP2RTMASK ? rmask : MASK;
 #if KAOS && !KWARP && !KIK
     const int lane = (int)es;
     real *stg = stw + lane;
@@ -176,17 +169,9 @@ __device__ __forceinline__ void phase2b_group(const int s0, const int ge, const 
             #pragma unroll
             for (int j = 0; j < ND; ++j) {
                 real *st = stale0 + 3 * j * BS;
-                if ((mask_ >> j) & 1u) {      // joint_jacobian!, algorithm.jl:65-81
+                if ((MASK >> j) & 1u) {       // joint_jacobian!, algorithm.jl:65-81
                     real cx, cy, cz;
-#if KJFSMEM
-                    // more than 12 columns: the frames do not fit in registers; six shared loads with immediate offsets
-                    JFrame<real> fj;
-                    fj.o[0] = jfs[(6 * j + 0) * BS]; fj.o[1] = jfs[(6 * j + 1) * BS]; fj.o[2] = jfs[(6 * j + 2) * BS];
-                    fj.a[0] = jfs[(6 * j + 3) * BS]; fj.a[1] = jfs[(6 * j + 4) * BS]; fj.a[2] = jfs[(6 * j + 5) * BS];
-                    jac_col(fj, ((KREV >> j) & 1u) != 0, px, py, pz, cx, cy, cz);
-#else
                     jac_col(jfr[j], ((KREV >> j) & 1u) != 0, px, py, pz, cx, cy, cz);
-#endif
                     if (KSTALE) { st[0] = cx; st[BS] = cy; st[2 * BS] = cz; }
                     KP2_G(j, fma_(grad[0], cx, fma_(grad[1], cy, grad[2] * cz)));   // transpose(grad) * jac
                 } else if (KSTALE) {          // column left over from an earlier sphere (collision.jl:76,90)
@@ -287,7 +272,6 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_ik_kernel(const __g
             #define KST_T(k, v) Tl[k] = (v)
             #define KST_J(k, v) Jm[k] = (v)
             #define KCEN_SET(s, i, v)
-            #define KJF_OUT(j, i, v)
             #define KSYNC()
 #include "kin_gen_phase1.inc"
         }
@@ -445,7 +429,6 @@ extern "C" __global__ void __launch_bounds__(KBS, 1) kin_gen_kernel(const __grid
 #else
     #define KCEN_SET(s, i, v)
 #endif
-    #define KJF_OUT(j, i, v)
     #define KSYNC()
     {
 #include "kin_gen_phase1.inc"
@@ -519,7 +502,7 @@ extern "C" __global__ void __launch_bounds__(KBS, 1) kin_gen_kernel(const __grid
 }
 #endif
 
-#if !KWS && !KIK && !KWARP
+#if !KIK && !KWARP
 #if KQB > 0
 __device__ __forceinline__ void kin_grid_barrier(unsigned *sync, unsigned n_cta) {
     __syncthreads();
@@ -644,8 +627,7 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
     real *cent0 = scr;
     real *stale0 = scr + 3 * KS * BS;
     real *hand = stale0 + (KSTALE ? 3 * KND : 0) * BS;
-    real *jfs = hand + 2 * SPH_GROUP * BS;                    // KJFSMEM: joint frames [6 j + i][thread]
-    smem_next = tb + tab_reals + (3 * KS + (KSTALE ? 3 * KND : 0) + 2 * SPH_GROUP + (KJFSMEM ? 6 * KND : 0)) * BS;
+    smem_next = tb + tab_reals + (3 * KS + (KSTALE ? 3 * KND : 0) + 2 * SPH_GROUP) * BS;
     {
         const real *src = reinterpret_cast<const real *>(A.boxes);
         for (int i = tid; i < n_box * BOX_REALS; i += BS) tb[i] = src[i];
@@ -824,11 +806,6 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
 #else
             #define KCEN_SET(s, i, v)
 #endif
-#if KJFSMEM
-            #define KJF_OUT(j, i, v) jfs[(6 * (j) + (i)) * BS] = (v)
-#else
-            #define KJF_OUT(j, i, v)
-#endif
             {
 #include "kin_gen_phase1.inc"
 #if KCOLL
@@ -840,14 +817,10 @@ extern "C" __global__ void __launch_bounds__(KBS, KMINB) kin_gen_kernel(const __
                 real *Gp0 = reinterpret_cast<real *>(A.grads_out) + KREC_BASE((long long)KND * KS);
                 int32_t *Ap0 = KARGMIN ? A.argmin_out + KREC_BASE(KS) : nullptr;
                 #define KP2AARGS tb, n_box, cent0, hand
-#if KJFSMEM
-                #define KJFR_DEFINED
-                JFrame<real> jfr[KND];                        // unused: the frames were parked in the scratch by KJF_OUT
-#endif
 #if KAOS
-                #define KP2BARGS tb, rad, cent0, stale0, hand, jfr, A.grad_mode, trunc, voff, Vp0, Gp0, Ap0, (size_t)lane, stw, nvalid, jfs, mk
+                #define KP2BARGS tb, rad, cent0, stale0, hand, jfr, A.grad_mode, trunc, voff, Vp0, Gp0, Ap0, (size_t)lane, stw, nvalid
 #else
-                #define KP2BARGS tb, rad, cent0, stale0, hand, jfr, A.grad_mode, trunc, voff, Vp0, Gp0, Ap0, es, jfs, mk
+                #define KP2BARGS tb, rad, cent0, stale0, hand, jfr, A.grad_mode, trunc, voff, Vp0, Gp0, Ap0, es
 #endif
 #include "kin_gen_phase2.inc"
 #endif

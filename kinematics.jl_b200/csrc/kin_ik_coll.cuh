@@ -147,7 +147,7 @@ __host__ __device__ inline size_t ikc_dyn_smem_per_thread(int nd) { return sizeo
 // the sphere block (merit term mu psi_p^2, multiplier update, rank-one update of H and g where psi_p > 0, viol) and the
 // same weight mu, after it.  Written with `if constexpr`: the instances without it are the code they were before.
 // LINKS (kin_ik_solve_links, n_links >= 2): the residual and the J'J / J'e accumulation run over the links, link by
-// link and row by row, in the order the one-warp kernel uses too.
+// link and row by row.
 template <int NDT, bool ROT, bool SELF = false, bool LINKS = false>
 __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF, LINKS> A) {
     extern __shared__ double ikc_smem[];
@@ -395,279 +395,6 @@ __global__ void __launch_bounds__(128) ik_coll_step_kernel(const IkcArgsT<SELF, 
     }
     #pragma unroll
     for (int a = 0; a < ND; ++a) A.q_try[a * ld + i] = fmin(fmax(q[a] - W.x(a), A.lo[a]), A.hi[a]);
-}
-
-// The same step with one WARP per problem (opt-in: KIN_IK_STEP=warp): lane a owns column a of the configuration and row
-// a of the normal equations (registers; rows are held to IKC_MAX_DOF entries, every loop unrolled with the run-time column
-// count as a guard).  The rank-one updates H += j j' go over the lanes with one shuffle per column, the Cholesky
-// factorisation is right-looking (column k: pivot broadcast, scale, then every lane updates its row with the shuffled
-// L[b][k]) and the two triangular solves pass x[k] along by shuffle; the backward solve needs column a of L on lane a,
-// gathered by a shuffle transposition first.  Every entry receives the same operations in the same order as in the
-// one-thread kernel (an entry (a, b) is updated with -L[a][k] L[b][k] for k = 0 .. b-1 either way), so the iterates are
-// bit-identical to it -- which is what it is kept for: an independent parallelisation of the step that the tests hold
-// against the one-thread kernels (test_batched_collision_aware_ik, test_device_resident_ik_solve_dual_arm).  It was
-// written to cut the latency of the run-time-sized instance and does not: a warp per problem leaves 12+ lanes idle and
-// touches one sector per matrix entry (the state is SoA over problems), measured 1.7 ms against 1.06 ms per launch on
-// 42 k problems of 18 columns, 9.3 against 4.6 ms on 262 k.
-// SELF: the pair block of ik_coll_step_kernel<., ., true>, with the same operations per entry in the same order.
-// LINKS: the multi-link pose block of ik_coll_step_kernel<., ., ., true>, likewise.
-template <bool ROT, bool SELF = false, bool LINKS = false>
-__global__ void __launch_bounds__(128) ik_coll_step_warp_kernel(const IkcArgsT<SELF, LINKS> A) {
-    constexpr int MAXC = IKC_MAX_DOF, ROWS = ROT ? 6 : 3;
-    constexpr unsigned FULL = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const long long i = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);      // position in the active list
-    if (i >= A.n_act) return;                                                   // (warp-uniform, like every branch below
-    const long long n = A.act ? A.act[i] : i;                                   //  that is not a lane test)
-    if (A.status[n]) return;
-    const int ND = A.nd;
-    const long long ld = A.ld;
-    const double PI = 3.14159265358979323846;
-    const double mu = A.mu, margin = A.margin;
-    const int S = A.n_sph;
-    const bool mine = lane < ND;
-    const int a = mine ? lane : 0;
-
-    // ---- residual and merit at the trial point: every lane computes them (broadcast loads), as the one-thread kernel does ----
-    double e[LINKS ? 6 * IKC_MAX_LINKS : ROWS];
-    if constexpr (LINKS) {
-        #pragma unroll
-        for (int l = 0; l < IKC_MAX_LINKS; ++l)
-            if (l < A.n_links) ikc_link_residual(A.T + 12 * l * ld + i, ld, A.targets + n * 6 * A.n_links + 6 * l, (A.rot_mask >> l) & 1u, e + 6 * l);
-    } else {
-        const double *Tn = A.T + i, *tg = A.targets + n * 6;
-        #pragma unroll
-        for (int k = 0; k < 3; ++k) e[k] = Tn[(9 + k) * ld] - tg[k];
-        if (ROT) {
-            const double r00 = Tn[0], r10 = Tn[ld], r20 = Tn[2 * ld], r01 = Tn[3 * ld], r11 = Tn[4 * ld], r21 = Tn[5 * ld],
-                         r02 = Tn[6 * ld], r12 = Tn[7 * ld], r22 = Tn[8 * ld];
-            const double yaw = atan2(r10, r00);
-            double s1, c1;
-            sincos(yaw, &s1, &c1);
-            const double pitch = atan2(-r20, sqrt(fma(r21, r21, r22 * r22)));
-            const double roll = atan2(fma(r02, s1, -(r12 * c1)), fma(r11, c1, -(r01 * s1)));
-            const double ang[3] = {roll - tg[3], pitch - tg[4], yaw - tg[5]};
-            #pragma unroll
-            for (int k = 0; k < 3; ++k) e[3 + k] = ang[k] - 2.0 * PI * floor((ang[k] + PI) / (2.0 * PI));
-        }
-    }
-    double ft = 0.0;
-    if constexpr (LINKS) {
-        #pragma unroll
-        for (int l = 0; l < IKC_MAX_LINKS; ++l)
-            if (l < A.n_links) {
-                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
-                #pragma unroll
-                for (int r = 0; r < 6; ++r)
-                    if (r < rl) ft = fma(e[6 * l + r], e[6 * l + r], ft);
-            }
-    } else {
-        #pragma unroll
-        for (int r = 0; r < ROWS; ++r) ft = fma(e[r], e[r], ft);
-    }
-    double phi_t = ft;
-    for (int s = 0; s < S; ++s) {
-        const double d = A.V[s * ld + i];
-        const double psi = d >= A.trunc ? 0.0 : fmax(0.0, margin - d + A.mult[s * ld + n] / mu);
-        phi_t = fma(mu * psi, psi, phi_t);
-    }
-    if constexpr (SELF) {
-        #pragma unroll 1
-        for (int p = 0; p < A.n_pairs; ++p) {
-            const double d = A.VP[p * ld + i];
-            const double psi = d >= A.self_trunc ? 0.0 : fmax(0.0, A.self_margin - d + A.multP[p * ld + n] / mu);
-            phi_t = fma(mu * psi, psi, phi_t);
-        }
-    }
-    const bool ok = phi_t < A.phi[n];
-    double damp = A.damp[n];
-    __syncwarp();
-    if (A.it > 0) {
-        damp *= ok ? 0.3 : 4.0;
-        damp = fmin(fmax(damp, 1e-9), 1e4);
-        if (lane == 0) A.damp[n] = damp;
-    }
-
-    double q_a, g_a, Hrow[MAXC];                // row `lane` of the lower triangle: Hrow[b], b <= lane
-    if (ok) {
-        q_a = A.q_try[a * ld + i];
-        g_a = 0.0;
-        #pragma unroll
-        for (int b = 0; b < MAXC; ++b) Hrow[b] = 0.0;
-        if constexpr (LINKS) {
-            #pragma unroll
-            for (int l = 0; l < IKC_MAX_LINKS; ++l) {
-                if (l >= A.n_links) break;
-                const int rl = ((A.rot_mask >> l) & 1u) ? 6 : 3;
-                const double *Jl = A.J + (long long)l * ROWS * ND * ld;
-                double el[6];
-                #pragma unroll
-                for (int r = 0; r < 6; ++r) el[r] = e[6 * l + r];
-                #pragma unroll 1
-                for (int r = 0; r < rl; ++r) {
-                    const double ja = mine ? Jl[(long long)(a * ROWS + r) * ld + i] : 0.0;
-                    double er = el[0];
-                    #pragma unroll
-                    for (int k = 1; k < 6; ++k)
-                        if (r == k) er = el[k];
-                    g_a = fma(ja, er, g_a);
-                    #pragma unroll
-                    for (int b = 0; b < MAXC; ++b) {
-                        const double jb = __shfl_sync(FULL, ja, b);
-                        if (b <= lane) Hrow[b] = fma(ja, jb, Hrow[b]);
-                    }
-                }
-            }
-        } else {
-            #pragma unroll
-            for (int r = 0; r < ROWS; ++r) {
-                const double ja = mine ? A.J[(long long)(a * ROWS + r) * ld + i] : 0.0;
-                g_a = fma(ja, e[r], g_a);
-                #pragma unroll
-                for (int b = 0; b < MAXC; ++b) {
-                    const double jb = __shfl_sync(FULL, ja, b);
-                    if (b <= lane) Hrow[b] = fma(ja, jb, Hrow[b]);
-                }
-            }
-        }
-        double phi_n = ft, viol = -CUDART_INF;
-        #pragma unroll 1
-        for (int s = 0; s < S; ++s) {
-            const double d = A.V[s * ld + i];
-            double lam = 0.0, psi = 0.0;
-            if (d < A.trunc) {
-                viol = fmax(viol, margin - d);
-                lam = mu * fmax(0.0, margin - d + A.mult[s * ld + n] / mu);    // first-order multiplier update
-                psi = fmax(0.0, margin - d + lam / mu);
-            }
-            __syncwarp();                                                       // every lane has read the old multiplier
-            if (lane == 0) A.mult[s * ld + n] = lam;
-            if (psi > 0.0) {
-                const double ga = mine ? A.G[(long long)(s * ND + a) * ld + i] : 0.0;
-                const double w = mu * psi;
-                g_a = fma(-w, ga, g_a);
-                const double ma = mu * ga;
-                #pragma unroll
-                for (int b = 0; b < MAXC; ++b) {
-                    const double gb = __shfl_sync(FULL, ga, b);
-                    if (b <= lane) Hrow[b] = fma(ma, gb, Hrow[b]);
-                }
-                phi_n = fma(w, psi, phi_n);
-            }
-        }
-        if constexpr (SELF) {
-            const double sm = A.self_margin;
-            #pragma unroll 1
-            for (int p = 0; p < A.n_pairs; ++p) {
-                const double d = A.VP[p * ld + i];
-                double lam = 0.0, psi = 0.0;
-                if (d < A.self_trunc) {
-                    viol = fmax(viol, sm - d);
-                    lam = mu * fmax(0.0, sm - d + A.multP[p * ld + n] / mu);
-                    psi = fmax(0.0, sm - d + lam / mu);
-                }
-                __syncwarp();                                                   // every lane has read the old multiplier
-                if (lane == 0) A.multP[p * ld + n] = lam;
-                if (psi > 0.0) {
-                    const double ga = mine ? A.GP[(long long)(p * ND + a) * ld + i] : 0.0;
-                    const double w = mu * psi;
-                    g_a = fma(-w, ga, g_a);
-                    const double ma = mu * ga;
-                    #pragma unroll
-                    for (int b = 0; b < MAXC; ++b) {
-                        const double gb = __shfl_sync(FULL, ga, b);
-                        if (b <= lane) Hrow[b] = fma(ma, gb, Hrow[b]);
-                    }
-                    phi_n = fma(w, psi, phi_n);
-                }
-            }
-        }
-        if (mine) {
-            A.q[a * ld + n] = q_a;
-            A.g[a * ld + n] = g_a;
-            #pragma unroll
-            for (int b = 0; b < MAXC; ++b)
-                if (b <= lane) A.H[(long long)(lane * (lane + 1) / 2 + b) * ld + n] = Hrow[b];
-        }
-        const bool done = ft < A.ftol && viol <= A.ctol;
-        if (lane == 0) {
-            A.phi[n] = phi_n;
-            A.fpose[n] = ft;
-            A.viol[n] = viol;
-            A.its[n] = A.it;
-            if (done) A.status[n] = 1;              // q_try == q already
-        }
-        if (done) return;
-    } else {
-        q_a = A.q[a * ld + n];
-        g_a = A.g[a * ld + n];
-        #pragma unroll
-        for (int b = 0; b < MAXC; ++b) Hrow[b] = (mine && b <= lane) ? A.H[(long long)(lane * (lane + 1) / 2 + b) * ld + n] : 0.0;
-    }
-
-    // ---- step: active set on the limits, Cholesky of H + damp (I + diag H), q_try = clamp(q - x) ----
-    const double lo_a = A.lo[a], hi_a = A.hi[a];
-    const bool fr_a = !mine || !(((q_a <= lo_a + 1e-12) && (g_a > 0.0)) || ((q_a >= hi_a - 1e-12) && (g_a < 0.0)));
-    #pragma unroll
-    for (int b = 0; b < MAXC; ++b) {
-        const bool fr_b = __shfl_sync(FULL, (int)fr_a, b) != 0;
-        if (b < lane) Hrow[b] = (fr_a && fr_b) ? Hrow[b] : 0.0;
-        else if (b == lane) Hrow[b] = fr_a ? fma(damp, 1.0 + Hrow[b], Hrow[b]) : 1.0;
-    }
-    double x_a = fr_a ? g_a : 0.0;
-    #pragma unroll
-    for (int k = 0; k < MAXC; ++k) {
-        if (k < ND) {
-            const double hk = Hrow[k];
-            const double dk = __shfl_sync(FULL, hk, k);                          // the finished sum of the diagonal entry (k, k)
-            const double p = sqrt(dk > 1e-300 ? dk : 1e-300);
-            const double lak = lane == k ? p : hk / p;                           // L[lane][k] (lanes below k: unused)
-            Hrow[k] = lak;
-            #pragma unroll
-            for (int b = k + 1; b < MAXC; ++b) {
-                const double lbk = __shfl_sync(FULL, lak, b);
-                if (b <= lane) Hrow[b] = fma(-lak, lbk, Hrow[b]);
-            }
-        }
-    }
-    double dg = 1.0;                             // L[lane][lane]
-    #pragma unroll
-    for (int b = 0; b < MAXC; ++b)
-        if (b == lane) dg = Hrow[b];
-    #pragma unroll
-    for (int k = 0; k < MAXC; ++k) {             // forward: L y = x
-        if (k < ND) {
-            if (lane == k) x_a = x_a / dg;
-            const double xk = __shfl_sync(FULL, x_a, k);
-            if (lane > k) x_a = fma(-Hrow[k], xk, x_a);
-        }
-    }
-    double col[MAXC];                            // column `lane` of L: col[k] = L[k][lane], k > lane
-    #pragma unroll
-    for (int k = 1; k < MAXC; ++k) {
-        col[k] = 0.0;
-        #pragma unroll
-        for (int j = 0; j < k; ++j) {
-            const double v = __shfl_sync(FULL, Hrow[j], k);
-            if (lane == j) col[k] = v;
-        }
-    }
-    double xs[MAXC];                             // the finished x[k], known to every lane
-    #pragma unroll
-    for (int k = MAXC - 1; k >= 0; --k) {        // backward: L' x = y
-        xs[k] = 0.0;
-        if (k < ND) {
-            if (lane == k) {
-                double sum = x_a;
-                #pragma unroll
-                for (int kk = k + 1; kk < MAXC; ++kk)
-                    if (kk < ND) sum = fma(-col[kk], xs[kk], sum);
-                x_a = sum / dg;
-            }
-            xs[k] = __shfl_sync(FULL, x_a, k);
-        }
-    }
-    if (mine) A.q_try[a * ld + i] = fmin(fmax(q_a - x_a, lo_a), hi_a);
 }
 
 // Compaction of the active list: every still-running problem of the current list (act_in, or the identity when null)

@@ -1,7 +1,7 @@
 """A dual-arm mechanism (data/dual_arm.urdf: 15 columns, 18 with the planar base, 19 spheres, 3 boxes): the fused
-call and the collision-only call, interpreting kernel against the specialised one whose joint frames live in the shared
-scratch (GenOptions::jf_smem), SoA.   python profiles/sweep_dual_arm.py [log2 n]
-SWEEP_JIT_ONLY=1 with KIN_JIT_JF_REGS_MAX / KIN_JIT_BLOCK / KIN_JIT_MINB: launch-shape variants of the specialised kernel."""
+call and the collision-only call, interpreting kernel against the specialised one, SoA.
+python profiles/sweep_dual_arm.py [log2 n]
+SWEEP_JIT_ONLY=1 with KIN_JIT_BLOCK / KIN_JIT_MINB: launch-shape variants of the specialised kernel."""
 import ctypes as C
 import os
 import sys

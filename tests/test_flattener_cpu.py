@@ -246,10 +246,10 @@ def test_codegen_and_nvrtc_compile_without_a_gpu(tmp_path):
 
 
 @pytest.mark.parametrize("with_base", [False, True])
-def test_dual_arm_program_and_specialised_kernel_compile(with_base, tmp_path):
+def test_dual_arm_program_and_default_specialised_kernel_compile(with_base, tmp_path):
     """15 / 18 configuration columns (tests/scenes_dual_arm.py): the compiled program against the oracle through the
-    numpy interpreter, and the specialised kernel of the fused call -- joint frames parked in the shared scratch
-    (KJFSMEM), CTA shrunk until the scratch fits -- compiled with NVRTC for sm_100a, every layout."""
+    numpy interpreter, and the specialised kernel of the fused call -- joint frames in registers, one phase-2b instance
+    per relevance mask, CTA shrunk until the scratch fits -- compiled with NVRTC for sm_100a, every layout."""
     import ctypes as C
     import scenes_dual_arm as DA
     import scenes_synthetic as SS
@@ -283,35 +283,24 @@ def test_dual_arm_program_and_specialised_kernel_compile(with_base, tmp_path):
     expect = {(L.SOA, L.F64): (128, 2) if not with_base else (224, 1), (L.AOS, L.F64): None,
               (L.TILED32, L.F32): (256, 2) if not with_base else (480, 1), (L.TILED32, L.F64): (256, 1) if not with_base else (224, 1)}
     for (layout, prec), shape in expect.items():
-        for variant in (("default", "jf_smem", "rtmask") if layout == L.SOA else ("default",)):
-            jf_smem = variant == "jf_smem"
-            c = L.KinCall()
-            c.precision, c.layout, c.n, c.q = prec, layout, 1 << 20, 1
-            c.n_fk_links, c.fk_links, c.T_out = len(fk), fk.ctypes.data_as(C.POINTER(C.c_int32)), 1
-            c.truncation_dist = float("inf")
-            c.vals_out, c.grads_out = 1, 1
-            out_dir = tmp_path / ("l%d_p%d_%s" % (layout, prec, variant))
-            out_dir.mkdir()
-            # opt-in variants (measured, not faster, kept as knobs): joint frames parked in the shared scratch; one instance of
-            # phase 2b that tests the relevance mask at run time instead of one instance per distinct mask (13 here)
-            knob = {"jf_smem": ("KIN_JIT_JF_REGS_MAX", "12"), "rtmask": ("KIN_JIT_RTMASK", "1")}.get(variant)
-            if knob:
-                os.environ[knob[0]] = knob[1]
-            try:
-                L.check(lib.kin_codegen_dump(C.byref(d), C.byref(c), 1, str(out_dir).encode()))
-            finally:
-                if knob:
-                    os.environ.pop(knob[0], None)
-            cfg = (out_dir / "kin_gen_config.h").read_text()
-            assert ("#define KJFSMEM %d" % jf_smem) in cfg and ("#define KP2RTMASK %d" % (variant == "rtmask")) in cfg
-            n_inst = (out_dir / "kin_gen_phase2.inc").read_text().count("phase2b_group<")
-            assert n_inst == (1 if variant == "rtmask" else 13)
-            kbs = int(re.search(r"#define KBS (\d+)", cfg).group(1))
-            minb = int(re.search(r"#define KMINB (\d+)", cfg).group(1))
-            assert kbs % 32 == 0 and 32 <= kbs <= 512
-            if shape is not None and not jf_smem:
-                assert (kbs, minb) == shape, (layout, prec, kbs, minb)
-            assert (out_dir / "kin_gen.cubin").stat().st_size > 10000
+        c = L.KinCall()
+        c.precision, c.layout, c.n, c.q = prec, layout, 1 << 20, 1
+        c.n_fk_links, c.fk_links, c.T_out = len(fk), fk.ctypes.data_as(C.POINTER(C.c_int32)), 1
+        c.truncation_dist = float("inf")
+        c.vals_out, c.grads_out = 1, 1
+        out_dir = tmp_path / ("l%d_p%d" % (layout, prec))
+        out_dir.mkdir()
+        L.check(lib.kin_codegen_dump(C.byref(d), C.byref(c), 1, str(out_dir).encode()))
+        cfg = (out_dir / "kin_gen_config.h").read_text()
+        phase2 = (out_dir / "kin_gen_phase2.inc").read_text()
+        assert "const JFrame<real> jfr[KND] = {" in phase2
+        assert phase2.count("phase2b_group<") == 13          # one instance per distinct relevance mask
+        kbs = int(re.search(r"#define KBS (\d+)", cfg).group(1))
+        minb = int(re.search(r"#define KMINB (\d+)", cfg).group(1))
+        assert kbs % 32 == 0 and 32 <= kbs <= 512
+        if shape is not None:
+            assert (kbs, minb) == shape, (layout, prec, kbs, minb)
+        assert (out_dir / "kin_gen.cubin").stat().st_size > 10000
 
 
 def test_constant_and_duplicate_rows_claimed_by_the_generator_hold_in_the_oracle(tmp_path):

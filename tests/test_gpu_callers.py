@@ -135,7 +135,7 @@ def _thin_box():
     return pose, [0.05, 0.05, 0.5]                         # the pillar of test/test_planning.jl:23-25
 
 
-def test_batched_collision_aware_ik(monkeypatch):
+def test_batched_collision_aware_ik():
     """Config 4 with the reference's HARD collision constraint (inverse_kinematics.jl:14-19: dists - 0.02 >= 0 after the
     collision-free warm start) solved on the device for the whole batch (kin_ik_solve with collision = 1).
 
@@ -177,11 +177,6 @@ def test_batched_collision_aware_ik(monkeypatch):
     assert lib.kin_launch_count() - n0 == 1 + 61 * 2 + 2
     r1, c1, dm1 = outcome(q1)
     np.testing.assert_allclose(dmin1.cpu().numpy(), dm1, rtol=1e-12, atol=1e-12)
-    # the one-warp-per-problem step kernel (opt-in; an independent parallelisation of the step) on the same problems: the same iterates, bit for bit
-    monkeypatch.setenv("KIN_IK_STEP", "warp")
-    q1w, f1w, itsw, dmin1w = K.ik_solve_device(m, link, joints, dev(tg), q_free, with_rot=True, iters=60, sscc=sscc, sdf=box, margin=margin)
-    monkeypatch.delenv("KIN_IK_STEP")
-    assert torch.equal(q1w, q1) and torch.equal(f1w, f1) and torch.equal(itsw, its) and torch.equal(dmin1w, dmin1)
     q2, f2, dmin2 = K.inverse_kinematics_batch(m, link, joints, dev(tg), dev(q0), with_rot=True, iters=40, sscc=sscc, sdf=box, margin=margin,
                                                restarts=3, return_dmin=True)
     r2, c2, dm2 = outcome(q2)
@@ -609,7 +604,7 @@ def test_device_resident_ik_solve(with_base, monkeypatch):
 
 
 @pytest.mark.parametrize("with_base", [False, True])
-def test_device_resident_ik_solve_dual_arm(with_base, monkeypatch):
+def test_device_resident_ik_solve_dual_arm(with_base):
     """kin_ik_solve on a model beyond 12 configuration columns (tests/scenes_dual_arm.py: 15, 18 with the planar base -- the
     shape of the reference's PR2 inverse-kinematics test, test_inverse_kinematics.jl:26-88): the generated one-launch
     kernel for the pose-only solve, and the collision-constrained solve whose step kernel runs its run-time-sized
@@ -655,21 +650,23 @@ def test_device_resident_ik_solve_dual_arm(with_base, monkeypatch):
     print("dual-arm constrained IK (%d columns): reached %.1f %% / clear %.1f %% / both %.1f %%"
           % (nd, 100 * reached.mean(), 100 * clear.mean(), 100 * (reached & clear).mean()))
     assert clear.mean() > 0.97 and (reached & clear).mean() > (0.90 if with_base else 0.60)
-    # the step kernel above 12 columns is the run-time-sized one-thread-per-problem instance (normal equations in shared
-    # memory); the one-warp-per-problem kernel, an independent parallelisation of the same step, gives the same iterates
-    monkeypatch.setenv("KIN_IK_STEP", "warp")
-    q4, f4, dmin4 = K.inverse_kinematics_batch(m, link, joints, dev(tg), dev(q0), with_rot=True, iters=40, sscc=sscc, sdf=sdf, margin=0.02,
-                                               restarts=2, return_dmin=True)
-    monkeypatch.delenv("KIN_IK_STEP")
-    assert torch.equal(q4, q3) and torch.equal(f4, f3) and torch.equal(dmin4, dmin)
-    # position-only targets (3 rows of residual) through both step kernels
-    outs = []
-    for mode in ("warp", "thread"):
-        monkeypatch.setenv("KIN_IK_STEP", mode)
-        outs.append(K.ik_solve_device(m, link, joints, dev(tg[:512]), dev(q0[:512]), with_rot=False, iters=30, sscc=sscc, sdf=sdf, margin=0.02))
-        monkeypatch.delenv("KIN_IK_STEP")
-    for x, y in zip(*outs):
-        assert torch.equal(x, y)
+    # position-only targets (3 rows of residual), one solve
+    q4, f4, its4, dmin4 = K.ik_solve_device(m, link, joints, dev(tg[:512]), dev(q0[:512]), with_rot=False, iters=30, sscc=sscc, sdf=sdf,
+                                            margin=0.02)
+    assert int(its4.max()) > 1
+    reached4 = (_pose_err(m, joints, link, q4, tg[:512], with_rot=False) < 1e-3).cpu().numpy()
+    clear4 = (dmin4 >= 0.02 - 1e-3).cpu().numpy()
+    print("dual-arm constrained IK, position only (%d columns), one solve: reached %.1f %% / clear %.1f %% / both %.1f %%"
+          % (nd, 100 * reached4.mean(), 100 * clear4.mean(), 100 * (reached4 & clear4).mean()))
+    # first B200 run: 68.2 % (fixed base) and 92.6 % (planar base) reached and clear, 97.1 % / 99.6 % clear
+    assert clear4.mean() > 0.94 and (reached4 & clear4).mean() > (0.87 if with_base else 0.62)
+    q4n, f4n, d4n = q4.cpu().numpy(), f4.cpu().numpy(), dmin4.cpu().numpy()
+    assert np.all(q4n >= lo - 1e-12) and np.all(q4n <= hi + 1e-12)
+    for n in range(0, 512, 37):
+        R.set_joint_angles(mo, jo, q4n[n])
+        np.testing.assert_allclose(d4n[n], R.compute_coll_dists(so, jo, sdf_o).min(), rtol=1e-10, atol=1e-12)
+        fo, _ = R.ik_objective(mo, link_o, jo, q4n[n], target_T(tg[n, :3], tg[n, 3:]), False)
+        np.testing.assert_allclose(f4n[n], fo, rtol=1e-9, atol=1e-18)
 
 
 def test_staged_ik_solve_is_bitwise_the_single_launch(monkeypatch):

@@ -2,8 +2,8 @@
 model (run-time-sized step kernel, 15 / 18 columns, the default 145-pair table) and Fetch (unrolled step kernel, 8 columns,
 the 64-pair table without the constant pair that overlaps in every configuration).  Returned distances and objectives
 are held to the oracles (tests/self_collision_ref.py for the pairs, the C oracle for spheres vs boxes and the pose
-objective); the one-warp step kernel and the solve without compaction are held to the default path bit for bit; the
-single-problem SLSQP driver is held to the same scipy SLSQP driven by the oracles."""
+objective); the solve without compaction is held to the default path bit for bit; the single-problem SLSQP driver is
+held to the same scipy SLSQP driven by the oracles."""
 import ctypes as C
 
 import numpy as np
@@ -133,18 +133,37 @@ def _same(a, b):
 
 
 @pytest.mark.parametrize("with_rot", [True, False])
-def test_warp_step_is_bitwise_the_thread_step(with_rot, monkeypatch):
-    """KIN_IK_STEP=warp against the one-thread kernels: the run-time-sized instance (dual arm, 18 columns) and an
-    unrolled one (Fetch, 8 columns); q, f, iterations and the final pair distance identical."""
-    m, joints, sscc, sdf, _, _, _, _, link, tg, q0 = _dual_arm_problems(True, 512, 41)
-    fm, fj, fs, _, _, _, fpairs, flink, ftg, fq0 = _fetch_problems(512, 43)
-    for args, kw in (((m, link, joints, tg, q0), dict(sscc=sscc)), ((fm, flink, fj, ftg, fq0), dict(sscc=fs, self_pairs=fpairs))):
-        ref = _solve(*args, with_rot=with_rot, **kw)
-        monkeypatch.setenv("KIN_IK_STEP", "warp")
-        out = _solve(*args, with_rot=with_rot, **kw)
-        monkeypatch.delenv("KIN_IK_STEP")
-        assert len(ref) == 4 and int(ref[2].max()) > 1
-        _same(ref, out)
+def test_one_solve_from_random_seeds(with_rot):
+    """One solve under the pairs alone, from random in-limit seeds, with and without the rotation rows: the
+    run-time-sized step kernel (dual arm, 18 columns, default table) and an unrolled one (Fetch, 8 columns, 64 pairs).
+    Iterates inside the limits; the reported pair distance and objective are the oracles' at the returned q."""
+    m, joints, sscc, _, mo, jo, so, _, link, tg, q0 = _dual_arm_problems(True, 512, 41)
+    fm, fj, fs, fmo, fjo, fso, fpairs, flink, ftg, fq0 = _fetch_problems(512, 43)
+    runs = (("dual arm", m, joints, sscc, mo, jo, so, link, "l_tool", tg, q0, None),
+            ("Fetch", fm, fj, fs, fmo, fjo, fso, flink, "gripper_link", ftg, fq0, fpairs))
+    for name, m, joints, sscc, mo, jo, so, link, link_name, tg, q0, pairs in runs:
+        out = _solve(m, link, joints, tg, q0, with_rot=with_rot, sscc=sscc, self_pairs=pairs)
+        assert len(out) == 4
+        q, f, its, sd = out
+        assert int(its.max()) > 1
+        err = _pose_err(m, joints, link, q, tg, with_rot).cpu().numpy()
+        clear = (sd >= MARGIN - 1e-3).cpu().numpy()
+        print("%s IK under self-collision, one solve (with_rot=%s): reached %.1f %% / clear %.1f %% / both %.1f %%"
+              % (name, with_rot, 100 * (err < 1e-3).mean(), 100 * clear.mean(), 100 * ((err < 1e-3) & clear).mean()))
+        # first B200 run: 93.2 - 97.9 % reached and clear, 99.6 - 100 % clear
+        assert clear.mean() > 0.97 and ((err < 1e-3) & clear).mean() > 0.88
+        lo, hi = _limits(joints, q0.shape[1])
+        qn, fn, sdn = q.cpu().numpy(), f.cpu().numpy(), sd.cpu().numpy()
+        assert np.all(qn >= lo - 1e-12) and np.all(qn <= hi + 1e-12)
+        pairs_o = K.self_collision_pairs(sscc, joints) if pairs is None else pairs
+        link_o = R.find_link(mo, link_name)
+        for n in range(0, len(qn), 37):
+            R.set_joint_angles(mo, jo, qn[n])
+            _, _, raw = SR.self_coll_dists_and_grads(so, jo, pairs_o)
+            np.testing.assert_allclose(sdn[n], raw.min(), rtol=1e-10, atol=1e-12)
+            fo, _ = R.ik_objective(mo, link_o, jo, qn[n], target_T(tg[n, :3], tg[n, 3:]), with_rot)
+            if err[n] < 1e-1:                                # no 2 pi wrap in play
+                np.testing.assert_allclose(fn[n], fo, rtol=1e-9, atol=1e-18)
 
 
 def test_no_compaction_is_bitwise_the_active_list(monkeypatch):

@@ -616,10 +616,10 @@ def test_specialised_kernel_fp32_and_general_models(monkeypatch):
 @pytest.mark.parametrize("with_base", [False, True])
 @pytest.mark.parametrize("layout", [L.SOA, L.AOS, L.TILED32])
 def test_specialised_kernel_on_a_dual_arm_model(layout, with_base, monkeypatch):
-    """15 / 18 configuration columns (tests/scenes_dual_arm.py: the PR2 size class of fridge_demo.jl): the joint frames
-    of phase 2 no longer fit in registers, the specialised kernel parks them in its per-thread shared scratch
-    (GenOptions::jf_smem) and shrinks the CTA until the scratch fits.  Bit-identical to the interpreting kernel, and
-    both against the oracle; FP64 and FP32."""
+    """15 / 18 configuration columns (tests/scenes_dual_arm.py: the PR2 size class of fridge_demo.jl): the per-thread
+    shared scratch no longer fits the default launch shape, the specialised kernel keeps the joint frames of phase 2 in
+    registers and shrinks the CTA until the scratch fits.  Bit-identical to the interpreting kernel, and both against
+    the oracle; FP64 and FP32."""
     import scenes_dual_arm as DA
     import scenes_synthetic as SS
     from kinematics_jl_b200.device import current_q, evaluate
@@ -650,16 +650,6 @@ def test_specialised_kernel_on_a_dual_arm_model(layout, with_base, monkeypatch):
                 outs.append(o)
             for key in ("T", "J", "vals", "grads", "argmin"):
                 assert torch.equal(outs[0][key], outs[1][key]), (key, kw, dtype)
-            if dtype == torch.float64 and kw is combos[0] and layout == L.SOA:
-                # opt-in code shape: ONE instance of phase 2b that tests the relevance mask at run time (KIN_JIT_RTMASK)
-                monkeypatch.setenv("KIN_JIT_RTMASK", "1")
-                o = evaluate(dm, Qc, ql, N, layout=layout, fk_links=ids, jac_links=tools, with_rot=True, rpy_jac=True,
-                             collision=True, want_argmin=True, launch_info=True, **kw)
-                torch.cuda.synchronize()
-                monkeypatch.delenv("KIN_JIT_RTMASK")
-                assert o["launch"]["block"] < 0
-                for key in ("T", "J", "vals", "grads", "argmin"):
-                    assert torch.equal(outs[0][key], o[key]), (key, "rtmask")
         if dtype == torch.float64:        # the last combination (analytic gradient is an extension: FD combination re-run for the oracle)
             sub = slice(0, 400)
             b = outs[1]
