@@ -99,8 +99,28 @@ typedef enum { KIN_SCRATCH_REFERENCE = 0, KIN_SCRATCH_CLEAN = 1 } KinScratchMode
  * frame in the world) and a size triple:
  *   KIN_PRIM_BOX       size = full extents (BoxSDF.width)
  *   KIN_PRIM_SPHERE    size = (radius, -, -)
- *   KIN_PRIM_CYLINDER  size = (radius, length, -), axis = local z, centred on the pose (URDF <cylinder>) */
-typedef enum { KIN_PRIM_BOX = 0, KIN_PRIM_SPHERE = 1, KIN_PRIM_CYLINDER = 2 } KinPrimKind;
+ *   KIN_PRIM_CYLINDER  size = (radius, length, -), axis = local z, centred on the pose (URDF <cylinder>)
+ *   KIN_PRIM_GRID      size ignored; a sampled signed-distance grid (KinGrid below), centred on the pose */
+typedef enum { KIN_PRIM_BOX = 0, KIN_PRIM_SPHERE = 1, KIN_PRIM_CYLINDER = 2, KIN_PRIM_GRID = 3 } KinPrimKind;
+
+/* Voxel-grid signed distance fields (EXTENSION: what a depth camera, a mesh or a mapping stack delivers).
+ * A grid has nx, ny, nz >= 2 float32 samples at spacing s > 0, x fastest: v[(k*ny + j)*nx + i] (a Julia
+ * Array{Float32}(nx, ny, nz), numpy (nz, ny, nx) in C order).  Centred on its row's pose: sample (i, j, k) sits at the
+ * local point ((i - (nx-1)/2) s, (j - (ny-1)/2) s, (k - (nz-1)/2) s).  At a world point p, per axis:
+ *   l = inv_pose * p,  u = fma(l, 1/s, (n-1)/2),  c = clamp(u, 0, n-1),  i0 = min(floor(c), n-2),  t = c - i0
+ *   f = trilinear interpolation of the 8 corners of cell i0, each widened exactly to the call's precision, in the
+ *       order  a_jk = lerp(v_0jk, v_1jk, t_x),  b_k = lerp(a_0k, a_1k, t_y),  f = lerp(b_0, b_1, t_z)
+ *       with lerp(a, b, t) = fma(t, b - a, a)
+ *   d = fma(s, |u - c|, f): outside the grid box the distance to the box is added, so d is continuous everywhere
+ *       and finite far away; inside, d = f.
+ * A grid row competes in the union's first-minimum argmin like every other kind.  Gradients: KIN_GRAD_FD /
+ * KIN_GRAD_FD_DIRECT take the generic forward difference (eps 1e-7, against the cached value); KIN_GRAD_ANALYTIC the
+ * gradient of d in the chosen cell: (1/s) df/dt on the axes where u lies in [0, n-1], (u - c) / |u - c| on the others,
+ * rotated to the world (R * g_local).  FP64 calls interpolate in double and FP32 calls in float; the samples are float32
+ * in both.  The kernels read the corners through L1 / L2 (never shared memory): a 1-2 cm grid of a room is MBs to tens
+ * of MBs and stays resident in the B200's 126 MB L2. */
+typedef struct KinGrid KinGrid;
+#define KIN_MAX_GRID_VALUES (1 << 28)   /* nx * ny * nz: 1 GB of samples */
 
 #define KIN_MAX_LINKS 512
 #define KIN_MAX_JOINTS 32          /* control joints (bitmask width), base columns excluded */
@@ -207,6 +227,21 @@ KIN_API int kin_model_set_boxes(KinModel *model, int32_t n_boxes, const double *
  * KinPrimKind).  A table with a sphere / cylinder row makes the specialised kernels carry one warp-uniform test per
  * row; box-only tables compile exactly the code they always did. */
 KIN_API int kin_model_set_primitives(KinModel *model, int32_t n, const int32_t *kinds, const double *pose, const double *size);
+/* kin_model_set_primitives with voxel-grid rows: grids[n] is non-null exactly on the KIN_PRIM_GRID rows (whose size is
+ * not read); grids == NULL is kin_model_set_primitives.  The model keeps its own reference to every grid it names, so
+ * the caller may kin_grid_destroy its handle at once.  Errors before anything changes (KIN_ERR_INVALID_ARGUMENT): a grid
+ * row without a grid, a grid on another row, a grid created on another device than the model. */
+KIN_API int kin_model_set_scene(KinModel *model, int32_t n, const int32_t *kinds, const double *pose, const double *size,
+                                const KinGrid *const *grids);
+/* Creates a grid on the CURRENT device from nx*ny*nz float32 samples (host or device memory; copied with
+ * cudaMemcpyAsync on the legacy default stream, then synchronised).  Errors: a dimension < 2, a spacing that is not
+ * positive and finite, null values (KIN_ERR_INVALID_ARGUMENT); nx*ny*nz > KIN_MAX_GRID_VALUES (KIN_ERR_LIMIT). */
+KIN_API int kin_grid_create(int32_t nx, int32_t ny, int32_t nz, double spacing, const float *values, KinGrid **out);
+/* Rewrites the samples in place (host or device memory, ordered on `stream`), e.g. a perception refresh.  Must not race
+ * with launches that read the grid, the rule of kin_model_set_boxes; nothing is recompiled. */
+KIN_API int kin_grid_set_values(KinGrid *grid, const float *values, void *stream);
+/* Releases the caller's reference; the storage goes with the last reference (the models whose table names it). */
+KIN_API int kin_grid_destroy(KinGrid *grid);
 KIN_API int kin_model_n_dof(const KinModel *model);      /* n_joints (+3) */
 KIN_API int kin_model_n_spheres(const KinModel *model);
 KIN_API int kin_model_n_boxes(const KinModel *model);
@@ -289,6 +324,10 @@ KIN_API int kin_sdf_points(int32_t n_boxes, const double *box_pose, const double
 KIN_API int kin_sdf_points_prims(int32_t n, const int32_t *kinds, const double *pose, const double *size, int32_t precision,
                                  int32_t layout, const void *pts, int64_t n_pts, int32_t grad_mode, void *vals_out,
                                  void *grads_out, int32_t *argmin_out, void *stream);
+/* ... with voxel-grid rows (grids as in kin_model_set_scene; every grid on the current device) */
+KIN_API int kin_sdf_points_scene(int32_t n, const int32_t *kinds, const double *pose, const double *size,
+                                 const KinGrid *const *grids, int32_t precision, int32_t layout, const void *pts, int64_t n_pts,
+                                 int32_t grad_mode, void *vals_out, void *grads_out, int32_t *argmin_out, void *stream);
 
 /* Pose residuals of one link against target poses -- the per-iteration evaluations of the IK and
  * planning callers:

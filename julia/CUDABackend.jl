@@ -200,6 +200,40 @@ function set_primitives!(dm::DeviceMechanism, kinds::Vector{Cint}, pose::Matrix{
         (Ptr{Cvoid}, Cint, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}), dm.handle, length(kinds), pointer(kinds), pointer(pose), pointer(size_)))
 end
 
+# Extension: a sampled signed-distance grid (include/kin_b200.h, KinGrid) on the current device.  `values` is an
+# Array{Float32}(nx, ny, nz), x fastest as the library stores it; the grid is centred on the pose of its table row.
+mutable struct GridSDF
+    handle::Ptr{Cvoid}
+    dims::NTuple{3, Int}
+    spacing::Float64
+    function GridSDF(values::Array{Float32, 3}, spacing::Real)
+        handle = Ref{Ptr{Cvoid}}(C_NULL)
+        GC.@preserve values check(ccall((:kin_grid_create, libkin), Cint, (Cint, Cint, Cint, Cdouble, Ptr{Cfloat}, Ref{Ptr{Cvoid}}),
+                                        size(values, 1), size(values, 2), size(values, 3), spacing, pointer(values), handle))
+        g = new(handle[], size(values), Float64(spacing))
+        finalizer(x -> ccall((:kin_grid_destroy, libkin), Cint, (Ptr{Cvoid},), x.handle), g)
+        return g
+    end
+end
+
+# new samples in place (a perception refresh); ordered on the legacy default stream, nothing recompiles
+function update!(g::GridSDF, values::Array{Float32, 3})
+    @assert size(values) == g.dims
+    GC.@preserve values check(ccall((:kin_grid_set_values, libkin), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Cvoid}),
+                                    g.handle, pointer(values), C_NULL))
+end
+
+# set_primitives! with grid rows: grids[i] is the GridSDF of a kind-3 row, nothing elsewhere (its size column is not
+# read).  The model keeps its own reference to every grid, so a GridSDF may be collected afterwards.
+function set_scene!(dm::DeviceMechanism, kinds::Vector{Cint}, pose::Matrix{Cdouble}, size_::Matrix{Cdouble},
+                    grids::Vector{Union{GridSDF, Nothing}})
+    @assert size(pose) == (16, length(kinds)) && size(size_) == (3, length(kinds)) && length(grids) == length(kinds)
+    handles = Ptr{Cvoid}[g === nothing ? C_NULL : g.handle for g in grids]
+    GC.@preserve kinds pose size_ handles grids check(ccall((:kin_model_set_scene, libkin), Cint,
+        (Ptr{Cvoid}, Cint, Ptr{Cint}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Ptr{Cvoid}}), dm.handle, length(kinds), pointer(kinds),
+        pointer(pose), pointer(size_), pointer(handles)))
+end
+
 function make_call(dm, Q, layout, fk_links, T, jac_links, J, with_rot, rpy_jac, keep_irrelevant, vals, grads, argmin,
                    truncation_dist, grad_mode, scratch_mode, vals_offset, qptr, dptr, stream)
     N = nbatch(Q, layout)

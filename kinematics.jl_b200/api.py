@@ -9,7 +9,7 @@ from .mechanism import (FIXED, PRISMATIC, REVOLUTE, BoxMetaData, CylinderMetaDat
                         parent_link, set_base_pose, set_joint_angle, set_joint_angles, upper_limit)
 from .load_urdf import parse_urdf
 from .algorithm import get_jacobian, get_jacobian_, get_transform
-from .sdf import BoxSDF, CylinderSDF, SphereSDF, UnionSDF
+from .sdf import BoxSDF, CylinderSDF, GridSDF, SphereSDF, UnionSDF
 from .collision import (SweptSphereCollisionChecker, add_coll_links, compute_coll_dists,
                         compute_coll_dists_and_grads, compute_coll_summary, compute_self_coll_dists,
                         compute_self_coll_dists_and_grads, compute_self_coll_summary, self_collision_pairs)

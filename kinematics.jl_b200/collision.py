@@ -58,7 +58,7 @@ def _prepare(sscc, joints, sdf):
     _check_joints(m, joints)
     dm = device_model(m)
     dm.set_spheres(sscc._parents, sscc._centers, sscc.sphere_radii)
-    dm.set_boxes(*sdf.world_primitives())
+    dm.set_boxes(*sdf.world_scene())
     return m, dm
 
 

@@ -100,8 +100,20 @@ struct HostStage {          // resources of kin_eval_host, created on first use
 
 }  // namespace
 
+// Device storage of a voxel-grid SDF (kin_grid_create): a kin::GridHeader, then the float32 samples at
+// kin::GRID_VALUES_OFFSET.  Shared by the caller's KinGrid handle and every model whose table names the grid.
+struct GridStore {
+    int device = 0;
+    int32_t n[3] = {0, 0, 0};
+    void *d = nullptr;
+    size_t values() const { return (size_t)n[0] * n[1] * n[2]; }
+    ~GridStore();
+};
+struct KinGrid { std::shared_ptr<GridStore> st; };
+
 struct KinModel {
     kin::HostModel hm;
+    std::vector<std::shared_ptr<GridStore>> grids;   // the grids the SDF table names (their rows hold the addresses)
     int device = 0, n_sm = 0, dev_smem = 0;
     std::atomic<int> ws_smem_limit[2][2][2] = {};   // opt-in shared-memory limit set on this model's device, per WS kernel
     cudaMemPool_t pool = nullptr;   // stream-ordered workspace pool that keeps its memory between calls
@@ -129,6 +141,15 @@ struct DeviceGuard {
     ~DeviceGuard() { if (switched) cudaSetDevice(prev); }
 };
 
+}  // namespace
+
+GridStore::~GridStore() {
+    DeviceGuard guard(device);
+    cudaFree(d);
+}
+
+namespace {
+
 int load_spheres(kin::HostModel &hm, int32_t n, const int32_t *link, const double *center, const double *radius) {
     if (n < 0 || n > KIN_MAX_SPHERES) return fail(KIN_ERR_LIMIT, "n_spheres exceeds KIN_MAX_SPHERES");
     if (n > 0 && (!link || !center || !radius)) return fail(KIN_ERR_INVALID_ARGUMENT, "null sphere table");
@@ -144,19 +165,28 @@ int load_spheres(kin::HostModel &hm, int32_t n, const int32_t *link, const doubl
     return KIN_OK;
 }
 
-// The SDF table: boxes (BoxSDF, sdf.jl:48-74) and, as an extension, spheres / cylinders.  kinds == null: all boxes.
-// size: box = full widths; sphere = (radius, -, -); cylinder = (radius, length, -), axis = local z (URDF convention).
-int load_prims(kin::HostModel &hm, int32_t n, const int32_t *kinds, const double *pose, const double *size) {
+// The SDF table: boxes (BoxSDF, sdf.jl:48-74) and, as an extension, spheres / cylinders / voxel grids.  kinds == null:
+// all boxes.  size: box = full widths; sphere = (radius, -, -); cylinder = (radius, length, -), axis = local z (URDF
+// convention); grid: ignored, grids[b] names the grid (grids == null: no grid rows).  device >= 0: every grid must live
+// on that device.
+int load_prims(kin::HostModel &hm, int32_t n, const int32_t *kinds, const double *pose, const double *size,
+               const KinGrid *const *grids = nullptr, int device = -1) {
     if (n < 0 || n > KIN_MAX_BOXES) return fail(KIN_ERR_LIMIT, "n_boxes exceeds KIN_MAX_BOXES");
-    if (n > 0 && (!pose || !size)) return fail(KIN_ERR_INVALID_ARGUMENT, "null box table");
+    if (n > 0 && (!pose || (!size && !grids))) return fail(KIN_ERR_INVALID_ARGUMENT, "null box table");
     for (int b = 0; b < n; ++b) {            // validate before mutating
         const int k = kinds ? kinds[b] : KIN_PRIM_BOX;
-        if (k != KIN_PRIM_BOX && k != KIN_PRIM_SPHERE && k != KIN_PRIM_CYLINDER) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown primitive kind");
-        if (k != KIN_PRIM_BOX && !(size[3 * b] >= 0.0)) return fail(KIN_ERR_INVALID_ARGUMENT, "negative radius");
+        const KinGrid *g = grids ? grids[b] : nullptr;
+        if (k != KIN_PRIM_BOX && k != KIN_PRIM_SPHERE && k != KIN_PRIM_CYLINDER && k != KIN_PRIM_GRID)
+            return fail(KIN_ERR_INVALID_ARGUMENT, "unknown primitive kind");
+        if (k == KIN_PRIM_GRID && !g) return fail(KIN_ERR_INVALID_ARGUMENT, "a KIN_PRIM_GRID row without a grid");
+        if (k != KIN_PRIM_GRID && g) return fail(KIN_ERR_INVALID_ARGUMENT, "a grid on a row that is not KIN_PRIM_GRID");
+        if (k != KIN_PRIM_GRID && !size) return fail(KIN_ERR_INVALID_ARGUMENT, "null size table");
+        if (k != KIN_PRIM_BOX && k != KIN_PRIM_GRID && !(size[3 * b] >= 0.0)) return fail(KIN_ERR_INVALID_ARGUMENT, "negative radius");
+        if (g && device >= 0 && g->st->device != device) return fail(KIN_ERR_INVALID_ARGUMENT, "the grid lives on another device");
     }
     hm.n_box = n;
     hm.box_inv.resize(n); hm.box_half.assign(3 * (size_t)n, 0.0);
-    hm.box_kind.assign(n, 0); hm.box_round.assign(n, 0.0);
+    hm.box_kind.assign(n, 0); hm.box_round.assign(n, 0.0); hm.box_grid.assign(n, 0ull);
     for (int b = 0; b < n; ++b) {
         kin::Xf P = kin::Xf::from_colmajor16(pose + 16 * b), inv;
         // inv(tf) = (-R' t, R')  (transform.jl:62-65)
@@ -168,6 +198,8 @@ int load_prims(kin::HostModel &hm, int32_t n, const int32_t *kinds, const double
         const int k = kinds ? kinds[b] : KIN_PRIM_BOX;
         if (k == KIN_PRIM_SPHERE) {            // a rounded box with zero half extents
             hm.box_kind[b] = 1; hm.box_round[b] = size[3 * b];
+        } else if (k == KIN_PRIM_GRID) {
+            hm.box_kind[b] = 3; hm.box_grid[b] = (unsigned long long)(uintptr_t)grids[b]->st->d;
         } else if (k == KIN_PRIM_CYLINDER) {
             hm.box_kind[b] = 2;
             hm.box_half[3 * b] = hm.box_half[3 * b + 1] = size[3 * b];
@@ -321,6 +353,7 @@ int get_program(KinModel *m, const KinCall *c, std::shared_ptr<DeviceProgram> &o
             return fail(KIN_ERR_INVALID_ARGUMENT, err);
         const kin::Program &p = dp->prog;
         std::vector<float> r32(p.reals.begin(), p.reals.end());
+        kin::fix_grid_rows_f32(p.reals.data() + p.h.ro_box, r32.data() + p.h.ro_box, p.h.n_box);
         cudaError_t e;
         if ((e = cudaMalloc(&dp->d_int, sizeof(int32_t) * p.ints.size())) != cudaSuccess ||
             (e = cudaMalloc(&dp->d_r64, sizeof(double) * p.reals.size())) != cudaSuccess ||
@@ -882,12 +915,20 @@ int kin_model_set_boxes(KinModel *m, int32_t n, const double *pose, const double
 }
 
 int kin_model_set_primitives(KinModel *m, int32_t n, const int32_t *kinds, const double *pose, const double *width) {
+    return kin_model_set_scene(m, n, kinds, pose, width, nullptr);
+}
+
+int kin_model_set_scene(KinModel *m, int32_t n, const int32_t *kinds, const double *pose, const double *width,
+                        const KinGrid *const *grids) {
     if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
     DeviceGuard guard(m->device);
     std::lock_guard<std::mutex> lock(m->mu);
     const int old_n = m->hm.n_box;
-    int rc = load_prims(m->hm, n, kinds, pose, width);
+    int rc = load_prims(m->hm, n, kinds, pose, width, grids, m->device);
     if (rc != KIN_OK) return rc;
+    m->grids.clear();                            // the model's own references: the caller may destroy its handles
+    for (int b = 0; grids && b < n; ++b)
+        if (grids[b]) m->grids.push_back(grids[b]->st);
     if (n != old_n) { clear_cache(m); return KIN_OK; }
     // Same number of boxes (the obstacle moved, sdf.jl:14-32): the compiled programs stay valid, only the box rows
     // of their real sections are rewritten in place -- no recompilation, no cudaMalloc / cudaFree.
@@ -898,9 +939,52 @@ int kin_model_set_primitives(KinModel *m, int32_t n, const int32_t *kinds, const
         double *rows = &dp->prog.reals[h.ro_box];
         kin::emit_box_rows(m->hm, rows);
         std::vector<float> r32(rows, rows + (size_t)n * kin::BOX_REALS);
+        kin::fix_grid_rows_f32(rows, r32.data(), n);
         CUDA_TRY(cudaMemcpy(dp->d_r64 + h.ro_box, rows, sizeof(double) * r32.size(), cudaMemcpyHostToDevice));
         CUDA_TRY(cudaMemcpy(dp->d_r32 + h.ro_box, r32.data(), sizeof(float) * r32.size(), cudaMemcpyHostToDevice));
     }
+    return KIN_OK;
+}
+
+int kin_grid_create(int32_t nx, int32_t ny, int32_t nz, double spacing, const float *values, KinGrid **out) {
+    if (!out) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
+    *out = nullptr;
+    if (!values) return fail(KIN_ERR_INVALID_ARGUMENT, "null grid values");
+    if (nx < 2 || ny < 2 || nz < 2) return fail(KIN_ERR_INVALID_ARGUMENT, "a grid needs at least 2 samples per axis");
+    if ((double)nx * ny * nz > (double)KIN_MAX_GRID_VALUES) return fail(KIN_ERR_LIMIT, "grid exceeds KIN_MAX_GRID_VALUES");
+    if (!(spacing > 0.0) || std::isinf(spacing)) return fail(KIN_ERR_INVALID_ARGUMENT, "grid spacing must be positive and finite");
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
+        cudaGetLastError();
+        return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
+    }
+    auto st = std::make_shared<GridStore>();
+    CUDA_TRY(cudaGetDevice(&st->device));
+    st->n[0] = nx; st->n[1] = ny; st->n[2] = nz;
+    kin::GridHeader hd;
+    std::memset(&hd, 0, sizeof hd);
+    for (int k = 0; k < 3; ++k) hd.n[k] = st->n[k];
+    hd.s = spacing; hd.inv_s = 1.0 / spacing;
+    hd.s_f = (float)spacing; hd.inv_s_f = 1.0f / (float)spacing;
+    const size_t bytes = sizeof(float) * st->values();
+    CUDA_TRY(cudaMalloc(&st->d, kin::GRID_VALUES_OFFSET + bytes));
+    CUDA_TRY(cudaMemcpyAsync(st->d, &hd, sizeof hd, cudaMemcpyHostToDevice, 0));
+    CUDA_TRY(cudaMemcpyAsync((char *)st->d + kin::GRID_VALUES_OFFSET, values, bytes, cudaMemcpyDefault, 0));
+    CUDA_TRY(cudaStreamSynchronize(0));
+    *out = new KinGrid{st};
+    return KIN_OK;
+}
+
+int kin_grid_set_values(KinGrid *grid, const float *values, void *stream) {
+    if (!grid || !values) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
+    DeviceGuard guard(grid->st->device);
+    CUDA_TRY(cudaMemcpyAsync((char *)grid->st->d + kin::GRID_VALUES_OFFSET, values, sizeof(float) * grid->st->values(),
+                             cudaMemcpyDefault, (cudaStream_t)stream));
+    return KIN_OK;
+}
+
+int kin_grid_destroy(KinGrid *grid) {
+    delete grid;
     return KIN_OK;
 }
 
@@ -1302,6 +1386,13 @@ int kin_sdf_points(int32_t n_boxes, const double *box_pose, const double *box_wi
 int kin_sdf_points_prims(int32_t n_boxes, const int32_t *kinds, const double *box_pose, const double *box_width, int32_t precision,
                          int32_t layout, const void *pts, int64_t n, int32_t grad_mode, void *vals_out, void *grads_out,
                          int32_t *argmin_out, void *stream_) {
+    return kin_sdf_points_scene(n_boxes, kinds, box_pose, box_width, nullptr, precision, layout, pts, n, grad_mode, vals_out,
+                                grads_out, argmin_out, stream_);
+}
+
+int kin_sdf_points_scene(int32_t n_boxes, const int32_t *kinds, const double *box_pose, const double *box_width,
+                         const KinGrid *const *grids, int32_t precision, int32_t layout, const void *pts, int64_t n,
+                         int32_t grad_mode, void *vals_out, void *grads_out, int32_t *argmin_out, void *stream_) {
     if (n < 0 || (n > 0 && (!pts || !vals_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null points or vals_out");
     if (n_boxes <= 0) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_sdf_points needs at least one box");
     if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
@@ -1312,13 +1403,16 @@ int kin_sdf_points_prims(int32_t n_boxes, const int32_t *kinds, const double *bo
         cudaGetLastError();
         return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
     }
+    int cur = 0;
+    CUDA_TRY(cudaGetDevice(&cur));
     kin::HostModel hm;
-    int rc = load_prims(hm, n_boxes, kinds, box_pose, box_width);
+    int rc = load_prims(hm, n_boxes, kinds, box_pose, box_width, grids, cur);
     if (rc != KIN_OK) return rc;
     if (n == 0) return KIN_OK;
     std::vector<double> t64((size_t)n_boxes * kin::BOX_REALS, 0.0);
     kin::emit_box_rows(hm, t64.data());
     std::vector<float> t32(t64.begin(), t64.end());
+    kin::fix_grid_rows_f32(t64.data(), t32.data(), n_boxes);
     const size_t es = precision == KIN_F32 ? 4 : 8, bytes = es * t64.size();
     cudaStream_t stream = (cudaStream_t)stream_;
     void *d_tab = nullptr;

@@ -74,7 +74,8 @@ __device__ __forceinline__ void tf_mul_const(const Tf<real> &a, const real *__re
 
 // One row of the SDF table in registers: inv_R[9] row-major, inv_t[3], half extents[3], kind (slot 15: 0 = box,
 // 1 = rounded box -- a sphere is a rounded box with zero half extents --, 2 = cylinder along the local z axis with
-// h[0] = radius, h[2] = half length); slot 16 holds the rounding radius (read only on the general path).
+// h[0] = radius, h[2] = half length, 3 = voxel grid, see GridHeader); slot 16 holds the rounding radius (read only on
+// the general path).
 template <typename real> struct BoxRow { real r[9], t[3], h[3], kind; };
 __device__ __forceinline__ void load_box(const float *__restrict__ b, BoxRow<float> &o) {
     #pragma unroll
@@ -266,16 +267,83 @@ __device__ __forceinline__ bool box_gradient_fd_series(const BoxRow<double> &b, 
 }
 __device__ __forceinline__ bool box_gradient_fd_series(const BoxRow<float> &, float, float, float, float, float[3]) { return false; }
 
+// ---- voxel-grid SDF rows (kind 3, extension; include/kin_b200.h: KinGrid) ----
+// A grid row holds the inverse pose (slots 0-11) and kind 3 (slot 15); the device address of its grid storage sits as
+// raw bits in the row's last 8 bytes (FP64: slot 17, FP32: slots 16-17, low word first), written explicitly into both
+// copies of the table because a conversion of the doubles would destroy it.  The storage starts with this header; the
+// float32 samples follow at GRID_VALUES_OFFSET, x fastest.
+struct GridHeader {
+    int32_t n[3], pad;
+    double s, inv_s;            // spacing and 1 / spacing in both precisions
+    float s_f, inv_s_f, pad_f[2];
+};
+constexpr int GRID_VALUES_OFFSET = 64;
+static_assert(sizeof(GridHeader) <= GRID_VALUES_OFFSET, "grid header overlaps the values");
+
+__device__ __forceinline__ const GridHeader *grid_of(const double *rowp) {
+    return reinterpret_cast<const GridHeader *>(__double_as_longlong(rowp[17]));
+}
+__device__ __forceinline__ const GridHeader *grid_of(const float *rowp) {
+    const unsigned long long lo = __float_as_uint(rowp[16]), hi = __float_as_uint(rowp[17]);
+    return reinterpret_cast<const GridHeader *>(lo | (hi << 32));
+}
+__device__ __forceinline__ void grid_scale(const GridHeader *G, double &s, double &is) { s = __ldg(&G->s); is = __ldg(&G->inv_s); }
+__device__ __forceinline__ void grid_scale(const GridHeader *G, float &s, float &is) { s = __ldg(&G->s_f); is = __ldg(&G->inv_s_f); }
+template <typename real> __device__ __forceinline__ real lerp_(real a, real b, real t) { return fma_(t, b - a, a); }
+
+// d = f(c) + s |u - c| at the local point l (include/kin_b200.h states the formula and the interpolation order).  With
+// GRAD, gl receives its gradient in the grid frame: (1/s) df/dc on the axes where u lies in [0, n-1], (u - c) / |u - c|
+// on the others.  The 8 corners are read through the read-only cache (__ldg): a scene-sized grid lives in L2.
+template <typename real, bool GRAD>
+__device__ __forceinline__ real grid_eval(const GridHeader *G, real lx, real ly, real lz, real gl[3]) {
+    real s, is;
+    grid_scale(G, s, is);
+    const real l[3] = {lx, ly, lz};
+    int n[3], i0[3];
+    real t[3], e[3];
+    #pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        n[k] = __ldg(&G->n[k]);
+        const real top = real(n[k] - 1);
+        const real u = fma_(l[k], is, real(0.5) * top);
+        const real c = fmin(fmax(u, real(0)), top);         // a NaN coordinate lands on 0: no read outside the grid
+        i0[k] = min((int)floor(c), n[k] - 2);
+        t[k] = c - real(i0[k]);
+        e[k] = u - c;
+    }
+    const long long nx = n[0], nxy = (long long)n[0] * n[1];
+    const float *v = reinterpret_cast<const float *>(reinterpret_cast<const char *>(G) + GRID_VALUES_OFFSET) +
+                     ((long long)i0[2] * nxy + (long long)i0[1] * nx + i0[0]);
+    const real v000 = __ldg(v), v100 = __ldg(v + 1), v010 = __ldg(v + nx), v110 = __ldg(v + nx + 1);
+    const real v001 = __ldg(v + nxy), v101 = __ldg(v + nxy + 1), v011 = __ldg(v + nxy + nx), v111 = __ldg(v + nxy + nx + 1);
+    const real a00 = lerp_(v000, v100, t[0]), a10 = lerp_(v010, v110, t[0]);
+    const real a01 = lerp_(v001, v101, t[0]), a11 = lerp_(v011, v111, t[0]);
+    const real b0 = lerp_(a00, a10, t[1]), b1 = lerp_(a01, a11, t[1]);
+    const real f = lerp_(b0, b1, t[2]);
+    const real o = sqrt_(fma_(e[0], e[0], fma_(e[1], e[1], e[2] * e[2])));
+    if (GRAD) {
+        real df[3];
+        df[0] = lerp_(lerp_(v100 - v000, v110 - v010, t[1]), lerp_(v101 - v001, v111 - v011, t[1]), t[2]);
+        df[1] = lerp_(a10 - a00, a11 - a01, t[2]);
+        df[2] = b1 - b0;
+        #pragma unroll
+        for (int k = 0; k < 3; ++k) gl[k] = e[k] != real(0) ? e[k] / o : df[k] * is;
+    }
+    return fma_(s, o, f);
+}
+
 // ---- primitives other than boxes (extension; KPRIMS) ----
 // Signed distance of one general row at p.  Out of line and rare by construction (a scene of boxes never gets here):
 // it reads the row through the pointer so that the call carries four arguments.
 //   kind 1  rounded box:  d = |max(q, 0)| + min(max q, 0) - rho,  q = |inv_pose p| - h   (sphere: h = 0, rho = radius)
 //   kind 2  cylinder:     the same formula on q = (hypot(l_x, l_y) - radius, |l_z| - half length)
+//   kind 3  voxel grid:   grid_eval above
 template <typename real>
 __device__ __noinline__ real prim_dist_general(const real *rowp, real px, real py, real pz) {
     const real lx = fma_(rowp[0], px, fma_(rowp[1], py, fma_(rowp[2], pz, rowp[9])));
     const real ly = fma_(rowp[3], px, fma_(rowp[4], py, fma_(rowp[5], pz, rowp[10])));
     const real lz = fma_(rowp[6], px, fma_(rowp[7], py, fma_(rowp[8], pz, rowp[11])));
+    if (rowp[15] == real(3)) return grid_eval<real, false>(grid_of(rowp), lx, ly, lz, nullptr);
     if (rowp[15] == real(2)) {
         const real q0 = sqrt_(fma_(lx, lx, ly * ly)) - rowp[12], q1 = abs_(lz) - rowp[14];
         const real m0 = relu_(q0), m1 = relu_(q1), mx = q0 > q1 ? q0 : q1;
@@ -307,7 +375,9 @@ __device__ __noinline__ void prim_gradient_general(const real *rowp, int grad_mo
     l[0] = fma_(rowp[0], px, fma_(rowp[1], py, fma_(rowp[2], pz, rowp[9])));
     l[1] = fma_(rowp[3], px, fma_(rowp[4], py, fma_(rowp[5], pz, rowp[10])));
     l[2] = fma_(rowp[6], px, fma_(rowp[7], py, fma_(rowp[8], pz, rowp[11])));
-    if (rowp[15] == real(2)) {
+    if (rowp[15] == real(3)) {
+        grid_eval<real, true>(grid_of(rowp), l[0], l[1], l[2], gl);
+    } else if (rowp[15] == real(2)) {
         const real rxy = sqrt_(fma_(l[0], l[0], l[1] * l[1]));
         const real q0 = rxy - rowp[12], q1 = abs_(l[2]) - rowp[14];
         const real m0 = relu_(q0), m1 = relu_(q1), nrm = sqrt_(fma_(m0, m0, m1 * m1));

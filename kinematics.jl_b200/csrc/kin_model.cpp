@@ -118,7 +118,14 @@ void emit_box_rows(const HostModel &m, double *dst) {
         std::memcpy(br + 12, &m.box_half[3 * b], sizeof(double) * 3);
         br[15] = (size_t)b < m.box_kind.size() ? (double)m.box_kind[b] : 0.0;
         br[16] = (size_t)b < m.box_round.size() ? m.box_round[b] : 0.0;
+        if (br[15] == 3.0) std::memcpy(br + 17, &m.box_grid[b], sizeof(double));     // the address as raw bits
     }
+}
+
+void fix_grid_rows_f32(const double *rows64, float *rows32, int n) {
+    for (int b = 0; b < n; ++b)
+        if (rows64[(size_t)b * BOX_REALS + 15] == 3.0)
+            std::memcpy(rows32 + (size_t)b * BOX_REALS + 16, rows64 + (size_t)b * BOX_REALS + 17, sizeof(double));
 }
 
 namespace {

@@ -33,6 +33,7 @@ struct HostModel {
     std::vector<double> box_half;   // 0.5 * width (sdf.jl:68)
     std::vector<int> box_kind;      // row kind of the device table: 0 box, 1 rounded box (sphere), 2 cylinder (extension)
     std::vector<double> box_round;  // rounding radius of a kind-1 row (the sphere's radius)
+    std::vector<unsigned long long> box_grid;   // device address of a kind-3 row's grid storage (KinGrid), else 0
     std::vector<int> topo;          // parents before children
     std::vector<unsigned> relmask;  // [L] bit c set <=> control column c moves link (rptable, mechanism.jl:117-139)
 
@@ -48,6 +49,8 @@ struct Program {
 
 // the box table of a program: n_box rows of BOX_REALS doubles (inverse pose, half extents, kind, rounding radius, pad)
 void emit_box_rows(const HostModel &m, double *dst);
+// the FP32 copy of n rows converted from the FP64 ones: puts back the grid addresses the conversion destroyed
+void fix_grid_rows_f32(const double *rows64, float *rows32, int n);
 
 // fk_links / jac_links are 0-based link indices in output order.
 bool compile_program(const HostModel &m, const std::vector<int> &fk_links, const std::vector<int> &jac_links,

@@ -105,13 +105,23 @@ class DeviceModel:
             _lib.check(_lib.lib().kin_model_set_self_pairs(self.h, len(pairs), _iptr(pairs)))
             self._pair_sig, self.n_self_pairs = sig, len(pairs)
 
-    def set_boxes(self, poses, widths, kinds=None):
+    def set_boxes(self, poses, widths, kinds=None, grids=None):
+        """The SDF table (``kin_model_set_boxes`` / ``_primitives``; with a GridSDF in ``grids``, ``kin_model_set_scene``).
+        A grid enters the signature by identity only: its samples live in the grid's own device storage, which the
+        model shares, so ``GridSDF.update`` needs no new call here."""
         poses = np.ascontiguousarray(np.asarray(poses, dtype=np.float64).reshape(-1, 4, 4).transpose(0, 2, 1)).reshape(-1, 16)
         widths = np.ascontiguousarray(widths, dtype=np.float64).reshape(-1, 3)
         kinds = np.zeros(len(poses), dtype=np.int32) if kinds is None else np.ascontiguousarray(kinds, dtype=np.int32)
+        has_grid = grids is not None and any(g is not None for g in grids)
         sig = (poses.tobytes(), widths.tobytes(), kinds.tobytes())
+        if has_grid:
+            sig += (tuple(g.serial if g is not None else 0 for g in grids),)
         if sig != self._box_sig:
-            if kinds.any():         # sphere / cylinder rows (extension)
+            if has_grid:
+                from .sdf import grid_handles
+                _lib.check(_lib.lib().kin_model_set_scene(self.h, len(poses), _iptr(kinds), _dptr(poses), _dptr(widths),
+                                                          grid_handles(grids)))
+            elif kinds.any():       # sphere / cylinder rows (extension)
                 _lib.check(_lib.lib().kin_model_set_primitives(self.h, len(poses), _iptr(kinds), _dptr(poses), _dptr(widths)))
             else:
                 _lib.check(_lib.lib().kin_model_set_boxes(self.h, len(poses), _dptr(poses), _dptr(widths)))

@@ -16,7 +16,8 @@ F64, F32 = 0, 1
 SOA, AOS, TILED32 = 0, 1, 2
 FIXED, REVOLUTE, PRISMATIC = 0, 1, 2
 GRAD_FD, GRAD_ANALYTIC, GRAD_FD_DIRECT = 0, 1, 2
-PRIM_BOX, PRIM_SPHERE, PRIM_CYLINDER = 0, 1, 2
+PRIM_BOX, PRIM_SPHERE, PRIM_CYLINDER, PRIM_GRID = 0, 1, 2, 3
+MAX_GRID_VALUES = 1 << 28
 SCRATCH_REFERENCE, SCRATCH_CLEAN = 0, 1
 POSE_IK_OBJECTIVE, POSE_CONSTRAINT = 0, 1
 
@@ -67,7 +68,8 @@ EXPORTS = ["kin_last_error", "kin_abi_version", "kin_build_id", "kin_debug_build
            "kin_query_launch", "kin_sdf_points", "kin_program_dump", "kin_pose_residual", "kin_pose_residual_multi", "kin_probe_fp64",
            "kin_jit_status", "kin_jit_stats", "kin_codegen_dump", "kin_ik_solve", "kin_host_transfer_bytes",
            "kin_model_set_self_pairs", "kin_model_n_self_pairs", "kin_self_collision", "kin_ik_solve_self",
-           "kin_ik_solve_links"]
+           "kin_ik_solve_links", "kin_grid_create", "kin_grid_set_values", "kin_grid_destroy", "kin_model_set_scene",
+           "kin_sdf_points_scene"]
 
 
 def source_files():
@@ -198,6 +200,12 @@ def lib():
         L.kin_model_set_primitives.argtypes = [C.c_void_p, C.c_int32, _ip, _dp, _dp]
         L.kin_sdf_points_prims.argtypes = [C.c_int32, _ip, _dp, _dp, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_int32,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kin_model_set_scene.argtypes = [C.c_void_p, C.c_int32, _ip, _dp, _dp, C.POINTER(C.c_void_p)]
+        L.kin_sdf_points_scene.argtypes = [C.c_int32, _ip, _dp, _dp, C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_void_p,
+                                           C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kin_grid_create.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_void_p, C.POINTER(C.c_void_p)]
+        L.kin_grid_set_values.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        L.kin_grid_destroy.argtypes = [C.c_void_p]
         for f in (L.kin_model_n_dof, L.kin_model_n_spheres, L.kin_model_n_boxes):
             f.argtypes = [C.c_void_p]
         L.kin_eval.argtypes = [C.c_void_p, C.POINTER(KinCall)]
