@@ -42,9 +42,8 @@
  *     kin_eval calls on different streams are allowed.  One model per device.
  *   - which kernel runs is the library's business and never changes a result bit: batches of >= 32768 configurations
  *     (and small batches that keep coming) run kernels generated for the model and compiled with NVRTC on first use
- *     (see kin_jit_status below); without NVRTC large FP64 SoA / tiled collision launches run the warp-specialised
- *     kernel (csrc/kin_kernels_ws.cuh), which takes ~28 MB of temporary device scratch per launch from a model-private
- *     stream-ordered pool (allocated and freed on `stream`); everything else runs the interpreting kernel.
+ *     (see kin_jit_status below); everything else, and every call when NVRTC is unavailable, runs the interpreting
+ *     kernel.
  *   - KIN_LAYOUT_TILED32 buffers hold WHOLE tiles: the kernels may write the padding slots of the last tile.
  */
 #ifndef KIN_B200_H

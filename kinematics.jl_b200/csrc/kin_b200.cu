@@ -18,7 +18,6 @@
 
 #include "../../include/kin_b200.h"
 #include "kin_kernels.cuh"
-#include "kin_kernels_ws.cuh"
 #include "kin_ik_coll.cuh"
 #include "kin_model.hpp"
 #include "kin_codegen.hpp"
@@ -115,7 +114,6 @@ struct KinModel {
     kin::HostModel hm;
     std::vector<std::shared_ptr<GridStore>> grids;   // the grids the SDF table names (their rows hold the addresses)
     int device = 0, n_sm = 0, dev_smem = 0;
-    std::atomic<int> ws_smem_limit[2][2][2] = {};   // opt-in shared-memory limit set on this model's device, per WS kernel
     cudaMemPool_t pool = nullptr;   // stream-ordered workspace pool that keeps its memory between calls
     std::mutex mu;            // guards hm and the program cache (held only while a program is looked up / compiled)
     std::mutex stage_mu;      // one host-staged call at a time per model (kin_eval_host)
@@ -256,15 +254,6 @@ const KernelFn kKernels[2][3][kNumBS][2][2] = {{KIN_BS_ROW(double, 0), KIN_BS_RO
 const KernelFn kSelfKernels[2][3][kNumBS][2] = {{KIN_BS_ROW_S(double, 0), KIN_BS_ROW_S(double, 1), KIN_BS_ROW_S(double, 2)},
                                                 {KIN_BS_ROW_S(float, 0), KIN_BS_ROW_S(float, 1), KIN_BS_ROW_S(float, 2)}};
 
-// Warp-specialised fused kernel (kin_kernels_ws.cuh): FP64, SoA / tiled, collision, <= 8 columns, a chain without
-// save slots, ring fits in shared memory, and a batch large enough to fill one 384-thread CTA per SM a few times.
-// [layout: SoA, tiled][planar base][collision-only call: the producer also does the box search]
-#define KIN_WS(lay, base) {kin::kin_eval_ws_kernel<lay, base, false>, kin::kin_eval_ws_kernel<lay, base, true>}
-const KernelFn kWsKernels[2][2][2] = {{KIN_WS(0, false), KIN_WS(0, true)}, {KIN_WS(2, false), KIN_WS(2, true)}};
-
-// collision-only variant: no link transforms / Jacobians requested, no truncation (with a finite truncation
-// distance most spheres skip the gradient stage, the consumers are idle already and the box search would make the
-// producer the bottleneck: trajectory stack of config 5 0.19 -> 0.23 ms), and its larger consumer state still fits
 // does the program's SDF table hold rows other than boxes (slot 15 of a row = kind)?
 bool prog_has_prims(const kin::Program &p) {
     for (int b = 0; b < p.h.n_box; ++b)
@@ -272,22 +261,10 @@ bool prog_has_prims(const kin::Program &p) {
     return false;
 }
 
-bool ws_pre(const KinModel *m, const KinCall *c, const DeviceProgram *dp) {
-    return !c->T_out && !c->J_out && std::isinf(c->truncation_dist) && c->truncation_dist > 0 && !std::getenv("KIN_DISABLE_WS_PRE") &&
-           kin::ws_smem_bytes(dp->prog.h, true) <= (size_t)m->dev_smem;
-}
-constexpr long long kWsMinBatch = 80 * 1024;   // measured crossover (profiles/crossover_ws.py): 64 Ki -3 %, 128 Ki +11 %
-
-bool ws_eligible(const KinModel *m, const KinCall *c, const DeviceProgram *dp) {
-    const kin::ProgHeader &h = dp->prog.h;
-    if (std::getenv("KIN_DISABLE_WS")) return false;          // tuning / test aid: force kin_eval_kernel
-    if (c->precision != KIN_F64 || (c->layout != KIN_LAYOUT_SOA && c->layout != KIN_LAYOUT_TILED32)) return false;
-    // <= 8 control joints (+ the planar base); no save slots (so_jf - so_save = 12 x save slots): a chain
-    if (!c->vals_out || h.n_sph <= 0 || h.n_joints > kin::JF_REGS || h.n_dof > kin::WS_MAX_COLS) return false;
-    if (h.so_jf != h.so_save) return false;
-    if (c->n < kWsMinBatch && !std::getenv("KIN_FORCE_WS")) return false;
-    if (prog_has_prims(dp->prog)) return false;               // the hand-tuned kernel knows boxes only
-    return kin::ws_smem_bytes(h, false) <= (size_t)m->dev_smem;
+// Persistent CTAs: as many as are resident on the device at once, but no more than there are tiles of `block`
+// configurations.
+long long persistent_grid(const KinModel *m, int occ, int block, long long n) {
+    return std::min<long long>((long long)occ * m->n_sm, (n + block - 1) / block);
 }
 
 int configure(KinModel *m, DeviceProgram *dp, int pi, int li, bool self = false) {
@@ -521,7 +498,7 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     return o;
 }
 
-bool jit_wanted(const KinModel *m, const KinCall *c, const DeviceProgram *dp, bool count = true) {
+bool jit_wanted(const KinModel *m, const KinCall *c, const DeviceProgram *dp, bool count) {
     (void)m;
     if (std::getenv("KIN_DISABLE_JIT")) return false;
     const bool small = use_warp_kernel(c, dp->prog.h);
@@ -573,14 +550,8 @@ size_t jit_smem(const kin::GenOptions &o, const kin::ProgHeader &h, const JitKer
     return rs * reals;
 }
 
-// Returns the compiled kernel for this call's option set (compiling it on first use), or null when specialisation
-// is unavailable for it (NVRTC missing, compile error, does not fit): the caller then uses the interpreting kernels.
-std::shared_ptr<JitKernel> get_jit_with(KinModel *m, DeviceProgram *dp, const kin::GenOptions &o, const char *kernel_name);
-
-std::shared_ptr<JitKernel> get_jit(KinModel *m, const KinCall *c, DeviceProgram *dp) {
-    return get_jit_with(m, dp, gen_options(m, c, dp), "kin_gen_kernel");
-}
-
+// Returns the compiled kernel for this option set (compiling it on first use), or null when specialisation is
+// unavailable for it (NVRTC missing, compile error, does not fit): the caller then uses the interpreting kernels.
 std::shared_ptr<JitKernel> get_jit_with(KinModel *m, DeviceProgram *dp, const kin::GenOptions &o, const char *kernel_name) {
     const std::string key = o.key();
     std::lock_guard<std::mutex> lock(dp->jit_mu);
@@ -639,8 +610,44 @@ std::shared_ptr<JitKernel> get_jit_with(KinModel *m, DeviceProgram *dp, const ki
     return k;
 }
 
-int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, cudaStream_t stream) {
-    const kin::GenOptions o = gen_options(m, c, dp);
+// Which kernel a kin_eval call runs and with what launch shape: launch() launches it, kin_query_launch() reports it.
+struct LaunchPlan {
+    std::shared_ptr<JitKernel> jit;     // the model-specialised kernel, or null: `kernel`, an interpreting one
+    kin::GenOptions opt;                // the option set of `jit`
+    KernelFn kernel = nullptr;
+    int block = 0, regs = 0;
+    long long grid = 0;
+    size_t smem = 0;
+};
+
+// count_small_calls: whether this call counts towards specialising a program that keeps being called with small
+// batches (jit_wanted).
+LaunchPlan plan_launch(KinModel *m, const KinCall *c, DeviceProgram *dp, bool count_small_calls) {
+    LaunchPlan p;
+    if (jit_wanted(m, c, dp, count_small_calls)) {
+        p.opt = gen_options(m, c, dp);
+        p.jit = get_jit_with(m, dp, p.opt, "kin_gen_kernel");
+        if (p.jit) {
+            const JitKernel &k = *p.jit;
+            p.block = k.block; p.regs = k.regs;
+            p.smem = jit_smem(p.opt, dp->prog.h, k);
+            p.grid = p.opt.warp ? (c->n + k.block / 32 - 1) / (k.block / 32)      // one warp per configuration, not persistent
+                                : persistent_grid(m, k.occ, k.block, c->n);
+            return p;
+        }
+    }
+    const int pi = c->precision == KIN_F32 ? 1 : 0, li = c->layout;
+    const int coll = (dp->prog.h.n_sph > 0 && c->vals_out) ? 1 : 0, jr = (coll && dp->prog.h.n_dof <= kin::JF_REGS) ? 1 : 0;
+    p.kernel = kKernels[pi][li][dp->bs_index[pi][li]][coll][jr];
+    p.block = dp->block[pi][li]; p.regs = dp->regs[pi][li];
+    p.smem = dp->smem[pi][li];
+    p.grid = persistent_grid(m, dp->occ[pi][li], p.block, c->n);
+    return p;
+}
+
+int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, const LaunchPlan &p, cudaStream_t stream) {
+    const kin::GenOptions &o = p.opt;
+    const JitKernel &k = *p.jit;
     const kin::ProgHeader &h = dp->prog.h;
     kin::GenArgs a;
     std::memset(&a, 0, sizeof a);
@@ -650,11 +657,6 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
     a.n = c->n; a.ld = c->batch_stride ? c->batch_stride : c->n;
     a.n_box = h.n_box; a.grad_mode = c->grad_mode;
     a.truncation_dist = c->truncation_dist; a.vals_offset = c->vals_offset;
-    const long long tiles = (c->n + k.block - 1) / k.block;
-    long long grid = (long long)k.occ * m->n_sm;
-    if (grid > tiles) grid = tiles;
-    if (o.warp) grid = (c->n + k.block / 32 - 1) / (k.block / 32);        // one warp per configuration, not persistent
-    if (grid < 1) return KIN_OK;
     void *args[] = {&a};
     if (k.sched) {
         // a zero-initialised tile counter per launch (stream-ordered, so concurrent launches have their own)
@@ -662,7 +664,7 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
         CUDA_TRY(cudaMallocFromPoolAsync((void **)&next, sizeof(unsigned), m->pool, stream));
         a.tile_next = next;
         cudaError_t e = cudaMemsetAsync(next, 0, sizeof(unsigned), stream);
-        if (e == cudaSuccess) e = cudaLaunchKernel((const void *)k.kern, dim3((unsigned)grid), dim3((unsigned)k.block), args, jit_smem(o, h, k), stream);
+        if (e == cudaSuccess) e = cudaLaunchKernel((const void *)k.kern, dim3((unsigned)p.grid), dim3((unsigned)k.block), args, p.smem, stream);
         cudaFreeAsync(next, stream);
         if (e != cudaSuccess) return fail_cuda(e, "launching the specialised kernel");
     } else if (k.cooperative) {
@@ -673,8 +675,8 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
         a.sync = sync;
         cudaLaunchConfig_t cfg;
         std::memset(&cfg, 0, sizeof cfg);
-        cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)k.block);
-        cfg.dynamicSmemBytes = jit_smem(o, h, k); cfg.stream = stream;
+        cfg.gridDim = dim3((unsigned)p.grid); cfg.blockDim = dim3((unsigned)k.block);
+        cfg.dynamicSmemBytes = p.smem; cfg.stream = stream;
         cudaLaunchAttribute attr;
         attr.id = cudaLaunchAttributeCooperative;
         attr.val.cooperative = 1;
@@ -683,7 +685,7 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
         cudaFreeAsync(sync, stream);
         if (e != cudaSuccess) return fail_cuda(e, "launching the specialised kernel (cooperative)");
     } else {
-        CUDA_TRY(cudaLaunchKernel((const void *)k.kern, dim3((unsigned)grid), dim3((unsigned)k.block), args, jit_smem(o, h, k), stream));
+        CUDA_TRY(cudaLaunchKernel((const void *)k.kern, dim3((unsigned)p.grid), dim3((unsigned)k.block), args, p.smem, stream));
     }
     g_launches.fetch_add(1);
     g_jit_launches.fetch_add(1);
@@ -699,11 +701,10 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, JitKernel &k, c
 }
 
 int launch(KinModel *m, const KinCall *c, DeviceProgram *dp, cudaStream_t stream) {
-    if (jit_wanted(m, c, dp)) {
-        std::shared_ptr<JitKernel> jk = get_jit(m, c, dp);
-        if (jk) return launch_jit(m, c, dp, *jk, stream);
-    }
-    const int pi = c->precision == KIN_F32 ? 1 : 0, li = c->layout;
+    const LaunchPlan p = plan_launch(m, c, dp, /*count_small_calls=*/true);
+    if (p.grid < 1) return KIN_OK;
+    if (p.jit) return launch_jit(m, c, dp, p, stream);
+    const int pi = c->precision == KIN_F32 ? 1 : 0;
     kin::KernelArgs a;
     std::memset(&a, 0, sizeof a);
     a.h = dp->prog.h;
@@ -716,37 +717,7 @@ int launch(KinModel *m, const KinCall *c, DeviceProgram *dp, cudaStream_t stream
     a.with_rot = c->with_rot ? 1 : 0; a.rpy_jac = c->rpy_jac ? 1 : 0; a.keep_irrelevant = c->keep_irrelevant ? 1 : 0;
     a.grad_mode = c->grad_mode; a.scratch_ref = c->scratch_mode == KIN_SCRATCH_REFERENCE;
     a.truncation_dist = c->truncation_dist; a.vals_offset = c->vals_offset;
-    if (ws_eligible(m, c, dp)) {
-        const int wi = li == KIN_LAYOUT_TILED32 ? 1 : 0;
-        const int bi = dp->prog.h.n_dof > dp->prog.h.n_joints ? 1 : 0, pi_ = ws_pre(m, c, dp) ? 1 : 0;
-        const KernelFn k = kWsKernels[wi][bi][pi_];
-        const size_t smem = kin::ws_smem_bytes(dp->prog.h, pi_ != 0);
-        if (m->ws_smem_limit[wi][bi][pi_].load() < (int)smem) {         // function attributes are per device
-            CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, m->dev_smem));
-            m->ws_smem_limit[wi][bi][pi_].store(m->dev_smem);
-        }
-        const long long tiles = (c->n + kin::WS_TILE - 1) / kin::WS_TILE;
-        const long long grid = tiles < m->n_sm ? tiles : m->n_sm;
-        if (grid < 1) return KIN_OK;
-        // hand-over ring: stream-ordered scratch from the model's pool (concurrent launches get their own)
-        void *ring = nullptr;
-        CUDA_TRY(cudaMallocFromPoolAsync(&ring, kin::ws_ring_bytes(dp->prog.h, (int)grid, pi_ != 0), m->pool, stream));
-        a.ws_ring = ring;
-        k<<<(unsigned)grid, kin::WS_THREADS, smem, stream>>>(a);
-        cudaError_t le = cudaGetLastError();
-        cudaFreeAsync(ring, stream);
-        if (le != cudaSuccess) return fail_cuda(le, "launching kin_eval_ws_kernel");
-        g_launches.fetch_add(1);
-        return KIN_OK;
-    }
-    const int block = dp->block[pi][li];
-    const long long tiles = (c->n + block - 1) / block;
-    long long grid = (long long)dp->occ[pi][li] * m->n_sm;
-    if (grid > tiles) grid = tiles;
-    if (grid < 1) return KIN_OK;
-    const size_t smem = dp->smem[pi][li];
-    const int coll = (dp->prog.h.n_sph > 0 && c->vals_out) ? 1 : 0, jr = (coll && dp->prog.h.n_dof <= kin::JF_REGS) ? 1 : 0;
-    kKernels[pi][li][dp->bs_index[pi][li]][coll][jr]<<<(unsigned)grid, block, smem, stream>>>(a);
+    p.kernel<<<(unsigned)p.grid, p.block, p.smem, stream>>>(a);
     CUDA_TRY(cudaGetLastError());
     g_launches.fetch_add(1);
     return KIN_OK;
@@ -1034,43 +1005,14 @@ int kin_query_launch(KinModel *m, const KinCall *c, int32_t *regs, int32_t *smem
     int rc = validate_call(m, c);
     if (rc != KIN_OK) return rc;
     DeviceGuard guard(m->device);
-    std::shared_ptr<DeviceProgram> dp_;
-    rc = get_program(m, c, dp_);
+    std::shared_ptr<DeviceProgram> dp;
+    rc = get_program(m, c, dp);
     if (rc != KIN_OK) return rc;
-    DeviceProgram *dp = dp_.get();
-    const int pi = c->precision == KIN_F32 ? 1 : 0, li = c->layout;
-    if (jit_wanted(m, c, dp, /*count=*/false)) {
-        std::shared_ptr<JitKernel> jk = get_jit(m, c, dp);
-        if (jk) {
-            const long long tiles = (c->n + jk->block - 1) / jk->block;
-            long long g = (long long)jk->occ * m->n_sm;
-            if (g > tiles) g = tiles;
-            if (gen_options(m, c, dp).warp) g = (c->n + jk->block / 32 - 1) / (jk->block / 32);
-            if (regs) *regs = jk->regs;
-            if (smem_bytes) *smem_bytes = (int32_t)jit_smem(gen_options(m, c, dp), dp->prog.h, *jk);
-            if (block) *block = -jk->block;          // negative block size: the model-specialised (NVRTC) kernel
-            if (grid) *grid = (int32_t)g;
-            return KIN_OK;
-        }
-    }
-    if (ws_eligible(m, c, dp)) {
-        cudaFuncAttributes fa;
-        const bool pre = ws_pre(m, c, dp);
-        CUDA_TRY(cudaFuncGetAttributes(&fa, kWsKernels[li == KIN_LAYOUT_TILED32 ? 1 : 0][dp->prog.h.n_dof > dp->prog.h.n_joints ? 1 : 0][pre ? 1 : 0]));
-        const long long tiles = (c->n + kin::WS_TILE - 1) / kin::WS_TILE;
-        if (regs) *regs = fa.numRegs;            // launch value; setmaxnreg moves it to 88 (producer) / 208 (consumers), 120 / 192 in the collision-only variant
-        if (smem_bytes) *smem_bytes = (int32_t)kin::ws_smem_bytes(dp->prog.h, pre);
-        if (block) *block = kin::WS_THREADS;
-        if (grid) *grid = (int32_t)(tiles < m->n_sm ? tiles : m->n_sm);
-        return KIN_OK;
-    }
-    const int b = dp->block[pi][li];
-    long long tiles = (c->n + b - 1) / b, g = (long long)dp->occ[pi][li] * m->n_sm;
-    if (g > tiles) g = tiles;
-    if (regs) *regs = dp->regs[pi][li];
-    if (smem_bytes) *smem_bytes = (int32_t)dp->smem[pi][li];
-    if (block) *block = b;
-    if (grid) *grid = (int32_t)g;
+    const LaunchPlan p = plan_launch(m, c, dp.get(), /*count_small_calls=*/false);
+    if (regs) *regs = p.regs;
+    if (smem_bytes) *smem_bytes = (int32_t)p.smem;
+    if (block) *block = p.jit ? -p.block : p.block;      // negative block size: the model-specialised (NVRTC) kernel
+    if (grid) *grid = (int32_t)p.grid;
     return KIN_OK;
 }
 
@@ -1532,9 +1474,7 @@ int self_collision_launch(KinModel *m, const DevicePairs &pairs, int32_t precisi
     a.self_pairs = pairs.d; a.n_self_pairs = pairs.n;
     a.dmin_out = dmin_out; a.amin_out = amin_out;
     const int block = dp->self_block[pi][li];
-    const long long tiles = (n + block - 1) / block;
-    long long grid = (long long)dp->self_occ[pi][li] * m->n_sm;
-    if (grid > tiles) grid = tiles;
+    const long long grid = persistent_grid(m, dp->self_occ[pi][li], block, n);
     const int jr = dp->prog.h.n_dof <= kin::JF_REGS ? 1 : 0;
     kSelfKernels[pi][li][dp->self_bs_index[pi][li]][jr]<<<(unsigned)grid, block, dp->self_smem[pi][li], stream>>>(a);
     CUDA_TRY(cudaGetLastError());

@@ -1,7 +1,7 @@
 // kin_device_math.cuh -- the per-configuration arithmetic of libkin_b200 as plain device functions: rigid
 // transforms (transform.jl), the box SDF in key form and its gradients (sdf.jl:34-41,67-74,108-119), Euler-rate
 // coefficients (algorithm.jl:56-63), Jacobian columns (algorithm.jl:65-81).  Shared by the ahead-of-time kernels
-// (kin_kernels.cuh, kin_kernels_ws.cuh) and by the model-specialised kernels that kin_codegen.cpp generates and NVRTC
+// (kin_kernels.cuh) and by the model-specialised kernels that kin_codegen.cpp generates and NVRTC
 // compiles at run time (this file is embedded in the library as text for that purpose), so it must compile under
 // NVRTC without any host header.
 #pragma once
@@ -491,7 +491,6 @@ struct GenArgs {
     void *T_out, *J_out, *vals_out, *grads_out;
     int32_t *argmin_out;
     const void *boxes;           // device: n_box rows of BOX_REALS reals (rewritten in place by kin_model_set_boxes)
-    void *ws_ring;               // warp-specialised variant: global hand-over ring
     unsigned *tile_next;         // claimed tiles (KSCHED): the tile counter, zeroed before every launch
     unsigned *sync;              // input batching (KQB > 0): two zero-initialised words of the grid-wide barrier
     long long n, ld;

@@ -51,7 +51,6 @@ struct KernelArgs {
     int with_rot, rpy_jac, keep_irrelevant;
     int grad_mode, scratch_ref;  // scratch_ref = 1: reproduce the reference's shared Jacobian scratch
     double truncation_dist, vals_offset;
-    void *ws_ring;               // kin_eval_ws_kernel only: global hand-over ring (kin_kernels_ws.cuh)
     // self-collision instances only (SELF = true); appended so that the fields above keep their offsets
     const int2 *self_pairs;      // [n_self_pairs] 0-based sphere ids (i, j), read with warp-uniform loads through L1
     void *dmin_out;              // [n] min over pairs of the untruncated distance, nullable

@@ -195,15 +195,22 @@ def test_fridge_union_points_vs_oracle():
     np.testing.assert_allclose(host(g_fd), gf_ref, rtol=0, atol=1e-7)
 
 
+def _select_kernel(monkeypatch, specialised):
+    """Run the following kin_eval calls on the model-specialised kernel (whatever the batch size) or on the
+    interpreting kernel."""
+    monkeypatch.delenv("KIN_DISABLE_JIT", raising=False)
+    monkeypatch.delenv("KIN_FORCE_JIT", raising=False)
+    monkeypatch.setenv("KIN_FORCE_JIT" if specialised else "KIN_DISABLE_JIT", "1")
+
+
 @pytest.mark.parametrize("with_base", [False, True])
 @pytest.mark.parametrize("layout", [L.SOA, L.TILED32])
 @pytest.mark.parametrize("n", [1, 300, 70001])
-def test_warp_specialised_kernel_is_bitwise_identical(layout, n, with_base, monkeypatch):
-    """Large FP64 SoA / tiled collision launches take the warp-specialised kernel (kin_kernels_ws.cuh: producer
-    warps walk the chain, consumer warps do the sphere work).  It runs the same arithmetic in the same order as
-    kin_eval_kernel, so every output must be bitwise identical -- for ragged batches, with and without
-    truncation, in both scratch modes and all gradient modes."""
-    monkeypatch.setenv("KIN_DISABLE_JIT", "1")      # these tests compare the two AHEAD-OF-TIME kernels
+def test_fused_kernels_are_bitwise_identical(layout, n, with_base, monkeypatch):
+    """The fused call (FK of 25 links + two rpy Jacobians + collision) in FP64 SoA / tiled: the interpreting kernel
+    and the model-specialised kernel run the same arithmetic in the same order, so every output must be bitwise
+    identical (up to the sign of a zero) -- for ragged batches, with and without truncation, in both scratch modes
+    and all gradient modes."""
     m, joints, sscc, sdf, mo, jo, so, sdf_o = _fridge_scene(with_base)
     q = scenes.random_configs(jo, n, with_base, seed=17, zeros_every=97)
     from kinematics_jl_b200.device import current_q, evaluate
@@ -225,29 +232,28 @@ def test_warp_specialised_kernel_is_bitwise_identical(layout, n, with_base, monk
              dict(truncation_dist=0.08, grad_mode=K.GRAD_FD_DIRECT, scratch_mode=K.SCRATCH_REFERENCE, vals_offset=0.03),
              dict(truncation_dist=0.3, grad_mode=K.GRAD_ANALYTIC, scratch_mode=K.SCRATCH_CLEAN)]
     for kw in cases:
-        monkeypatch.delenv("KIN_DISABLE_WS", raising=False)
-        monkeypatch.setenv("KIN_FORCE_WS", "1")
+        _select_kernel(monkeypatch, specialised=False)
         n0 = L.lib().kin_launch_count()
-        ws, block = run(**kw)
-        assert L.lib().kin_launch_count() == n0 + 1 and block == 384          # one warp-specialised launch
-        monkeypatch.setenv("KIN_DISABLE_WS", "1")
         classic, block = run(**kw)
-        assert block in (32, 64, 96, 128)
-        for k in ws:
-            assert torch.equal(ws[k], classic[k]), (k, kw)
+        assert L.lib().kin_launch_count() == n0 + 1 and block in (32, 64, 96, 128)
+        _select_kernel(monkeypatch, specialised=True)
+        spec, block = run(**kw)
+        assert block < 0, L.lib().kin_jit_status()
+        for k in classic:
+            assert torch.equal(spec[k], classic[k]), (k, kw)
     # and against the oracle once
     v_ref, g_ref, am_ref = R.batch_collision(so, jo, sdf_o, q[:2000], np.inf, R.GRAD_FD, R.SCRATCH_REFERENCE)
-    monkeypatch.delenv("KIN_DISABLE_WS", raising=False)
-    ws, _ = run(**cases[0])
-    np.testing.assert_allclose(host(ws["vals"])[:2000], v_ref, rtol=RTOL, atol=ATOL)
-    np.testing.assert_allclose(host(ws["grads"])[:2000], g_ref.transpose(0, 2, 1), rtol=0, atol=1e-7)
+    _select_kernel(monkeypatch, specialised=False)
+    classic, block = run(**cases[0])
+    assert block > 0
+    np.testing.assert_allclose(host(classic["vals"])[:2000], v_ref, rtol=RTOL, atol=ATOL)
+    np.testing.assert_allclose(host(classic["grads"])[:2000], g_ref.transpose(0, 2, 1), rtol=0, atol=1e-7)
 
 
-def test_warp_specialised_kernel_argument_combinations_and_streams(monkeypatch):
-    """The warp-specialised kernel with outputs switched off one by one (collision only, distances only, no
-    argmin, translation-only geometric Jacobian), bitwise against kin_eval_kernel; then two launches in flight on
-    two streams at once (each takes its own hand-over ring from the model's pool) against the serial result."""
-    monkeypatch.setenv("KIN_DISABLE_JIT", "1")      # these tests compare the two AHEAD-OF-TIME kernels
+def test_fused_kernel_argument_combinations_and_streams(monkeypatch):
+    """The fused call with outputs switched off one by one (collision only, distances only, no argmin,
+    translation-only geometric Jacobian): the model-specialised kernel bitwise against the interpreting kernel; then,
+    on the default kernel, launches in flight on two streams at once against the serial result."""
     from kinematics_jl_b200.device import current_q, evaluate
     m, joints, sscc, sdf, mo, jo, so, sdf_o = _fridge_scene(False)
     n = 40000
@@ -258,7 +264,7 @@ def test_warp_specialised_kernel_argument_combinations_and_streams(monkeypatch):
     Q, ql, N = current_q(m)
     fk = [K.find_link(m, "gripper_link").id, K.find_link(m, "head_camera_link").id]
     jac = [K.find_link(m, "elbow_flex_link").id]
-    combos = [dict(collision=True),                                                        # collision only: producer does the box search
+    combos = [dict(collision=True),                                                        # collision only
               dict(collision=True, grad_mode=K.GRAD_ANALYTIC, scratch_mode=K.SCRATCH_CLEAN, want_argmin=True),
               dict(collision=True, truncation_dist=0.05, vals_offset=0.02),                # collision only, truncated
               dict(collision=True, with_grads=False, want_argmin=True),                    # distances + argmin
@@ -271,19 +277,18 @@ def test_warp_specialised_kernel_argument_combinations_and_streams(monkeypatch):
         return out
 
     for kw in combos:
-        monkeypatch.delenv("KIN_DISABLE_WS", raising=False)
-        monkeypatch.setenv("KIN_FORCE_WS", "1")
-        ws = run(kw)
-        assert ws["launch"]["block"] == 384
-        monkeypatch.setenv("KIN_DISABLE_WS", "1")
+        _select_kernel(monkeypatch, specialised=True)
+        spec = run(kw)
+        assert spec["launch"]["block"] < 0, L.lib().kin_jit_status()
+        _select_kernel(monkeypatch, specialised=False)
         classic = run(kw)
-        assert classic["launch"]["block"] != 384
+        assert classic["launch"]["block"] > 0
         torch.cuda.synchronize()
-        for k in ws:
+        for k in spec:
             if k != "launch":
-                assert torch.equal(ws[k].contiguous(), classic[k].contiguous()), (k, kw)
+                assert torch.equal(spec[k].contiguous(), classic[k].contiguous()), (k, kw)
     # concurrent launches on two streams
-    monkeypatch.delenv("KIN_DISABLE_WS", raising=False)
+    monkeypatch.delenv("KIN_DISABLE_JIT", raising=False)
     kw = combos[-1]
     serial = run(kw)
     torch.cuda.synchronize()
@@ -300,12 +305,11 @@ def test_warp_specialised_kernel_argument_combinations_and_streams(monkeypatch):
 
 
 @pytest.mark.parametrize("with_base", [False, True])
-def test_warp_specialised_kernel_on_a_second_model_vs_oracle(with_base, monkeypatch):
+def test_fused_kernel_on_a_second_model_vs_oracle(with_base, monkeypatch):
     """A different chain (the PR2 right arm of data/ground_truth.json: fixed joints between the controlled ones, so
     attachments carry non-trivial constant transforms), 10 spheres on 3 links in an order that is NOT the chain
-    order, a union of 3 rotated boxes: warp-specialised kernel against the oracle and bitwise against
-    kin_eval_kernel."""
-    monkeypatch.setenv("KIN_DISABLE_JIT", "1")      # these tests compare the two AHEAD-OF-TIME kernels
+    order, a union of 3 rotated boxes: the interpreting kernel against the oracle and bitwise against the
+    model-specialised kernel."""
     from kinematics_jl_b200.device import current_q, evaluate
     from kinematics_jl_b200.transform import rotz
     g = json.load(open(os.path.join(DATA, "ground_truth.json")))
@@ -333,20 +337,20 @@ def test_warp_specialised_kernel_on_a_second_model_vs_oracle(with_base, monkeypa
     Q, ql, N = current_q(m)
     kw = dict(layout=L.SOA, fk_links=[l.id for l in m.links[:11]], jac_links=[K.find_link(m, "r_wrist_roll_link").id],
               with_rot=True, rpy_jac=True, collision=True, want_argmin=True, truncation_dist=0.4, launch_info=True)
-    monkeypatch.setenv("KIN_FORCE_WS", "1")
-    ws = evaluate(dm, Q, ql, N, **kw)
-    assert ws["launch"]["block"] == 384
-    monkeypatch.setenv("KIN_DISABLE_WS", "1")
+    _select_kernel(monkeypatch, specialised=True)
+    spec = evaluate(dm, Q, ql, N, **kw)
+    assert spec["launch"]["block"] < 0, L.lib().kin_jit_status()
+    _select_kernel(monkeypatch, specialised=False)
     classic = evaluate(dm, Q, ql, N, **kw)
-    assert classic["launch"]["block"] != 384
+    assert classic["launch"]["block"] > 0
     for k in ("T", "J", "vals", "grads", "argmin"):
-        assert torch.equal(ws[k].contiguous(), classic[k].contiguous()), k
+        assert torch.equal(spec[k].contiguous(), classic[k].contiguous()), k
     v_ref, g_ref, am_ref = R.batch_collision(so, jo, sdf_o, q, 0.4, R.GRAD_FD, R.SCRATCH_REFERENCE)
-    np.testing.assert_allclose(host(ws["vals"]), v_ref, rtol=RTOL, atol=ATOL)
-    assert np.array_equal(ws["argmin"].cpu().numpy(), am_ref)
-    np.testing.assert_allclose(host(ws["grads"]), g_ref.transpose(0, 2, 1), rtol=0, atol=1e-7)
+    np.testing.assert_allclose(host(classic["vals"]), v_ref, rtol=RTOL, atol=ATOL)
+    assert np.array_equal(classic["argmin"].cpu().numpy(), am_ref)
+    np.testing.assert_allclose(host(classic["grads"]), g_ref.transpose(0, 2, 1), rtol=0, atol=1e-7)
     T_ref = R.batch_fk(mo, jo, q, mo.links[:11])[:, :, :3, :]
-    np.testing.assert_allclose(host(ws["T"]), T_ref, rtol=RTOL, atol=ATOL)
+    np.testing.assert_allclose(host(classic["T"]), T_ref, rtol=RTOL, atol=ATOL)
 
 
 def test_fd_series_matches_direct_fd_near_every_kink():
