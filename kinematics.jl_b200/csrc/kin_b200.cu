@@ -14,6 +14,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/kin_b200.h"
@@ -64,6 +65,19 @@ struct JitKernel {
     ~JitKernel() { if (lib) cudaLibraryUnload(lib); }
 };
 
+using KernelFn = void (*)(const kin::KernelArgs);
+
+// What an ahead-of-time kernel instance computes: FK / Jacobian only, with collision, or the self-collision phase
+// over the model's pair table instead of phase 2 (kin_self_collision: kin_eval_kernel<..., SELF = true>).
+enum Kind { KIND_FKJ = 0, KIND_COLL = 1, KIND_SELF = 2 };
+
+// The ahead-of-time kernel a program runs for one (precision, layout, kind) and its launch shape (configure).
+struct LaunchShape {
+    KernelFn kernel = nullptr;
+    int block = 0, occ = 0, regs = 0;     // block == 0: not configured yet
+    size_t smem = 0;
+};
+
 struct DeviceProgram {
     kin::Program prog;
     std::mutex jit_mu;
@@ -73,13 +87,7 @@ struct DeviceProgram {
     double *d_r64 = nullptr;
     float *d_r32 = nullptr;
     ~DeviceProgram() { cudaFree(d_int); cudaFree(d_r64); cudaFree(d_r32); }
-    // launch configuration per (precision, layout)
-    int block[2][3] = {{0, 0, 0}, {0, 0, 0}}, occ[2][3] = {{0, 0, 0}, {0, 0, 0}}, regs[2][3] = {{0, 0, 0}, {0, 0, 0}};
-    int bs_index[2][3] = {{0, 0, 0}, {0, 0, 0}};
-    size_t smem[2][3] = {{0, 0, 0}, {0, 0, 0}};
-    // the same for the self-collision kernels (kin_self_collision), configured on first use
-    int self_block[2][3] = {{0, 0, 0}, {0, 0, 0}}, self_occ[2][3] = {{0, 0, 0}, {0, 0, 0}}, self_bs_index[2][3] = {{0, 0, 0}, {0, 0, 0}};
-    size_t self_smem[2][3] = {{0, 0, 0}, {0, 0, 0}};
+    LaunchShape shape[2][3][3];          // [precision][layout][kind], configured on first use
 };
 
 // A model's self-collision pair table on its device (kin_model_set_self_pairs): 0-based sphere ids.  Reference-counted
@@ -88,6 +96,26 @@ struct DevicePairs {
     int2 *d = nullptr;
     int n = 0;
     ~DevicePairs() { cudaFree(d); }
+};
+
+// What kin::compile_program builds a program from, and the key of a model's program cache: 0-based ids of the links
+// whose transforms and Jacobians it computes, the collision phase and whether that keeps the reference's stale scratch.
+struct ProgramRequest {
+    std::vector<int> fk, jac;
+    bool coll, stale;
+    ProgramRequest(const int32_t *fk_links, int n_fk, const int32_t *jac_links, int n_jac, bool coll_, bool stale_)
+        : coll(coll_), stale(stale_) {
+        for (int i = 0; i < n_fk; ++i) fk.push_back(fk_links[i] - 1);
+        for (int i = 0; i < n_jac; ++i) jac.push_back(jac_links[i] - 1);
+    }
+    // a kin_eval call's: the links of the outputs it asks for; only the presence of the output pointers counts
+    explicit ProgramRequest(const KinCall *c)
+        : ProgramRequest(c->fk_links, c->T_out ? c->n_fk_links : 0, c->jac_links, c->J_out ? c->n_jac_links : 0, c->vals_out != nullptr,
+                         c->vals_out && c->grads_out && c->scratch_mode == KIN_SCRATCH_REFERENCE) {}
+    bool operator<(const ProgramRequest &o) const { return std::tie(coll, stale, fk, jac) < std::tie(o.coll, o.stale, o.fk, o.jac); }
+    bool compile(const kin::HostModel &hm, kin::Program &p, std::string &err) const {
+        return kin::compile_program(hm, fk, jac, coll, stale, kin::JF_REGS, p, err);
+    }
 };
 
 struct HostStage {          // resources of kin_eval_host, created on first use
@@ -119,7 +147,7 @@ struct KinModel {
     std::mutex stage_mu;      // one host-staged call at a time per model (kin_eval_host)
     // programs are reference-counted: a launch keeps its program alive even if kin_model_set_spheres /
     // kin_model_set_boxes on another thread drops the cache entry meanwhile
-    std::map<std::vector<int>, std::shared_ptr<DeviceProgram>> cache;
+    std::map<ProgramRequest, std::shared_ptr<DeviceProgram>> cache;
     std::shared_ptr<DevicePairs> self_pairs;   // null: no pair table
     HostStage stage;
 };
@@ -236,23 +264,16 @@ int host_model_from_desc(const KinModelDesc *d, kin::HostModel &hm) {
     return rc;
 }
 
-using KernelFn = void (*)(const kin::KernelArgs);
 constexpr int kNumBS = 4;
 const int kBS[kNumBS] = {128, 96, 64, 32};
 
-// [precision][layout][block size][collision][joint frames in registers]
-#define KIN_K(real, lay, bs, coll) {kin::kin_eval_kernel<real, lay, bs, coll, 0>, kin::kin_eval_kernel<real, lay, bs, coll, kin::JF_REGS>}
-#define KIN_BS_ROW(real, aos) \
-    {{KIN_K(real, aos, 128, false), KIN_K(real, aos, 128, true)}, {KIN_K(real, aos, 96, false), KIN_K(real, aos, 96, true)}, \
-     {KIN_K(real, aos, 64, false), KIN_K(real, aos, 64, true)}, {KIN_K(real, aos, 32, false), KIN_K(real, aos, 32, true)}}
-const KernelFn kKernels[2][3][kNumBS][2][2] = {{KIN_BS_ROW(double, 0), KIN_BS_ROW(double, 1), KIN_BS_ROW(double, 2)},
+// [precision][layout][block size][kind][joint frames in registers]
+#define KIN_K(real, lay, bs, coll, self) \
+    {kin::kin_eval_kernel<real, lay, bs, coll, 0, self>, kin::kin_eval_kernel<real, lay, bs, coll, kin::JF_REGS, self>}
+#define KIN_KINDS(real, lay, bs) {KIN_K(real, lay, bs, false, false), KIN_K(real, lay, bs, true, false), KIN_K(real, lay, bs, true, true)}
+#define KIN_BS_ROW(real, lay) {KIN_KINDS(real, lay, 128), KIN_KINDS(real, lay, 96), KIN_KINDS(real, lay, 64), KIN_KINDS(real, lay, 32)}
+const KernelFn kKernels[2][3][kNumBS][3][2] = {{KIN_BS_ROW(double, 0), KIN_BS_ROW(double, 1), KIN_BS_ROW(double, 2)},
                                                {KIN_BS_ROW(float, 0), KIN_BS_ROW(float, 1), KIN_BS_ROW(float, 2)}};
-
-// self-collision instances (kin_self_collision): [precision][layout][block size][joint frames in registers]
-#define KIN_KS(real, lay, bs) {kin::kin_eval_kernel<real, lay, bs, true, 0, true>, kin::kin_eval_kernel<real, lay, bs, true, kin::JF_REGS, true>}
-#define KIN_BS_ROW_S(real, lay) {KIN_KS(real, lay, 128), KIN_KS(real, lay, 96), KIN_KS(real, lay, 64), KIN_KS(real, lay, 32)}
-const KernelFn kSelfKernels[2][3][kNumBS][2] = {{KIN_BS_ROW_S(double, 0), KIN_BS_ROW_S(double, 1), KIN_BS_ROW_S(double, 2)},
-                                                {KIN_BS_ROW_S(float, 0), KIN_BS_ROW_S(float, 1), KIN_BS_ROW_S(float, 2)}};
 
 // does the program's SDF table hold rows other than boxes (slot 15 of a row = kind)?
 bool prog_has_prims(const kin::Program &p) {
@@ -267,67 +288,46 @@ long long persistent_grid(const KinModel *m, int occ, int block, long long n) {
     return std::min<long long>((long long)occ * m->n_sm, (n + block - 1) / block);
 }
 
-int configure(KinModel *m, DeviceProgram *dp, int pi, int li, bool self = false) {
+// The CTA size of the program's ahead-of-time kernel of `kind` with the most resident threads.  Called with m->mu held.
+int configure(KinModel *m, DeviceProgram *dp, int pi, int li, int kind) {
     const kin::ProgHeader &h = dp->prog.h;
-    const int coll = h.n_sph > 0 ? 1 : 0, jr = (coll && h.n_dof <= kin::JF_REGS) ? 1 : 0;
+    const int jr = (kind != KIND_FKJ && h.n_dof <= kin::JF_REGS) ? 1 : 0;
     const size_t rs = pi ? sizeof(float) : sizeof(double);
     const size_t tab = sizeof(int32_t) * (size_t)h.n_int + rs * (size_t)h.n_real;
     int dev_smem = 0;
     CUDA_TRY(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, m->device));
     int best = -1, best_threads = 0, best_occ = 0;
     size_t best_smem = 0;
-    const char *force = std::getenv("KIN_FORCE_BS");     // tuning aid: pin the CTA size
     for (int bi = 0; bi < kNumBS; ++bi) {
         const int b = kBS[bi];
-        if (force && std::atoi(force) != b) continue;
         size_t smem = tab + rs * (size_t)h.n_slots * b;
         if (li == KIN_LAYOUT_AOS) smem += rs * (size_t)kin::AOS_STAGE_REALS * (b / 32);   // warp-private staging
         if (smem > (size_t)dev_smem) continue;
-        KernelFn k = self ? kSelfKernels[pi][li][bi][jr] : kKernels[pi][li][bi][coll][jr];
+        KernelFn k = kKernels[pi][li][bi][kind][jr];
         CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, dev_smem));
         int occ = 0;
         CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, b, smem));
         if (occ * b > best_threads) { best = bi; best_threads = occ * b; best_occ = occ; best_smem = smem; }
     }
     if (best < 0) return fail(KIN_ERR_LIMIT, "model does not fit the shared-memory scratch of one CTA");
-    if (self) {
-        dp->self_block[pi][li] = kBS[best]; dp->self_bs_index[pi][li] = best; dp->self_occ[pi][li] = best_occ;
-        dp->self_smem[pi][li] = best_smem;
-        return KIN_OK;
-    }
+    const KernelFn k = kKernels[pi][li][best][kind][jr];
     cudaFuncAttributes fa;
-    CUDA_TRY(cudaFuncGetAttributes(&fa, kKernels[pi][li][best][coll][jr]));
-    dp->block[pi][li] = kBS[best]; dp->bs_index[pi][li] = best; dp->occ[pi][li] = best_occ; dp->smem[pi][li] = best_smem;
-    dp->regs[pi][li] = fa.numRegs;
+    CUDA_TRY(cudaFuncGetAttributes(&fa, k));
+    dp->shape[pi][li][kind] = {k, kBS[best], best_occ, fa.numRegs, best_smem};
     return KIN_OK;
 }
 
-int get_program(KinModel *m, const KinCall *c, std::shared_ptr<DeviceProgram> &out) {
-    const bool want_coll = c->vals_out != nullptr;
-    const bool want_stale = want_coll && c->grads_out && c->scratch_mode == KIN_SCRATCH_REFERENCE;
-    const int n_fk = c->T_out ? c->n_fk_links : 0, n_jac = c->J_out ? c->n_jac_links : 0;
-    std::vector<int> key;
-    key.reserve(n_fk + n_jac + 4);
-    key.push_back(want_coll ? (want_stale ? 2 : 1) : 0);
-    key.push_back(n_fk);
-    for (int i = 0; i < n_fk; ++i) key.push_back(c->fk_links[i]);
-    for (int i = 0; i < n_jac; ++i) key.push_back(c->jac_links[i]);
+int eval_kind(const KinCall *c) { return c->vals_out ? KIND_COLL : KIND_FKJ; }
+
+// The call's program (compiled and uploaded on first use), with the shape of its ahead-of-time kernel of `kind`.
+int get_program(KinModel *m, const KinCall *c, int kind, std::shared_ptr<DeviceProgram> &out) {
+    const ProgramRequest r(c);
     std::lock_guard<std::mutex> lock(m->mu);
-    auto it = m->cache.find(key);
+    auto it = m->cache.find(r);
     if (it == m->cache.end()) {
-        std::vector<int> fk(n_fk), jac(n_jac);
-        for (int i = 0; i < n_fk; ++i) {
-            if (c->fk_links[i] < 1 || c->fk_links[i] > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "fk link id out of range");
-            fk[i] = c->fk_links[i] - 1;
-        }
-        for (int i = 0; i < n_jac; ++i) {
-            if (c->jac_links[i] < 1 || c->jac_links[i] > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "jacobian link id out of range");
-            jac[i] = c->jac_links[i] - 1;
-        }
         std::shared_ptr<DeviceProgram> dp = std::make_shared<DeviceProgram>();
         std::string err;
-        if (!kin::compile_program(m->hm, fk, jac, want_coll, want_stale, kin::JF_REGS, dp->prog, err))
-            return fail(KIN_ERR_INVALID_ARGUMENT, err);
+        if (!r.compile(m->hm, dp->prog, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
         const kin::Program &p = dp->prog;
         std::vector<float> r32(p.reals.begin(), p.reals.end());
         kin::fix_grid_rows_f32(p.reals.data() + p.h.ro_box, r32.data() + p.h.ro_box, p.h.n_box);
@@ -340,24 +340,44 @@ int get_program(KinModel *m, const KinCall *c, std::shared_ptr<DeviceProgram> &o
             (e = cudaMemcpy(dp->d_r32, r32.data(), sizeof(float) * r32.size(), cudaMemcpyHostToDevice)) != cudaSuccess) {
             return fail_cuda(e, "uploading the kinematic program");
         }
-        it = m->cache.emplace(key, dp).first;
+        it = m->cache.emplace(r, dp).first;
     }
     std::shared_ptr<DeviceProgram> dp = it->second;
     const int pi = c->precision == KIN_F32 ? 1 : 0, li = c->layout;
-    if (dp->block[pi][li] == 0) {
-        int rc = configure(m, dp.get(), pi, li);
+    if (dp->shape[pi][li][kind].block == 0) {
+        int rc = configure(m, dp.get(), pi, li, kind);
         if (rc != KIN_OK) return rc;
     }
     out = dp;
     return KIN_OK;
 }
 
+// Fails unless a device is present (the entry points that create device state have no CPU fallback).
+int require_device() {
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
+        cudaGetLastError();
+        return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
+    }
+    return KIN_OK;
+}
+
+constexpr unsigned kAnyLayout = 1u << KIN_LAYOUT_SOA | 1u << KIN_LAYOUT_AOS | 1u << KIN_LAYOUT_TILED32;
+constexpr unsigned kSoaAos = 1u << KIN_LAYOUT_SOA | 1u << KIN_LAYOUT_AOS;
+
+// The batch of an entry point: precision, layout (one of the mask `layouts` of 1 << KIN_LAYOUT_*), size and input.
+int check_batch(int32_t precision, int32_t layout, long long n, const void *q, unsigned layouts) {
+    if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
+    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS && layout != KIN_LAYOUT_TILED32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
+    if (!(layouts >> layout & 1u)) return fail(KIN_ERR_INVALID_ARGUMENT, "this call supports the SoA and AoS layouts only");
+    if (n < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative batch size");
+    if (n > 0 && !q) return fail(KIN_ERR_INVALID_ARGUMENT, "q is null");
+    return KIN_OK;
+}
+
 int validate_call(const KinModel *m, const KinCall *c) {
     if (!m || !c) return fail(KIN_ERR_INVALID_ARGUMENT, "null model or call");
-    if (c->precision != KIN_F64 && c->precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
-    if (c->layout != KIN_LAYOUT_SOA && c->layout != KIN_LAYOUT_AOS && c->layout != KIN_LAYOUT_TILED32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
-    if (c->n < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative batch size");
-    if (c->n > 0 && !c->q) return fail(KIN_ERR_INVALID_ARGUMENT, "q is null");
+    if (int rc = check_batch(c->precision, c->layout, c->n, c->q, kAnyLayout)) return rc;
     if (c->batch_stride != 0 && c->batch_stride < c->n) return fail(KIN_ERR_INVALID_ARGUMENT, "batch_stride < n");
     if (c->T_out && (c->n_fk_links <= 0 || !c->fk_links)) return fail(KIN_ERR_INVALID_ARGUMENT, "T_out without fk_links");
     if (c->J_out && (c->n_jac_links <= 0 || !c->jac_links)) return fail(KIN_ERR_INVALID_ARGUMENT, "J_out without jac_links");
@@ -498,6 +518,32 @@ kin::GenOptions gen_options(const KinModel *m, const KinCall *c, const DevicePro
     return o;
 }
 
+// The links a solve places (kin_ik_solve / kin_ik_solve_self: the call's one link; kin_ik_solve_links: up to
+// KIN_IK_MAX_LINKS), in the order of the targets.  rows: residual rows per link in the kin_eval Jacobian (6 when any
+// link has rotation).
+static_assert(kin::IKC_MAX_LINKS == KIN_IK_MAX_LINKS, "the step kernels hold KIN_IK_MAX_LINKS residual blocks");
+struct IkLinks {
+    int n = 1;
+    int32_t ids[KIN_IK_MAX_LINKS] = {};
+    unsigned rot_mask = 0;
+    int rows() const { return rot_mask ? 6 : 3; }
+};
+IkLinks ik_one_link(const KinIkCall *c) {
+    IkLinks lk;
+    lk.ids[0] = c->link_id;
+    lk.rot_mask = c->with_rot ? 1u : 0u;
+    return lk;
+}
+
+// The generated one-launch IK kernel (kin_gen_skeleton.cuh: kin_ik_kernel) around the links' FK + Euler-rate Jacobians
+// (FP64 SoA, 128 threads: the defaults of GenOptions).
+kin::GenOptions ik_gen_options(const IkLinks &lk) {
+    kin::GenOptions o;
+    o.want_T = o.want_J = true; o.with_rot = lk.rot_mask ? 1 : 0; o.rpy_jac = 1;
+    o.ik = 1; o.ik_rot = lk.n > 1 ? lk.rot_mask : 0u;
+    return o;
+}
+
 bool jit_wanted(const KinModel *m, const KinCall *c, const DeviceProgram *dp, bool count) {
     (void)m;
     if (std::getenv("KIN_DISABLE_JIT")) return false;
@@ -620,11 +666,21 @@ struct LaunchPlan {
     size_t smem = 0;
 };
 
+// The ahead-of-time kernel of `kind` with the shape get_program configured for it.
+LaunchPlan plan_ahead_of_time(const KinModel *m, const KinCall *c, const DeviceProgram *dp, int kind) {
+    const LaunchShape &s = dp->shape[c->precision == KIN_F32 ? 1 : 0][c->layout][kind];
+    LaunchPlan p;
+    p.kernel = s.kernel;
+    p.block = s.block; p.regs = s.regs; p.smem = s.smem;
+    p.grid = persistent_grid(m, s.occ, s.block, c->n);
+    return p;
+}
+
 // count_small_calls: whether this call counts towards specialising a program that keeps being called with small
 // batches (jit_wanted).
 LaunchPlan plan_launch(KinModel *m, const KinCall *c, DeviceProgram *dp, bool count_small_calls) {
-    LaunchPlan p;
     if (jit_wanted(m, c, dp, count_small_calls)) {
+        LaunchPlan p;
         p.opt = gen_options(m, c, dp);
         p.jit = get_jit_with(m, dp, p.opt, "kin_gen_kernel");
         if (p.jit) {
@@ -636,13 +692,7 @@ LaunchPlan plan_launch(KinModel *m, const KinCall *c, DeviceProgram *dp, bool co
             return p;
         }
     }
-    const int pi = c->precision == KIN_F32 ? 1 : 0, li = c->layout;
-    const int coll = (dp->prog.h.n_sph > 0 && c->vals_out) ? 1 : 0, jr = (coll && dp->prog.h.n_dof <= kin::JF_REGS) ? 1 : 0;
-    p.kernel = kKernels[pi][li][dp->bs_index[pi][li]][coll][jr];
-    p.block = dp->block[pi][li]; p.regs = dp->regs[pi][li];
-    p.smem = dp->smem[pi][li];
-    p.grid = persistent_grid(m, dp->occ[pi][li], p.block, c->n);
-    return p;
+    return plan_ahead_of_time(m, c, dp, eval_kind(c));
 }
 
 int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, const LaunchPlan &p, cudaStream_t stream) {
@@ -700,16 +750,13 @@ int launch_jit(KinModel *m, const KinCall *c, DeviceProgram *dp, const LaunchPla
     return KIN_OK;
 }
 
-int launch(KinModel *m, const KinCall *c, DeviceProgram *dp, cudaStream_t stream) {
-    const LaunchPlan p = plan_launch(m, c, dp, /*count_small_calls=*/true);
-    if (p.grid < 1) return KIN_OK;
-    if (p.jit) return launch_jit(m, c, dp, p, stream);
-    const int pi = c->precision == KIN_F32 ? 1 : 0;
+// The arguments of an ahead-of-time kernel for a call (the self-collision fields stay zero).
+kin::KernelArgs kernel_args(const KinCall *c, const DeviceProgram *dp) {
     kin::KernelArgs a;
     std::memset(&a, 0, sizeof a);
     a.h = dp->prog.h;
     a.tab_i = dp->d_int;
-    a.tab_r = pi ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
+    a.tab_r = c->precision == KIN_F32 ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
     a.q = c->q;
     a.T_out = c->T_out; a.J_out = c->J_out; a.vals_out = c->vals_out; a.grads_out = c->grads_out;
     a.argmin_out = c->argmin_out;
@@ -717,10 +764,21 @@ int launch(KinModel *m, const KinCall *c, DeviceProgram *dp, cudaStream_t stream
     a.with_rot = c->with_rot ? 1 : 0; a.rpy_jac = c->rpy_jac ? 1 : 0; a.keep_irrelevant = c->keep_irrelevant ? 1 : 0;
     a.grad_mode = c->grad_mode; a.scratch_ref = c->scratch_mode == KIN_SCRATCH_REFERENCE;
     a.truncation_dist = c->truncation_dist; a.vals_offset = c->vals_offset;
+    return a;
+}
+
+int launch_ahead_of_time(const LaunchPlan &p, const kin::KernelArgs &a, cudaStream_t stream) {
     p.kernel<<<(unsigned)p.grid, p.block, p.smem, stream>>>(a);
     CUDA_TRY(cudaGetLastError());
     g_launches.fetch_add(1);
     return KIN_OK;
+}
+
+int launch(KinModel *m, const KinCall *c, DeviceProgram *dp, cudaStream_t stream) {
+    const LaunchPlan p = plan_launch(m, c, dp, /*count_small_calls=*/true);
+    if (p.grid < 1) return KIN_OK;
+    if (p.jit) return launch_jit(m, c, dp, p, stream);
+    return launch_ahead_of_time(p, kernel_args(c, dp), stream);
 }
 
 }  // namespace
@@ -765,20 +823,16 @@ int kin_codegen_dump(const KinModelDesc *d, const KinCall *c, int32_t compile, c
     kin::HostModel hm;
     int rc = host_model_from_desc(d, hm);
     if (rc != KIN_OK) return rc;
-    const bool want_coll = c->vals_out != nullptr;
-    const bool want_stale = want_coll && c->grads_out && c->scratch_mode == KIN_SCRATCH_REFERENCE;
-    const int n_fk = c->T_out ? c->n_fk_links : 0, n_jac = c->J_out ? c->n_jac_links : 0;
-    std::vector<int> fk(n_fk), jac(n_jac);
-    for (int i = 0; i < n_fk; ++i) fk[i] = c->fk_links[i] - 1;
-    for (int i = 0; i < n_jac; ++i) jac[i] = c->jac_links[i] - 1;
     DeviceProgram dp;
     std::string err;
-    if (!kin::compile_program(hm, fk, jac, want_coll, want_stale, kin::JF_REGS, dp.prog, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
+    if (!ProgramRequest(c).compile(hm, dp.prog, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
     kin::GenOptions o = gen_options(nullptr, c, &dp);
-    if (const char *ik = std::getenv("KIN_DUMP_IK")) {   // development aid: the batched-IK kernel of this link instead
-        o.ik = 1; o.rpy_jac = o.with_rot; o.ksync = 0; o.coll = false; o.block = 128; o.min_blocks = 1;
+    if (const char *ik = std::getenv("KIN_DUMP_IK")) {   // development aid: the batched-IK kernel of the call's links instead
+        IkLinks lk;
+        lk.n = dp.prog.h.n_fk;
         // several links (kin_ik_solve_links): the value is the rotation mask (bit l: link l has rotation rows)
-        if (dp.prog.h.n_fk > 1) o.ik_rot = (unsigned)std::strtoul(ik, nullptr, 0);
+        lk.rot_mask = lk.n > 1 ? (unsigned)std::strtoul(ik, nullptr, 0) : (c->with_rot ? 1u : 0u);
+        o = ik_gen_options(lk);
     }
     kin::GenSource g;
     if (!kin::generate_source(dp.prog, o, g, err)) return fail(KIN_ERR_INVALID_ARGUMENT, "codegen: " + err);
@@ -803,11 +857,7 @@ int kin_codegen_dump(const KinModelDesc *d, const KinCall *c, int32_t compile, c
 int kin_model_create(const KinModelDesc *d, KinModel **out) {
     if (!d || !out) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
     *out = nullptr;
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-        cudaGetLastError();
-        return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
-    }
+    if (int rc = require_device()) return rc;
     KinModel *m = new KinModel();
     int rc = host_model_from_desc(d, m->hm);
     if (rc != KIN_OK) { delete m; return rc; }
@@ -844,12 +894,10 @@ int kin_program_dump(const KinModelDesc *d, const int32_t *fk_links, int32_t n_f
     kin::HostModel hm;
     int rc = host_model_from_desc(d, hm);
     if (rc != KIN_OK) return rc;
-    std::vector<int> fk(n_fk), jac(n_jac);
-    for (int i = 0; i < n_fk; ++i) fk[i] = fk_links[i] - 1;
-    for (int i = 0; i < n_jac; ++i) jac[i] = jac_links[i] - 1;
     kin::Program p;
     std::string err;
-    if (!kin::compile_program(hm, fk, jac, want_coll != 0, want_stale != 0, kin::JF_REGS, p, err)) return fail(KIN_ERR_INVALID_ARGUMENT, err);
+    if (!ProgramRequest(fk_links, n_fk, jac_links, n_jac, want_coll != 0, want_stale != 0).compile(hm, p, err))
+        return fail(KIN_ERR_INVALID_ARGUMENT, err);
     const int hn = (int)(sizeof(kin::ProgHeader) / sizeof(int32_t));
     if (header_cap < hn || ints_cap < (int)p.ints.size() || reals_cap < (int)p.reals.size())
         return fail(KIN_ERR_LIMIT, "kin_program_dump: output buffers too small");
@@ -924,11 +972,7 @@ int kin_grid_create(int32_t nx, int32_t ny, int32_t nz, double spacing, const fl
     if (nx < 2 || ny < 2 || nz < 2) return fail(KIN_ERR_INVALID_ARGUMENT, "a grid needs at least 2 samples per axis");
     if ((double)nx * ny * nz > (double)KIN_MAX_GRID_VALUES) return fail(KIN_ERR_LIMIT, "grid exceeds KIN_MAX_GRID_VALUES");
     if (!(spacing > 0.0) || std::isinf(spacing)) return fail(KIN_ERR_INVALID_ARGUMENT, "grid spacing must be positive and finite");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-        cudaGetLastError();
-        return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
-    }
+    if (int rc = require_device()) return rc;
     auto st = std::make_shared<GridStore>();
     CUDA_TRY(cudaGetDevice(&st->device));
     st->n[0] = nx; st->n[1] = ny; st->n[2] = nz;
@@ -996,7 +1040,7 @@ int kin_eval(KinModel *m, const KinCall *c) {
     if (!c->T_out && !c->J_out && !c->vals_out) return KIN_OK;
     DeviceGuard guard(m->device);
     std::shared_ptr<DeviceProgram> dp;
-    rc = get_program(m, c, dp);
+    rc = get_program(m, c, eval_kind(c), dp);
     if (rc != KIN_OK) return rc;
     return launch(m, c, dp.get(), (cudaStream_t)c->stream);
 }
@@ -1006,7 +1050,7 @@ int kin_query_launch(KinModel *m, const KinCall *c, int32_t *regs, int32_t *smem
     if (rc != KIN_OK) return rc;
     DeviceGuard guard(m->device);
     std::shared_ptr<DeviceProgram> dp;
-    rc = get_program(m, c, dp);
+    rc = get_program(m, c, eval_kind(c), dp);
     if (rc != KIN_OK) return rc;
     const LaunchPlan p = plan_launch(m, c, dp.get(), /*count_small_calls=*/false);
     if (regs) *regs = p.regs;
@@ -1130,7 +1174,7 @@ int kin_eval_host(KinModel *m, const KinCall *c) {
     if (!c->T_out && !c->J_out && !c->vals_out) return KIN_OK;
     DeviceGuard guard(m->device);
     std::shared_ptr<DeviceProgram> dp_;
-    rc = get_program(m, c, dp_);
+    rc = get_program(m, c, eval_kind(c), dp_);
     if (rc != KIN_OK) return rc;
     DeviceProgram *dp = dp_.get();
     const size_t es = c->precision == KIN_F32 ? 4 : 8;
@@ -1337,18 +1381,14 @@ int kin_sdf_points_scene(int32_t n_boxes, const int32_t *kinds, const double *bo
                          int32_t grad_mode, void *vals_out, void *grads_out, int32_t *argmin_out, void *stream_) {
     if (n < 0 || (n > 0 && (!pts || !vals_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null points or vals_out");
     if (n_boxes <= 0) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_sdf_points needs at least one box");
-    if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
-    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
+    int rc = check_batch(precision, layout, n, pts, kSoaAos);
+    if (rc != KIN_OK) return rc;
     if (grad_mode != KIN_GRAD_FD && grad_mode != KIN_GRAD_ANALYTIC && grad_mode != KIN_GRAD_FD_DIRECT) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown grad_mode");
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
-        cudaGetLastError();
-        return fail(KIN_ERR_NO_DEVICE, "no CUDA device: libkin_b200 has no CPU fallback");
-    }
+    if ((rc = require_device()) != KIN_OK) return rc;
     int cur = 0;
     CUDA_TRY(cudaGetDevice(&cur));
     kin::HostModel hm;
-    int rc = load_prims(hm, n_boxes, kinds, box_pose, box_width, grids, cur);
+    rc = load_prims(hm, n_boxes, kinds, box_pose, box_width, grids, cur);
     if (rc != KIN_OK) return rc;
     if (n == 0) return KIN_OK;
     std::vector<double> t64((size_t)n_boxes * kin::BOX_REALS, 0.0);
@@ -1388,10 +1428,10 @@ int kin_pose_residual_multi(KinModel *m, int32_t precision, int32_t layout, cons
                             const int32_t *link_ids, const int32_t *with_rots, const void *target, int32_t target_per_config,
                             int32_t mode, void *val_out, void *jac_out, void *stream_) {
     if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
-    if (n < 0 || (n > 0 && (!q || !target || !val_out || !jac_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
+    if (int rc = check_batch(precision, layout, n, q, kSoaAos)) return rc;
+    if (n > 0 && (!target || !val_out || !jac_out)) return fail(KIN_ERR_INVALID_ARGUMENT, "null argument");
     if (n_links < 1 || n_links > 32 || !link_ids || !with_rots) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_pose_residual: 1..32 links");
     if (mode != KIN_POSE_IK_OBJECTIVE && mode != KIN_POSE_CONSTRAINT) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown pose mode");
-    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_pose_residual supports the SoA and AoS layouts");
     if (n == 0) return KIN_OK;
     DeviceGuard guard(m->device);
     cudaStream_t stream = (cudaStream_t)stream_;
@@ -1449,54 +1489,22 @@ int self_collision_launch(KinModel *m, const DevicePairs &pairs, int32_t precisi
                           long long ld, double truncation_dist, double vals_offset, void *vals_out, void *grads_out,
                           void *dmin_out, int32_t *amin_out, cudaStream_t stream) {
     // phase 1 of a collision call computes the sphere centres and joint frames: the self-collision kernels run the
-    // program of a plain collision call (no links requested, clean scratch); only the pointer's presence matters
+    // program of a plain collision call (no links requested, clean scratch); only the pointer's presence matters.
+    // Always the ahead-of-time kernel, and never counted in small_calls: kin_collision calls in KIN_SCRATCH_CLEAN share
+    // that program, and when they get specialised must not depend on self-collision calls.
     KinCall c;
     std::memset(&c, 0, sizeof c);
-    c.precision = precision; c.layout = layout; c.n = n; c.q = q;
-    c.vals_out = vals_out ? vals_out : dmin_out; c.scratch_mode = KIN_SCRATCH_CLEAN;
+    c.precision = precision; c.layout = layout; c.n = n; c.batch_stride = ld; c.q = q;
+    c.vals_out = vals_out ? vals_out : dmin_out; c.grads_out = grads_out; c.scratch_mode = KIN_SCRATCH_CLEAN;
+    c.truncation_dist = truncation_dist; c.vals_offset = vals_offset;
     std::shared_ptr<DeviceProgram> dp;
-    int rc = get_program(m, &c, dp);
+    int rc = get_program(m, &c, KIND_SELF, dp);
     if (rc != KIN_OK) return rc;
-    const int pi = precision == KIN_F32 ? 1 : 0, li = layout;
-    {
-        std::lock_guard<std::mutex> lock(m->mu);
-        if (dp->self_block[pi][li] == 0 && (rc = configure(m, dp.get(), pi, li, true)) != KIN_OK) return rc;
-    }
-    kin::KernelArgs a;
-    std::memset(&a, 0, sizeof a);
-    a.h = dp->prog.h;
-    a.tab_i = dp->d_int;
-    a.tab_r = pi ? (const void *)dp->d_r32 : (const void *)dp->d_r64;
-    a.q = q;
-    a.vals_out = vals_out; a.grads_out = grads_out;
-    a.n = n; a.ld = ld;
-    a.truncation_dist = truncation_dist; a.vals_offset = vals_offset;
+    kin::KernelArgs a = kernel_args(&c, dp.get());
+    a.vals_out = vals_out;                  // (c.vals_out holds dmin_out when only the summary is asked for)
     a.self_pairs = pairs.d; a.n_self_pairs = pairs.n;
     a.dmin_out = dmin_out; a.amin_out = amin_out;
-    const int block = dp->self_block[pi][li];
-    const long long grid = persistent_grid(m, dp->self_occ[pi][li], block, n);
-    const int jr = dp->prog.h.n_dof <= kin::JF_REGS ? 1 : 0;
-    kSelfKernels[pi][li][dp->self_bs_index[pi][li]][jr]<<<(unsigned)grid, block, dp->self_smem[pi][li], stream>>>(a);
-    CUDA_TRY(cudaGetLastError());
-    g_launches.fetch_add(1);
-    return KIN_OK;
-}
-
-// The links a solve places (kin_ik_solve / kin_ik_solve_self: the call's one link; kin_ik_solve_links: up to
-// KIN_IK_MAX_LINKS), in the order of the targets.  rows: residual rows per link in the kin_eval Jacobian (6 when any
-// link has rotation).
-static_assert(kin::IKC_MAX_LINKS == KIN_IK_MAX_LINKS, "the step kernels hold KIN_IK_MAX_LINKS residual blocks");
-struct IkLinks {
-    int n = 1;
-    int32_t ids[KIN_IK_MAX_LINKS] = {};
-    unsigned rot_mask = 0;
-    int rows() const { return rot_mask ? 6 : 3; }
-};
-IkLinks ik_one_link(const KinIkCall *c) {
-    IkLinks lk;
-    lk.ids[0] = c->link_id;
-    lk.rot_mask = c->with_rot ? 1u : 0u;
-    return lk;
+    return launch_ahead_of_time(plan_ahead_of_time(m, &c, dp.get(), KIND_SELF), a, stream);
 }
 
 // The pair block of kin_ik_solve_self: the table (kept alive for the whole solve) and the margin.
@@ -1549,9 +1557,6 @@ void launch_ik_coll_step_any(const kin::IkcArgsT<SELF, LINKS> &a, int nd, int ro
 int ik_solve_coll(KinModel *m, const KinIkCall *c, const IkLinks &lk, const IkSelfBlock *sb = nullptr) {
     const int nd = m->hm.n_dof(), S = c->collision ? m->hm.n_sph : 0, rows = lk.rows(), NL = lk.n;
     const int P = sb ? sb->pairs->n : 0;
-    if (c->collision && (S < 1 || m->hm.n_box < 1))
-        return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: collision requested but the model has no spheres / no boxes");
-    if (c->collision && !(c->margin == c->margin)) return fail(KIN_ERR_INVALID_ARGUMENT, "kin_ik_solve: margin is NaN");
     DeviceGuard guard(m->device);
     cudaStream_t stream = (cudaStream_t)c->stream;
     const long long n = c->n, ld = (n + 31) / 32 * 32;
@@ -1684,12 +1689,9 @@ int ik_solve_pose(KinModel *m, const KinIkCall *c, const IkLinks &lk) {
     pc.n_jac_links = lk.n; pc.jac_links = lk.ids; pc.J_out = (void *)c->q_out; pc.with_rot = lk.rot_mask ? 1 : 0; pc.rpy_jac = 1;
     pc.truncation_dist = INFINITY;
     std::shared_ptr<DeviceProgram> dp;
-    int rc = get_program(m, &pc, dp);
+    int rc = get_program(m, &pc, KIND_FKJ, dp);
     if (rc != KIN_OK) return rc;
-    kin::GenOptions o;
-    o.precision = 0; o.layout = 0; o.want_T = true; o.want_J = true; o.with_rot = pc.with_rot; o.rpy_jac = 1;
-    o.ik = 1; o.ik_rot = lk.n > 1 ? lk.rot_mask : 0u; o.block = (int)env_ll("KIN_IK_BLOCK", 128); o.min_blocks = (int)env_ll("KIN_IK_MINB", 1);
-    std::shared_ptr<JitKernel> k = get_jit_with(m, dp.get(), o, "kin_ik_kernel");
+    std::shared_ptr<JitKernel> k = get_jit_with(m, dp.get(), ik_gen_options(lk), "kin_ik_kernel");
     if (!k) return ik_solve_coll(m, c, lk);
     kin::IkArgs a;
     std::memset(&a, 0, sizeof a);
@@ -1784,8 +1786,8 @@ int ik_check_call(KinModel *m, const KinIkCall *c, const char *what) {
     return KIN_OK;
 }
 
-// kin_ik_solve_self / kin_ik_solve_links: the pair table (self_collision != 0) and the sphere / box tables
-// (collision != 0) are checked before anything is launched, then the common path.
+// Every solve: the pair table (self_collision != 0) and the sphere / box tables (collision != 0) are checked before
+// anything is launched, then the common path.
 int ik_solve_checked(KinModel *m, const KinIkCall *c, const IkLinks &lk, bool self_collision, double self_margin,
                      void *self_dmin_out, const char *what) {
     if (self_collision && std::isnan(self_margin)) return fail(KIN_ERR_INVALID_ARGUMENT, std::string(what) + ": self_margin is NaN");
@@ -1814,9 +1816,7 @@ int kin_ik_solve(KinModel *m, const KinIkCall *c) {
     int rc = ik_check_call(m, c, "kin_ik_solve");
     if (rc != KIN_OK) return rc;
     if (c->link_id < 1 || c->link_id > m->hm.n_links) return fail(KIN_ERR_INVALID_ARGUMENT, "link id out of range");
-    if (c->n == 0) return KIN_OK;
-    if (c->collision) return ik_solve_coll(m, c, ik_one_link(c));
-    return ik_solve_pose(m, c, ik_one_link(c));
+    return ik_solve_checked(m, c, ik_one_link(c), false, 0.0, nullptr, "kin_ik_solve");
 }
 
 // kin_ik_solve plus the self-collision pairs as a hard constraint: always the augmented-Lagrangian loop of ik_solve_coll.
@@ -1853,9 +1853,8 @@ int kin_ik_solve_links(KinModel *m, const KinIkCall *c, int32_t n_links, const i
 int kin_collision_summary(KinModel *m, int32_t precision, int32_t layout, const void *q, int64_t n, double margin,
                           void *dmin_out, int32_t *amin_out, void *cost_out, void *stream_) {
     if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
-    if (n < 0 || (n > 0 && (!q || !dmin_out))) return fail(KIN_ERR_INVALID_ARGUMENT, "null q or dmin_out");
-    if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
-    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS && layout != KIN_LAYOUT_TILED32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
+    if (int rc = check_batch(precision, layout, n, q, kAnyLayout)) return rc;
+    if (n > 0 && !dmin_out) return fail(KIN_ERR_INVALID_ARGUMENT, "null dmin_out");
     if (n == 0) return KIN_OK;
     DeviceGuard guard(m->device);
     const int S = m->hm.n_sph, nd = m->hm.n_dof();
@@ -1995,10 +1994,7 @@ int kin_collision(KinModel *m, int32_t precision, int32_t layout, const void *q,
 int kin_self_collision(KinModel *m, int32_t precision, int32_t layout, const void *q, int64_t n, double truncation_dist,
                        double vals_offset, void *vals_out, void *grads_out, void *dmin_out, int32_t *amin_out, void *stream) {
     if (!m) return fail(KIN_ERR_INVALID_ARGUMENT, "null model");
-    if (precision != KIN_F64 && precision != KIN_F32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown precision");
-    if (layout != KIN_LAYOUT_SOA && layout != KIN_LAYOUT_AOS && layout != KIN_LAYOUT_TILED32) return fail(KIN_ERR_INVALID_ARGUMENT, "unknown layout");
-    if (n < 0) return fail(KIN_ERR_INVALID_ARGUMENT, "negative batch size");
-    if (n > 0 && !q) return fail(KIN_ERR_INVALID_ARGUMENT, "q is null");
+    if (int rc = check_batch(precision, layout, n, q, kAnyLayout)) return rc;
     if (!vals_out && !dmin_out) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: neither vals_out nor dmin_out given");
     if (grads_out && !vals_out) return fail(KIN_ERR_INVALID_ARGUMENT, "self collision: grads_out needs vals_out");
     if (std::isnan(truncation_dist)) return fail(KIN_ERR_INVALID_ARGUMENT, "truncation_dist is NaN");

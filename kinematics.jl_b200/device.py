@@ -188,6 +188,32 @@ def untile32(x, N):
     return x.permute(0, nd - 1, *range(1, nd - 1)).reshape((x.shape[0] * 32,) + tuple(x.shape[1:-1]))[:N]
 
 
+def _relayout(Q, q_layout, layout):
+    """Q (batch-first (N, n_dof) in ``q_layout``) brought to the layout of a call: one layout per call."""
+    if layout == _lib.TILED32:
+        return tile32(Q.contiguous() if q_layout == _lib.AOS else Q)
+    if layout != q_layout:
+        return Q.t().contiguous().t() if layout == _lib.SOA else Q.contiguous()
+    return Q
+
+
+def _alloc(layout, N, shape_soa, shape_aos, dtype, dev):
+    """Output storage of a call: SoA / AoS shapes as given; tiled: (NT, components..., 32), the SoA component order
+    inside each tile."""
+    import torch
+    if layout == _lib.TILED32:
+        return torch.empty(((N + 31) // 32,) + tuple(shape_soa[:-1]) + (32,), dtype=dtype, device=dev)
+    return torch.empty(shape_soa if layout == _lib.SOA else shape_aos, dtype=dtype, device=dev)
+
+
+def _view(x, layout, N, perm_soa, perm_aos):
+    """Batch-first view of an output storage; tiled: a batch-first COPY (N, c1, ..., ck), then the SoA reordering of
+    the component axes (indices shifted by one)."""
+    if layout == _lib.TILED32:
+        return untile32(x, N).permute(0, *[p + 1 for p in perm_soa[1:]])
+    return x.permute(*perm_soa) if layout == _lib.SOA else x.permute(*perm_aos)
+
+
 def _into(buf, shape, dtype, dev):
     """Caller-provided output storage (SoA / AoS only): must be a contiguous tensor of exactly the storage shape."""
     if tuple(buf.shape) != tuple(shape) or buf.dtype != dtype or buf.device != dev or not buf.is_contiguous():
@@ -204,12 +230,7 @@ def evaluate(dm: DeviceModel, Q, q_layout, N, *, layout=None, fk_links=None, jac
     grads (N, n_dof, S), argmin (N, S)."""
     import torch
     layout = q_layout if layout is None else layout
-    tiled = layout == _lib.TILED32
-    NT = (N + 31) // 32
-    if tiled:                               # Q arrives batch-first (N, n_dof); re-tile it
-        Q = tile32(Q.contiguous() if q_layout == _lib.AOS else Q)
-    elif layout != q_layout:                # one layout per call: bring q to the output layout
-        Q = Q.t().contiguous().t() if layout == _lib.SOA else Q.contiguous()
+    Q = _relayout(Q, q_layout, layout)
     dt = Q.dtype
     dev = Q.device
     c = _lib.KinCall()
@@ -225,25 +246,12 @@ def evaluate(dm: DeviceModel, Q, q_layout, N, *, layout=None, fk_links=None, jac
     nd = dm.n_dof
     out = {}
     keep = []
-
-    def alloc(shape_soa, shape_aos, dtype=dt):
-        if tiled:                            # (NT, components..., 32): the SoA component order inside each tile
-            return torch.empty((NT,) + tuple(shape_soa[:-1]) + (32,), dtype=dtype, device=dev)
-        return torch.empty(shape_soa if layout == _lib.SOA else shape_aos, dtype=dtype, device=dev)
-
     pending = []                             # (key, storage, perm_soa, perm_aos): views are built after the launch
-
-    def view(x, perm_soa, perm_aos):
-        if tiled:                            # batch-first COPY of the tiled storage (N, c1, ..., ck), then the SoA
-            y = untile32(x, N)               # reordering of the component axes (indices shifted by one)
-            return y.permute(0, *[p + 1 for p in perm_soa[1:]])
-        return x.permute(*perm_soa) if layout == _lib.SOA else x.permute(*perm_aos)
-
     if fk_links is not None and len(fk_links):
         ids = np.ascontiguousarray(fk_links, dtype=np.int32)
         keep.append(ids)
         n = len(ids)
-        T = alloc((n, 4, 3, N), (N, n, 4, 3))
+        T = _alloc(layout, N, (n, 4, 3, N), (N, n, 4, 3), dt, dev)
         c.n_fk_links, c.fk_links, c.T_out = n, _iptr(ids), T.data_ptr()
         pending.append(("T", T, (3, 0, 2, 1), (0, 1, 3, 2)))
     if jac_links is not None and len(jac_links):
@@ -256,7 +264,7 @@ def evaluate(dm: DeviceModel, Q, q_layout, N, *, layout=None, fk_links=None, jac
                 raise ValueError("get_jacobian!: mat_out must be a %s tensor on %s holding %d x %d x %d values per "
                                  "configuration (got %s, %s, %d values)" % (dt, dev, n, rows, nd, J.dtype, J.device, J.numel()))
         else:
-            J = alloc((n, nd, rows, N), (N, n, nd, rows))
+            J = _alloc(layout, N, (n, nd, rows, N), (N, n, nd, rows), dt, dev)
         c.n_jac_links, c.jac_links, c.J_out = n, _iptr(ids), J.data_ptr()
         c.with_rot, c.rpy_jac, c.keep_irrelevant = int(with_rot), int(rpy_jac), int(keep_irrelevant)
         pending.append(("J", J, (3, 0, 2, 1), (0, 1, 3, 2)))
@@ -265,21 +273,22 @@ def evaluate(dm: DeviceModel, Q, q_layout, N, *, layout=None, fk_links=None, jac
             raise _lib.KinError("collision requested but the device model has no spheres / no boxes "
                                 "(add_coll_links and pass an SDF first)")
         S = dm.n_spheres
-        V = alloc((S, N), (N, S)) if vals_into is None else _into(vals_into, (S, N) if layout == _lib.SOA else (N, S), dt, dev)
+        V = _alloc(layout, N, (S, N), (N, S), dt, dev) if vals_into is None else \
+            _into(vals_into, (S, N) if layout == _lib.SOA else (N, S), dt, dev)
         c.vals_out = V.data_ptr()
         pending.append(("vals", V, (1, 0), (0, 1)))
         if with_grads:
-            G = alloc((S, nd, N), (N, S, nd)) if grads_into is None else \
+            G = _alloc(layout, N, (S, nd, N), (N, S, nd), dt, dev) if grads_into is None else \
                 _into(grads_into, (S, nd, N) if layout == _lib.SOA else (N, S, nd), dt, dev)
             c.grads_out = G.data_ptr()
             pending.append(("grads", G, (2, 1, 0), (0, 2, 1)))
         if want_argmin:
-            Am = alloc((S, N), (N, S), torch.int32)
+            Am = _alloc(layout, N, (S, N), (N, S), torch.int32, dev)
             c.argmin_out = Am.data_ptr()
             pending.append(("argmin", Am, (1, 0), (0, 1)))
     _lib.check(_lib.lib().kin_eval(dm.h, C.byref(c)))
     for key, store, perm_soa, perm_aos in pending:
-        out[key] = view(store, perm_soa, perm_aos)
+        out[key] = _view(store, layout, N, perm_soa, perm_aos)
     if launch_info:                          # which kernel configuration this call maps to (kin_query_launch)
         regs, smem, block, grid = C.c_int32(), C.c_int32(), C.c_int32(), C.c_int32()
         _lib.check(_lib.lib().kin_query_launch(dm.h, C.byref(c), C.byref(regs), C.byref(smem), C.byref(block), C.byref(grid)))
@@ -294,26 +303,10 @@ def evaluate_self(dm: DeviceModel, Q, q_layout, N, *, layout=None, with_vals=Tru
     amin (N,) int32 are plain arrays."""
     import torch
     layout = q_layout if layout is None else layout
-    tiled = layout == _lib.TILED32
-    if tiled:
-        Q = tile32(Q.contiguous() if q_layout == _lib.AOS else Q)
-    elif layout != q_layout:
-        Q = Q.t().contiguous().t() if layout == _lib.SOA else Q.contiguous()
+    Q = _relayout(Q, q_layout, layout)
     dt, dev, nd, P = Q.dtype, Q.device, dm.n_dof, dm.n_self_pairs
-    NT = (N + 31) // 32
-
-    def alloc(shape_soa, shape_aos):
-        if tiled:
-            return torch.empty((NT,) + tuple(shape_soa[:-1]) + (32,), dtype=dt, device=dev)
-        return torch.empty(shape_soa if layout == _lib.SOA else shape_aos, dtype=dt, device=dev)
-
-    def view(x, perm_soa, perm_aos):
-        if tiled:
-            return untile32(x, N).permute(0, *[p + 1 for p in perm_soa[1:]])
-        return x.permute(*perm_soa) if layout == _lib.SOA else x.permute(*perm_aos)
-
-    V = alloc((P, N), (N, P)) if with_vals else None
-    G = alloc((P, nd, N), (N, P, nd)) if with_grads else None
+    V = _alloc(layout, N, (P, N), (N, P), dt, dev) if with_vals else None
+    G = _alloc(layout, N, (P, nd, N), (N, P, nd), dt, dev) if with_grads else None
     dmin = torch.empty(N, dtype=dt, device=dev) if want_summary else None
     amin = torch.empty(N, dtype=torch.int32, device=dev) if want_summary else None
     ptr = lambda t: None if t is None else t.data_ptr()
@@ -322,9 +315,9 @@ def evaluate_self(dm: DeviceModel, Q, q_layout, N, *, layout=None, with_vals=Tru
                                              torch.cuda.current_stream(dev).cuda_stream if stream is None else stream))
     out = {}
     if V is not None:
-        out["vals"] = view(V, (1, 0), (0, 1))
+        out["vals"] = _view(V, layout, N, (1, 0), (0, 1))
     if G is not None:
-        out["grads"] = view(G, (2, 1, 0), (0, 2, 1))
+        out["grads"] = _view(G, layout, N, (2, 1, 0), (0, 2, 1))
     if want_summary:
         out["dmin"], out["amin"] = dmin, amin
     return out

@@ -116,6 +116,8 @@ def test_two_link_ik_kernel_compiles_for_sm_100a(tmp_path, with_base):
     cfg = (out / "kin_gen_config.h").read_text()
     assert "#define KIK 1" in cfg and "#define KIKROT 0x3u" in cfg
     assert re.search(r"KND = %d, .*KNFK = 2, KNJAC = 2, KROWS = 6;" % (18 if with_base else 15), cfg)
+    # the option set kin_ik_solve_links compiles: 64-bit component strides, whatever the dumped call's batch size
+    assert "#define KES32 0" in cfg
     cubin = out / "kin_gen.cubin"
     assert cubin.stat().st_size > 0
     tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
